@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload c4|c5|c4s] [--mode fantasy|lipschitz] [--precision tf32|tf32x3|fp64]
+                    [--dump-outputs DIR]
 
 A "step" = model upload -> GP posterior over the grid for all G GPs -> safe/minimiser/unsafe sets ->
 Lipschitz constants (Lipschitz mode) -> expander pair kernel -> arg-reductions -> x_new.  It EXCLUDES the
@@ -55,7 +56,14 @@ def parse():
     ap.add_argument("--no-lipschitz-steps", action="store_true", help="skip the reference-exact SafeOpt/GoOSE step times (extra key)")
     ap.add_argument("--no-reference-configs", action="store_true", help="skip the C1-C3 step times (extra key)")
     ap.add_argument("--prune", type=int, default=1, help="exact key-ordered tile pruning of the fantasy expander (default 1 = the library default; 0 = every pair)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def workload(name):
@@ -393,6 +401,56 @@ def c5_key(args, eng, torch, dist, stream, rank, world, dev, barrier):
     return out
 
 
+DUMP_POINTS = 1 << 18      # per-point outputs are dumped at this many seeded points of the shard (all of a smaller one)
+# step result fields -> the index field that is -1 when the reduction behind the value found no candidate
+_INDEX_OF = {"best_value": "best_idx", "per_value": "per_idx", "undecided_best_value": "undecided_best_idx",
+             "min_ucb0": "min_ucb0_idx", "min_lcb0": "min_lcb0_idx", "minimizer_var": "minimizer_idx",
+             "target_lcb": "target_idx"}
+
+
+class _DeviceF64:
+    """A float64 device buffer of the library, exposed to torch through __cuda_array_interface__ (no copy; only read,
+    but torch accepts no read-only flag)."""
+
+    def __init__(self, ptr, shape):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<f8", "data": (int(ptr), False),
+                                         "strides": None, "version": 3}
+
+
+def dump_outputs(out_dir, eng, res, torch, dev):
+    """--dump-outputs: what the last timed step computed, one DIR/<name>.npy per array.  The step's result as the
+    caller receives it (sets, L, expander fields, x_new_idx; float64, nested keys joined by "_") and the per-point
+    outputs the step leaves in the engine: posterior mean and variance (float64, (points, G) like GridEngine.posterior)
+    and the safe / minimiser / unsafe masks (float32 0/1), at `point_index` (float64), a fixed seeded sample of
+    DUMP_POINTS points of this rank's shard.  Under 40 MB in all (G <= 8).  The workloads are seeded, so two builds run
+    with the same arguments can be compared array for array, except two work counters that were seen to vary between
+    runs of one build (C4, 1 x B200): expander_n_ambiguous (pairs inside the TF32 error band, by one) and
+    expander_pairs_evaluated (pairs the pruning keeps, by 2e-6 of them).
+    A value whose index is -1 (no candidate) holds the library's +-inf sentinel; it is written as 0, as GridEngine
+    already reports expander_std and minimizer_std, and the index says that it is absent."""
+    from sbo_b200 import _capi as capi
+    out = {}
+    for k, v in res.items():
+        scope, prefix = (v, k + "_") if isinstance(v, dict) else (res, "")
+        for name in (v if isinstance(v, dict) else [k]):
+            a = np.asarray(scope[name], dtype=np.float64)
+            if _INDEX_OF.get(name) in scope:
+                a = np.where(np.asarray(scope[_INDEX_OF[name]]) < 0, 0.0, a)
+            out[prefix + name] = a
+    cnt = eng.count
+    sel = np.arange(cnt) if cnt <= DUMP_POINTS else np.sort(np.random.default_rng(0).choice(cnt, DUMP_POINTS, replace=False))
+    out["point_index"] = sel.astype(np.float64)
+    for name, kind in (("safe_mask", capi.MASK_SAFE), ("minimizer_mask", capi.MASK_MIN), ("unsafe_mask", capi.MASK_UNSAFE)):
+        out[name] = eng.mask(kind)[sel].astype(np.float32)
+    idx = torch.as_tensor(sel, device=dev)
+    for name, ptr in zip(("posterior_mean", "posterior_var"), eng.posterior_dev()):
+        buf = torch.as_tensor(_DeviceF64(ptr, (eng.G, cnt)), device=dev)          # [G][count], as the kernels write it
+        out[name] = buf.index_select(1, idx).T.contiguous().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -463,6 +521,8 @@ def run_ours(args):
     barrier()
     clk = clocks.stop()
     launches = eng.kernel_launches()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, res, torch, dev)
     ms = float(np.mean([a.elapsed_time(b) for a, b in ev]))
     # ---- end-to-end steps (host buffers in, host results out) ----
     t_e2e = []
