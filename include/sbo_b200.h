@@ -250,6 +250,10 @@ int64_t sbo_mem_peak(sbo_ctx* ctx, int reset);
  * phase: 0 model, 1 posterior(crosscov), 2 posterior(solve), 3 sets, 4 pairs, 5 argreduce, 6 pair preparation,
  *        7 FP64 refinement of the split-TF32 fantasy expander */
 int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms);
+/* FP64 refinement of the last pair stage on ctx (fantasy_refine = 2 / 1): the cells the pass was cut into and the FP64 rows
+ * V = L^-1 K(X, p) it computed (one cell: one row per distinct candidate and unsafe point of the ambiguous list; more cells
+ * compute the inner side's rows once per outer block).  0 / 0 when nothing was refined. */
+int sbo_refine_stats(sbo_ctx* ctx, int64_t* cells, int64_t* fp64_rows);
 /* tuning / diagnosis options (defaults reproduce the documented behaviour; none changes a result):
  *   "posterior_variant"  1 (default) FP64 tensor cores (DMMA) | 0 FP64 SIMT register tiles
  *   "posterior_tables"   1: on meshgrids the cross-covariance kernel multiplies separable SE-ARD factor tables instead of calling
@@ -265,11 +269,16 @@ int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms);
  *                        are evaluated; FP64 counts are unchanged | 0: every pair goes through the GEMM
  *   "prior_mean_zero"    1: zero prior mean for every GP at the next sbo_set_model (GP_Robust.py, StableOpt) | 0 (default) GP_Safe.py:331
  *   "fantasy_refine"     2 (default): the TF32 and TF32X3 fantasy expanders settle every pair inside their error bound in FP64
- *                        (the counts are the FP64 counts) | 1: TF32X3 only | 0: decide on the tensor-core value
+ *                        (the counts are the FP64 counts, at any grid size where the ambiguous pairs fit the list: fewer than 2^31
+ *                        per shard) | 1: TF32X3 only | 0: decide on the tensor-core value
  *                        | 3: bounds mode -- no FP64 pass: the counts are the pairs the error bound settles as newly safe (a lower bound
- *                        of the FP64 counts) and sbo_pair_result.n_undecided / undecided_best_* say what is left open (for shards
- *                        whose ambiguous pairs do not fit a list: C5)
+ *                        of the FP64 counts) and sbo_pair_result.n_undecided / undecided_best_* say what is left open (cheaper than
+ *                        the FP64 pass, and the mode for shards whose ambiguous pairs do not fit the list)
  *   "fantasy_refine_cap" > 0: initial capacity (pairs) of the ambiguous-pair list instead of the heuristic (test hook)
+ *   "fantasy_refine_mb"  device memory of the FP64 refinement (its FP64 rows, their posterior scratch and the cell buckets) in MB:
+ *                        0 (default) what cudaMemGetInfo reports free at the start of the pass less 1 GB | > 0 at most this much.
+ *                        When the rows of all listed points do not fit, the pass runs cell by cell (blocks of candidates x
+ *                        blocks of unsafe points); the counts do not change.  A budget below one row per side: SBO_ERR_NOMEM
  *   "fantasy_f64_variant" 1 (default): FP64 fantasy expander on the FP64 tensor cores (DMMA tiles) | 0: SIMT reference kernel
  *   "pair_cull"          1 (default): exact bounding-box tile culling in the Lipschitz pair kernels | 0 all pairs */
 int sbo_set_option(sbo_ctx* ctx, const char* name, int64_t value);

@@ -101,6 +101,7 @@ SIGNATURES = {
     "sbo_kernel_launches": (C.c_int64, [_P, C.c_int]),
     "sbo_mem_peak": (C.c_int64, [_P, C.c_int]),
     "sbo_phase_ms": (C.c_int, [_P, C.c_int, _D]),
+    "sbo_refine_stats": (C.c_int, [_P, _I64, _I64]),
     "sbo_set_option": (C.c_int, [_P, C.c_char_p, C.c_int64]),
     "sbo_release": (C.c_int, [_P, C.c_int]),
     "sbo_nll_batch": (C.c_int, [_P, C.c_int, C.c_int, _D, _D, C.c_int, _D, _D]),

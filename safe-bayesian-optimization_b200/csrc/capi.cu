@@ -11,11 +11,11 @@ int sbo_fail(sbo_ctx* ctx, int code, const std::string& msg) {
   return code;
 }
 
-int sbo_ensure(sbo_ctx* ctx, DevBuf& b, size_t bytes) {
+static int ensure(sbo_ctx* ctx, DevBuf& b, size_t bytes, bool headroom) {
   if (bytes == 0) bytes = 16;
   if (b.cap >= bytes) return SBO_OK;
   if (b.p) { cudaStreamSynchronize(ctx->stream); cudaFree(b.p); ctx->mem_now -= (int64_t)b.cap; b.p = nullptr; b.cap = 0; }
-  size_t want = bytes + bytes / 8;
+  size_t want = headroom ? bytes + bytes / 8 : bytes;
   cudaError_t e = cudaMalloc(&b.p, want);
   if (e != cudaSuccess) { cudaGetLastError(); want = bytes; e = cudaMalloc(&b.p, want); }
   if (e != cudaSuccess) {
@@ -26,6 +26,16 @@ int sbo_ensure(sbo_ctx* ctx, DevBuf& b, size_t bytes) {
   ctx->mem_now += (int64_t)want;
   if (ctx->mem_now > ctx->mem_peak) ctx->mem_peak = ctx->mem_now;
   return SBO_OK;
+}
+int sbo_ensure(sbo_ctx* ctx, DevBuf& b, size_t bytes) { return ensure(ctx, b, bytes, true); }
+int sbo_ensure_exact(sbo_ctx* ctx, DevBuf& b, size_t bytes) { return ensure(ctx, b, bytes, false); }
+
+void sbo_free(sbo_ctx* ctx, DevBuf& b) {
+  if (!b.p) return;
+  cudaStreamSynchronize(ctx->stream);
+  cudaFree(b.p);
+  ctx->mem_now -= (int64_t)b.cap;
+  b.p = nullptr; b.cap = 0;
 }
 
 static void free_buf(DevBuf& b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
@@ -95,7 +105,7 @@ int sbo_destroy(sbo_ctx* ctx) {
                     &ctx->kx, &ctx->lmax, &ctx->vall, &ctx->tile_bb, &ctx->nll_K, &ctx->nll_in, &ctx->m_safe, &ctx->m_unsafe, &ctx->m_min, &ctx->m_user, &ctx->m_exp,
                     &ctx->m_tgt, &ctx->partials, &ctx->result, &ctx->scan_a, &ctx->scan_b, &ctx->xs_idx, &ctx->zs_idx,
                     &ctx->xs_pay, &ctx->zs_pay, &ctx->hits, &ctx->counts, &ctx->pairctr, &ctx->imp_rows, &ctx->vx, &ctx->vz,
-                    &ctx->aux_x, &ctx->aux_z, &ctx->pp_x, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->pp_g, &ctx->tc_row, &ctx->tc_col, &ctx->tc_err, &ctx->exp_rows, &ctx->exp_v, &ctx->key_x, &ctx->key_z, &ctx->perm_x, &ctx->perm_z, &ctx->sort_ws, &ctx->tile_keys, &ctx->item_mask, &ctx->item_list, &ctx->gz_mask, &ctx->gz_idx, &ctx->gz_pay, &ctx->st_score, &ctx->st_mask, &ctx->tabs, &ctx->tc_stats, &ctx->amb_list, &ctx->amb_ctr, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts, &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_rows, &ctx->m_und})
+                    &ctx->aux_x, &ctx->aux_z, &ctx->pp_x, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->pp_g, &ctx->tc_row, &ctx->tc_col, &ctx->tc_err, &ctx->exp_rows, &ctx->exp_v, &ctx->key_x, &ctx->key_z, &ctx->perm_x, &ctx->perm_z, &ctx->sort_ws, &ctx->tile_keys, &ctx->item_mask, &ctx->item_list, &ctx->gz_mask, &ctx->gz_idx, &ctx->gz_pay, &ctx->st_score, &ctx->st_mask, &ctx->tabs, &ctx->tc_stats, &ctx->amb_list, &ctx->amb_ctr, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts, &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_rows, &ctx->m_und, &ctx->amb_cell, &ctx->amb_hist})
     free_buf(*b);
   ev_collect(ctx);
   for (cudaEvent_t e : ctx->evpool) cudaEventDestroy(e);
@@ -405,6 +415,13 @@ int64_t sbo_mem_peak(sbo_ctx* ctx, int reset) {
   return v;
 }
 
+int sbo_refine_stats(sbo_ctx* ctx, int64_t* cells, int64_t* fp64_rows) {
+  ENTER();
+  SBO_REQUIRE(cells && fp64_rows, "null out pointer");
+  *cells = ctx->refine_cells; *fp64_rows = ctx->refine_rows;
+  return SBO_OK;
+}
+
 int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms) {
   ENTER();
   SBO_REQUIRE(phase >= 0 && phase < 8 && ms, "bad phase");
@@ -434,6 +451,10 @@ int sbo_release(sbo_ctx* ctx, int what) {
   if (what & 1) { ctx->mem_now -= (int64_t)ctx->vall.cap; free_buf(ctx->vall); ctx->keep_v = 0; }
   if (what & 2) {
     for (DevBuf* b : {&ctx->vx, &ctx->vz, &ctx->exp_v, &ctx->tc_row, &ctx->tc_col, &ctx->imp_rows}) { ctx->mem_now -= (int64_t)b->cap; free_buf(*b); }
+    // workspaces of the FP64 refinement: the ambiguous-pair list, its points, rank maps, buckets and FP64 rows
+    for (DevBuf* b : {&ctx->amb_list, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts,
+                      &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_cell, &ctx->amb_hist})
+      sbo_free(ctx, *b);
     ctx->ps = PairStage{};
   }
   return SBO_OK;
@@ -450,6 +471,10 @@ int sbo_set_option(sbo_ctx* ctx, const char* name, int64_t value) {
   if (!strcmp(name, "prior_mean_zero")) { ctx->opt_prior_mean_zero = value; return SBO_OK; }
   if (!strcmp(name, "fantasy_refine_cap")) { ctx->opt_fantasy_refine_cap = value; return SBO_OK; }
   if (!strcmp(name, "fantasy_refine")) { ctx->opt_fantasy_refine = value; return SBO_OK; }
+  if (!strcmp(name, "fantasy_refine_mb")) {
+    SBO_REQUIRE(value >= 0, "fantasy_refine_mb must be >= 0 (0 = the free device memory)");
+    ctx->opt_fantasy_refine_mb = value; return SBO_OK;
+  }
   if (!strcmp(name, "fantasy_f64_variant")) { ctx->opt_fantasy_f64_variant = value; return SBO_OK; }
   if (!strcmp(name, "pair_cull")) { ctx->opt_pair_cull = value; return SBO_OK; }
   if (!strcmp(name, "fantasy_gx")) { ctx->opt_fantasy_gx = value; return SBO_OK; }

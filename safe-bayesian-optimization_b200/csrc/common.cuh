@@ -166,6 +166,8 @@ struct sbo_ctx {
   DevBuf exp_rows, exp_v;                 // single-GPU export buffers of the staged pair driver
   DevBuf key_x, key_z, perm_x, perm_z, sort_ws, tile_keys, item_mask, item_list;   // exact pruning of the fantasy expander
   DevBuf amb_list, amb_ctr, amb_mask, amb_xd, amb_zd, amb_rx, amb_rz, amb_pts, amb_vx, amb_vz, amb_rows, m_und;   // FP64 refinement of the split-TF32 expander
+  DevBuf amb_cell, amb_hist;              // cell-wise refinement: the ambiguous list bucketed by cell, per-cell counters
+  int64_t refine_cells = 0, refine_rows = 0;   // last pair stage: cells of the FP64 refinement and FP64 rows computed (sbo_refine_stats)
   DevBuf st_score, st_mask;               // StableOpt: per-x_c worst-case score and robust-safe bitmask
   DevBuf gz_mask, gz_idx, gz_pay;         // all-gathered unsafe set of a sharded Lipschitz expander
   PairStage ps;
@@ -190,6 +192,7 @@ struct sbo_ctx {
   int64_t opt_fantasy_refine = 2;     // tensor-core fantasy expander: pairs the FP32/TF32 error bound cannot settle are re-evaluated in FP64 (exact
                                       // counts): 2 (default) TF32 and TF32X3, 1 TF32X3 only, 0 off (decide on the tensor-core value)
   int64_t opt_fantasy_refine_cap = 0; // > 0: initial capacity of the ambiguous-pair list (tests force the overflow / re-run path with it)
+  int64_t opt_fantasy_refine_mb = 0;  // device memory of the FP64 refinement pass in MB: 0 (default) what is free, > 0 at most this
   int64_t opt_pair_cull = 1;         // Lipschitz pair kernels: exact bounding-box culling of staged tiles
   int64_t opt_fantasy_gx = 0;        // 2-CTA kernel: x tile pairs per raster group (0 = default)
 };
@@ -198,6 +201,8 @@ extern thread_local std::string g_sbo_last_error;
 
 int sbo_fail(sbo_ctx* ctx, int code, const std::string& msg);
 int sbo_ensure(sbo_ctx* ctx, DevBuf& b, size_t bytes);
+int sbo_ensure_exact(sbo_ctx* ctx, DevBuf& b, size_t bytes);   // as sbo_ensure, without the 1/8 head-room
+void sbo_free(sbo_ctx* ctx, DevBuf& b);                         // give a work buffer back to the driver
 
 #define SBO_CUDA(call)                                                                         \
   do {                                                                                         \
@@ -241,6 +246,7 @@ int stable_minmax(sbo_ctx* ctx, int n_controlled, int fun_kind, double beta, int
 int nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll);
 int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v);
 int posterior_vrows_dev(sbo_ctx* ctx, long long m, const double* pts_dev, double* vout);
+void posterior_vrows_scratch(const sbo_ctx* ctx, long long m, size_t* mv_bytes, size_t* k_bytes);
 int posterior_points(sbo_ctx* ctx, int64_t m, const double* x, double* mean, double* var);
 int posterior_point_grad(sbo_ctx* ctx, int gp, int64_t m, const double* x, double* grad);
 int sets_pass1(sbo_ctx* ctx, double beta, int rule, int strict, sbo_sets_result* out);

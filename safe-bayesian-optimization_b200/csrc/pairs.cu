@@ -924,10 +924,44 @@ __global__ void __launch_bounds__(256) k_amb_points(ModelSpec ms, long long m, l
   rank[id] = (int)r;
   for (int k = 0; k < ms.d; ++k) pts[(size_t)r * ms.d + k] = xn_soa[(size_t)k * ntot + id] * ms.Xstd[k] + ms.Xmean[k];
 }
+// ---------------------------------------------------------------------------------------------
+// Cell-wise pass for lists whose points' FP64 rows do not fit the device at once (C5: ~1.6 M + 1.6 M rows of 49 KB per
+// rank).  The compacted points are ranked, so a block is a contiguous rank range and cell = (outer block, inner block).
+// The list is bucketed by cell (histogram, exclusive scan, scatter; the order inside a cell is arbitrary and no count
+// depends on it); every outer block's rows are computed once, the inner blocks' rows once per outer block that pairs
+// with them.  Every pair is evaluated by the same k_refine_pairs arithmetic on the same FP64 rows as in one cell.
+// ---------------------------------------------------------------------------------------------
+struct CellPlan {
+  int bx, bz;              // block lengths in ranks (candidates, unsafe points)
+  long long nbx, nbz;      // blocks per side
+  bool z_outer;            // the z blocks form the outer loop (their rows are computed once)
+};
+__device__ __forceinline__ long long cell_of(const CellPlan& p, const int* __restrict__ rank_x, const int* __restrict__ rank_z, int2 e) {
+  const long long cx = rank_x[e.x] / p.bx, cz = rank_z[e.y] / p.bz;
+  return p.z_outer ? cz * p.nbx + cx : cx * p.nbz + cz;
+}
+__global__ void __launch_bounds__(256)
+k_cell_hist(long long n, const int2* __restrict__ list, CellPlan p, const int* __restrict__ rank_x, const int* __restrict__ rank_z,
+            int* __restrict__ hist) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n) atomicAdd(hist + cell_of(p, rank_x, rank_z, list[t]), 1);
+}
+__global__ void __launch_bounds__(256)
+k_cell_scatter(long long n, const int2* __restrict__ list, CellPlan p, const int* __restrict__ rank_x, const int* __restrict__ rank_z,
+               int* __restrict__ cursor, int2* __restrict__ out) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const int2 e = list[t];
+  out[atomicAdd(cursor + cell_of(p, rank_x, rank_z, e), 1)] = e;
+}
+
+// one warp per ambiguous pair of list[0..n_amb).  Vx / Vz hold the FP64 rows of the ranks [x0, x0 + mx) / [z0, z0 + mz_)
+// (one cell: all ranks, offsets 0)
 template <int D>
 __global__ void __launch_bounds__(256)
 k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list, long long nx, long long nz, long long mx, long long mz_,
-               const int* __restrict__ rank_x, const int* __restrict__ rank_z, const double* __restrict__ Vx, const double* __restrict__ Vz,
+               long long x0, long long z0, const int* __restrict__ rank_x, const int* __restrict__ rank_z,
+               const double* __restrict__ Vx, const double* __restrict__ Vz,
                const double* __restrict__ xn, const double* __restrict__ ax, const double* __restrict__ bx,
                const double* __restrict__ zn, const double* __restrict__ mz, const double* __restrict__ sz,
                int* __restrict__ counts, const int* __restrict__ row_perm, unsigned long long* __restrict__ n_safe) {
@@ -936,7 +970,7 @@ k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list,
   const int lane = threadIdx.x & 31;
   const int2 e = list[w];
   const long long xi = e.x, zi = e.y;
-  const long long rx = rank_x[xi], rz = rank_z[zi];
+  const long long rx = rank_x[xi] - x0, rz = rank_z[zi] - z0;
   bool ok = true;
   for (int c = 0; c < fc.nc && ok; ++c) {
     const double* vx = Vx + ((size_t)c * mx + rx) * fc.npad;
@@ -957,6 +991,56 @@ k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list,
     atomicAdd(counts + (row_perm ? row_perm[xi] : xi), 1);
     atomicAdd(n_safe, 1ULL);
   }
+}
+
+static int launch_refine(sbo_ctx* ctx, const FantasyConsts& fc, long long n, const int2* list, long long nx, long long nz,
+                         long long mx, long long mz_, long long x0, long long z0, const double* Vx, const double* Vz,
+                         int* counts, const int* row_perm) {
+  const int d = fc.d, nc = fc.nc;
+  const double* xn = (const double*)ctx->aux_x.p; const double* ax = xn + (size_t)d * nx; const double* bx = ax + (size_t)nc * nx;
+  const double* zn = (const double*)ctx->aux_z.p; const double* mz = zn + (size_t)d * nz; const double* sz = mz + (size_t)nc * nz;
+  unsigned long long* nsafe = (unsigned long long*)ctx->amb_ctr.p + 1;
+#define RP(DD) k_refine_pairs<DD><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0, (const int*)ctx->amb_rx.p, \
+      (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe)
+  switch (d) { case 1: RP(1); break; case 2: RP(2); break; case 3: RP(3); break; case 4: RP(4); break;
+               case 5: RP(5); break; case 6: RP(6); break; case 7: RP(7); break; default: RP(8); break; }
+#undef RP
+  SBO_LAUNCH_CHECK();
+  return SBO_OK;
+}
+
+#define REFINE_RESERVE ((size_t)1 << 30)        // automatic budget: device memory left to everything else
+#define REFINE_MAX_CELLS (1LL << 22)
+
+// FP64 rows + posterior scratch + buckets of a multi-cell pass with blocks (bx, bz)
+static size_t cell_pass_bytes(const sbo_ctx* ctx, long long n_amb, size_t row_b, long long bx, long long bz, long long cells) {
+  size_t mv, kb;
+  posterior_vrows_scratch(ctx, bx > bz ? bx : bz, &mv, &kb);
+  return (size_t)(bx + bz) * row_b + 2 * mv + kb + sizeof(int2) * (size_t)n_amb + sizeof(int) * 2 * (size_t)cells;
+}
+
+// the largest blocks whose pass fits `budget`: the inner side gets a quarter of the rows (all of its ranks if fewer), the
+// outer side the rest; of the two orientations the one that computes fewer rows (outer once, inner once per outer block)
+static bool plan_cells(const sbo_ctx* ctx, long long mx, long long mz, long long n_amb, size_t row_b, size_t budget, CellPlan* best) {
+  const size_t fixed = sizeof(int2) * (size_t)n_amb;
+  if (budget <= fixed + 2 * row_b) return false;
+  for (long long R = (long long)((budget - fixed) / row_b); R >= 2; R -= R / 8 > 1 ? R / 8 : 1) {
+    long long best_rows = -1;
+    for (int zo = 0; zo < 2; ++zo) {
+      const long long mo = zo ? mz : mx, mi = zo ? mx : mz;
+      long long bi = mi < R / 4 ? mi : (R / 4 > 1 ? R / 4 : 1);
+      const long long bo = mo < R - bi ? mo : R - bi;
+      bi = mi < R - bo ? mi : R - bo;
+      const long long no = cdiv(mo, bo), ni = cdiv(mi, bi);
+      if (bo > 2000000000LL || bi > 2000000000LL || no * ni > REFINE_MAX_CELLS) continue;
+      const long long rows = mo + mi * no;
+      CellPlan p{(int)(zo ? bi : bo), (int)(zo ? bo : bi), zo ? ni : no, zo ? no : ni, zo == 1};
+      if (cell_pass_bytes(ctx, n_amb, row_b, p.bx, p.bz, no * ni) > budget) continue;
+      if (best_rows < 0 || rows < best_rows) { best_rows = rows; *best = p; }
+    }
+    if (best_rows >= 0) return true;
+  }
+  return false;
 }
 
 static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx, long long nz, int* counts, const int* row_perm) {
@@ -986,27 +1070,102 @@ static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx,
   SBO_TRY(sbo_ensure(ctx, ctx->amb_rx, sizeof(int) * (size_t)nx));
   SBO_TRY(sbo_ensure(ctx, ctx->amb_rz, sizeof(int) * (size_t)nz));
   SBO_TRY(sbo_ensure(ctx, ctx->amb_pts, sizeof(double) * (size_t)(mx + mzd) * d));
-  SBO_TRY(sbo_ensure(ctx, ctx->amb_vx, sizeof(double) * (size_t)nc * mx * ms.npad));
-  SBO_TRY(sbo_ensure(ctx, ctx->amb_vz, sizeof(double) * (size_t)nc * mzd * ms.npad));
-  const double* xn = (const double*)ctx->aux_x.p; const double* ax = xn + (size_t)d * nx; const double* bx = ax + (size_t)nc * nx;
-  const double* zn = (const double*)ctx->aux_z.p; const double* mz = zn + (size_t)d * nz; const double* sz = mz + (size_t)nc * nz;
+  const double* xn = (const double*)ctx->aux_x.p;
+  const double* zn = (const double*)ctx->aux_z.p;
   double* ptx = (double*)ctx->amb_pts.p; double* ptz = ptx + (size_t)mx * d;
   k_amb_points<<<(unsigned)cdiv(mx, 256), 256, 0, ctx->stream>>>(ms, mx, nx, (const long long*)ctx->amb_xd.p, xn, (int*)ctx->amb_rx.p, ptx);
   SBO_LAUNCH_CHECK();
   k_amb_points<<<(unsigned)cdiv(mzd, 256), 256, 0, ctx->stream>>>(ms, mzd, nz, (const long long*)ctx->amb_zd.p, zn, (int*)ctx->amb_rz.p, ptz);
   SBO_LAUNCH_CHECK();
-  SBO_TRY(posterior_vrows_dev(ctx, mx, ptx, (double*)ctx->amb_vx.p));
-  SBO_TRY(posterior_vrows_dev(ctx, mzd, ptz, (double*)ctx->amb_vz.p));
-  unsigned long long* nsafe = (unsigned long long*)ctx->amb_ctr.p + 1;
-#define RP(DD) k_refine_pairs<DD><<<(unsigned)cdiv(n_amb, 8), 256, 0, ctx->stream>>>(fc, n_amb, list, nx, nz, mx, mzd, (const int*)ctx->amb_rx.p, \
-      (const int*)ctx->amb_rz.p, (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe)
-  switch (d) { case 1: RP(1); break; case 2: RP(2); break; case 3: RP(3); break; case 4: RP(4); break;
-               case 5: RP(5); break; case 6: RP(6); break; case 7: RP(7); break; default: RP(8); break; }
-#undef RP
-  SBO_LAUNCH_CHECK();
+
+  // memory budget of the pass: option fantasy_refine_mb, or what is free now plus the buffers the pass (re)uses, less a reserve
+  const size_t row_b = sizeof(double) * (size_t)nc * ms.npad;          // FP64 rows of one point, all constraints
+  size_t free_b = 0, total_b = 0;
+  SBO_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  size_t avail = free_b;
+  for (const DevBuf* b : {&ctx->amb_vx, &ctx->amb_vz, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->amb_cell, &ctx->amb_hist}) avail += b->cap;
+  size_t budget = avail > REFINE_RESERVE ? avail - REFINE_RESERVE : 0;
+  if (ctx->opt_fantasy_refine_mb > 0 && (size_t)ctx->opt_fantasy_refine_mb << 20 < budget) budget = (size_t)ctx->opt_fantasy_refine_mb << 20;
+  size_t mv1, kb1;
+  posterior_vrows_scratch(ctx, mx > mzd ? mx : mzd, &mv1, &kb1);
+  const size_t one_cell = (size_t)(mx + mzd) * row_b + 2 * mv1 + kb1;
+
+  const bool multi = one_cell > budget;
+  if (!multi) {
+    // one cell: every row at once (the buffers keep sbo_ensure's head-room when the budget has it)
+    const bool room = one_cell + one_cell / 8 <= budget;
+    SBO_TRY((room ? sbo_ensure : sbo_ensure_exact)(ctx, ctx->amb_vx, sizeof(double) * (size_t)nc * mx * ms.npad));
+    SBO_TRY((room ? sbo_ensure : sbo_ensure_exact)(ctx, ctx->amb_vz, sizeof(double) * (size_t)nc * mzd * ms.npad));
+    if (!room) {
+      SBO_TRY(sbo_ensure_exact(ctx, ctx->pp_m, mv1)); SBO_TRY(sbo_ensure_exact(ctx, ctx->pp_v, mv1)); SBO_TRY(sbo_ensure_exact(ctx, ctx->pp_k, kb1));
+    }
+    SBO_TRY(posterior_vrows_dev(ctx, mx, ptx, (double*)ctx->amb_vx.p));
+    SBO_TRY(posterior_vrows_dev(ctx, mzd, ptz, (double*)ctx->amb_vz.p));
+    SBO_TRY(launch_refine(ctx, fc, n_amb, list, nx, nz, mx, mzd, 0, 0, (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, counts, row_perm));
+    ctx->refine_cells = 1; ctx->refine_rows = mx + mzd;
+  } else {
+    CellPlan p{};
+    if (!plan_cells(ctx, mx, mzd, n_amb, row_b, budget, &p))
+      return sbo_fail(ctx, SBO_ERR_NOMEM, "split-TF32 refinement: " + std::to_string(budget >> 20) + " MB cannot hold the FP64 rows of one candidate "
+                                              "and one unsafe point with their scratch (" + std::to_string(n_amb) + " ambiguous pairs); raise option "
+                                              "fantasy_refine_mb (0 = the free device memory) or use fantasy_refine = 3");
+    const long long ncell = p.nbx * p.nbz;
+    // the budget was planned for exactly these buffers: drop what the context holds and allocate them without head-room
+    for (DevBuf* b : {&ctx->amb_vx, &ctx->amb_vz, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->amb_cell, &ctx->amb_hist}) sbo_free(ctx, *b);
+    size_t mv, kb;
+    posterior_vrows_scratch(ctx, p.bx > p.bz ? p.bx : p.bz, &mv, &kb);
+    SBO_TRY(sbo_ensure_exact(ctx, ctx->amb_vx, row_b * (size_t)p.bx));
+    SBO_TRY(sbo_ensure_exact(ctx, ctx->amb_vz, row_b * (size_t)p.bz));
+    SBO_TRY(sbo_ensure_exact(ctx, ctx->pp_m, mv)); SBO_TRY(sbo_ensure_exact(ctx, ctx->pp_v, mv)); SBO_TRY(sbo_ensure_exact(ctx, ctx->pp_k, kb));
+    SBO_TRY(sbo_ensure_exact(ctx, ctx->amb_cell, sizeof(int2) * (size_t)n_amb));
+    SBO_TRY(sbo_ensure_exact(ctx, ctx->amb_hist, sizeof(int) * 2 * (size_t)ncell));
+    // bucket the list by cell.  The host needs every cell's length to launch it, so the exclusive scan runs there
+    int* hist = (int*)ctx->amb_hist.p; int* cursor = hist + ncell;
+    int2* sorted = (int2*)ctx->amb_cell.p;
+    const int* rkx = (const int*)ctx->amb_rx.p; const int* rkz = (const int*)ctx->amb_rz.p;
+    SBO_CUDA(cudaMemsetAsync(hist, 0, sizeof(int) * (size_t)ncell, ctx->stream));
+    k_cell_hist<<<(unsigned)cdiv(n_amb, 256), 256, 0, ctx->stream>>>(n_amb, list, p, rkx, rkz, hist);
+    SBO_LAUNCH_CHECK();
+    std::vector<int> cnt((size_t)ncell), off((size_t)ncell);
+    SBO_CUDA(cudaMemcpyAsync(cnt.data(), hist, sizeof(int) * (size_t)ncell, cudaMemcpyDeviceToHost, ctx->stream));
+    SBO_CUDA(cudaStreamSynchronize(ctx->stream));
+    long long run = 0;
+    for (long long c = 0; c < ncell; ++c) { off[c] = (int)run; run += cnt[c]; }
+    SBO_CUDA(cudaMemcpyAsync(cursor, off.data(), sizeof(int) * (size_t)ncell, cudaMemcpyHostToDevice, ctx->stream));
+    k_cell_scatter<<<(unsigned)cdiv(n_amb, 256), 256, 0, ctx->stream>>>(n_amb, list, p, rkx, rkz, cursor, sorted);
+    SBO_LAUNCH_CHECK();
+    // outer blocks: rows once; inner blocks: rows for every outer block they have pairs with (empty cells are skipped)
+    const long long no = p.z_outer ? p.nbz : p.nbx, ni = p.z_outer ? p.nbx : p.nbz;
+    long long cells = 0, rows = 0;
+    for (long long o = 0; o < no; ++o) {
+      long long in_block = 0;
+      for (long long i = 0; i < ni; ++i) in_block += cnt[(size_t)(o * ni + i)];
+      if (in_block == 0) continue;
+      const long long b_o = p.z_outer ? p.bz : p.bx, m_o = p.z_outer ? mzd : mx;
+      const long long r0 = o * b_o, len_o = (m_o - r0) < b_o ? (m_o - r0) : b_o;
+      SBO_TRY(posterior_vrows_dev(ctx, len_o, (p.z_outer ? ptz : ptx) + (size_t)r0 * d, (double*)(p.z_outer ? ctx->amb_vz.p : ctx->amb_vx.p)));
+      rows += len_o;
+      for (long long i = 0; i < ni; ++i) {
+        const long long c = o * ni + i;
+        if (cnt[(size_t)c] == 0) continue;
+        const long long b_i = p.z_outer ? p.bx : p.bz, m_i = p.z_outer ? mx : mzd;
+        const long long q0 = i * b_i, len_i = (m_i - q0) < b_i ? (m_i - q0) : b_i;
+        SBO_TRY(posterior_vrows_dev(ctx, len_i, (p.z_outer ? ptx : ptz) + (size_t)q0 * d, (double*)(p.z_outer ? ctx->amb_vx.p : ctx->amb_vz.p)));
+        rows += len_i;
+        const long long x0 = p.z_outer ? q0 : r0, lx = p.z_outer ? len_i : len_o;
+        const long long z0 = p.z_outer ? r0 : q0, lz = p.z_outer ? len_o : len_i;
+        SBO_TRY(launch_refine(ctx, fc, cnt[(size_t)c], sorted + off[(size_t)c], nx, nz, lx, lz, x0, z0,
+                              (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, counts, row_perm));
+        ++cells;
+      }
+    }
+    ctx->refine_cells = cells; ctx->refine_rows = rows;
+  }
   SBO_CUDA(cudaMemcpyAsync(h, ctx->amb_ctr.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
   SBO_CUDA(cudaStreamSynchronize(ctx->stream));
   ps.n_refined_safe = (long long)h[1];
+  if (multi)      // up to tens of GB (C5): the next step's posterior needs them
+    for (DevBuf* b : {&ctx->amb_vx, &ctx->amb_vz, &ctx->amb_cell}) sbo_free(ctx, *b);
   return SBO_OK;
 }
 
@@ -1027,6 +1186,7 @@ int pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const doub
   const long long count = gs.count;
   PairStage& ps = ctx->ps;
   ps = PairStage{};
+  ctx->refine_cells = ctx->refine_rows = 0;
   ps.mode = mode; ps.precision = precision; ps.beta = beta;
   ps.row_doubles = 2 * d + 3 * nc + 1;
   if (mode == SBO_MODE_LIPSCHITZ) {

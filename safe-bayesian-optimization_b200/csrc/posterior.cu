@@ -763,6 +763,13 @@ int posterior_points(sbo_ctx* ctx, int64_t m, const double* x, double* mean, dou
   return SBO_OK;
 }
 
+// device scratch posterior_vrows_dev allocates for m points: pp_m and pp_v (mv_bytes each) and pp_k (k_bytes)
+void posterior_vrows_scratch(const sbo_ctx* ctx, long long m, size_t* mv_bytes, size_t* k_bytes) {
+  const ModelSpec& ms = ctx->ms;
+  *mv_bytes = sizeof(double) * (size_t)ms.G * m;
+  *k_bytes = sizeof(double) * (size_t)ms.G * ms.npad * chunk_points(ctx, ms, m);
+}
+
 // FP64 rows V_i = L_i^-1 K_i(X, p) of m explicit points already on the device (raw coordinates, [m][d] row-major), for
 // the constraints: vout[(G-1)][m][npad].  Used by the FP64 re-evaluation of the split-TF32 fantasy expander.
 int posterior_vrows_dev(sbo_ctx* ctx, long long m, const double* pts_dev, double* vout) {

@@ -51,6 +51,7 @@ class GridEngine:
         for env, opt in (("SBO_FANTASY_VARIANT", "fantasy_variant"), ("SBO_POSTERIOR_VARIANT", "posterior_variant"),
                          ("SBO_FANTASY_GX", "fantasy_gx"), ("SBO_POSTERIOR_CHUNK_MB", "posterior_chunk_mb"),
                          ("SBO_POSTERIOR_FUSED", "posterior_fused"), ("SBO_FANTASY_REFINE", "fantasy_refine"),
+                         ("SBO_FANTASY_REFINE_MB", "fantasy_refine_mb"),
                          ("SBO_POSTERIOR_TABLES", "posterior_tables")):
             if os.environ.get(env):
                 self.set_option(opt, int(os.environ[env]))
@@ -88,6 +89,12 @@ class GridEngine:
     def mem_peak(self, reset=False):
         """High-water mark (bytes) of the device memory of the context's work buffers."""
         return int(self._lib.sbo_mem_peak(self._h, 1 if reset else 0))
+
+    def refine_stats(self):
+        """FP64 refinement of the last pair stage: {"cells": cells of the pass, "fp64_rows": FP64 rows computed} (0/0: none)."""
+        cells, rows = C.c_int64(), C.c_int64()
+        self._ck(self._lib.sbo_refine_stats(self._h, C.byref(cells), C.byref(rows)))
+        return {"cells": int(cells.value), "fp64_rows": int(rows.value)}
 
     def phase_ms(self):
         out = {}
