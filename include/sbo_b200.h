@@ -159,7 +159,8 @@ int sbo_stable_minmax(sbo_ctx* ctx, int n_controlled, int fun_kind, double beta,
  *   x in S, z in Z  (SafeOpt.py:85-88,109-111; GoOSE.py:69-72,99-101).  L[G]: entry idx is used for
  *   constraint idx (the reference passes L_{G-1} for every idx, SafeOpt.py:110).
  * Fantasy mode (north_star, not in the reference): rank-1 posterior update of every constraint GP with
- *   the observation ucb_i(x); z is newly safe if every updated lcb_i(z) >= 0; g(x) = #newly-safe z.
+ *   the observation ucb_i(x); z is newly safe if every updated lcb_i(z) >= 0; g(x) = #newly-safe z.  The fantasy GoOSE
+ *   target is T = {z : some x in S makes z newly safe} (a column OR over the same pairs) and its argmin lcb_0.
  *   precision: FP64 (FP64 tensor cores: DMMA mma.sync.m8n8k4.f64 tiles), TF32 (tcgen05/TMEM GEMM, FP32 accumulate) or TF32X3
  *   (same kernel over split operands: x_hi.z_hi + x_hi.z_lo + x_lo.z_hi).
  */
@@ -170,16 +171,25 @@ typedef struct sbo_pair_result {
   int64_t pairs_algorithmic;                     /* n_x * n_z * (constraints)         */
   int64_t pairs_evaluated;                       /* after tile-level early exit       */
   int64_t n_hit;                                 /* |expander set| (union over idx) or |target set| */
-  int64_t n_ambiguous, n_refined_safe;           /* fantasy TF32/TF32X3: pairs inside the error bound (re-evaluated in FP64 unless bounds mode) / of those, newly safe */
+  int64_t n_ambiguous, n_refined_safe;           /* fantasy TF32/TF32X3: pairs inside the error bound (re-evaluated in FP64 unless bounds mode) / of those, newly safe;
+                                                    GoOSE target: n_refined_safe = unsafe points the FP64 pass added to T (points, not pairs) */
   /* bounds mode ("fantasy_refine" = 3): n_hit counts the candidates with at least one pair SETTLED newly safe (certified members of the
    * FP64 expander set); n_undecided the candidates with no settled pair but at least one pair inside the error bound (the FP64 set is
    * the certified set plus a subset of these); undecided_best_* = argmax var_0 over them (-1 if none).  The reported x_new (best_idx)
-   * equals the FP64 one whenever undecided_best_value < best_value.  counts[] then holds the settled counts, -1 for undecided candidates. */
+   * equals the FP64 one whenever undecided_best_value < best_value.  counts[] then holds the settled counts, -1 for undecided candidates.
+   * GoOSE target: n_hit = |certified T| (z with a pair the bound settles as safe); n_undecided = the z not certified with at least one pair
+   * inside the bound; undecided_best_* = argmin lcb_0 over them.  The FP64 T is the certified set plus a subset of the undecided z, so
+   * best_idx is the FP64 target whenever undecided_best_value > best_value. */
   int64_t n_undecided, undecided_best_idx; double undecided_best_value;
 } sbo_pair_result;
 int sbo_expander(sbo_ctx* ctx, int mode, int precision, double beta, const double* L /* G, lipschitz mode */,
                  sbo_pair_result* out, int32_t* counts /* count, fantasy mode, or NULL */);
 int sbo_goose_target(sbo_ctx* ctx, double beta, const double* L /* G */, sbo_pair_result* out);
+/* GoOSE target in either pair test: sbo_goose_target is the Lipschitz case.  Fantasy mode needs sbo_posterior with keep_v as for
+ * sbo_expander; the target mask is SBO_MASK_TARGET, which = 0, and the precisions and "fantasy_refine" modes mean what they mean for
+ * the expander (fantasy_refine = 2: the TF32 / TF32X3 target set is the FP64 one). */
+int sbo_goose_target_ex(sbo_ctx* ctx, int mode, int precision, double beta, const double* L /* G, lipschitz mode */,
+                        sbo_pair_result* out);
 /* ---- the same pair stage in five steps, for a grid sharded over ranks (SURVEY.md section 8e) ---------------
  * Every rank pairs ALL candidates x in S (gathered from all ranks) with ITS OWN unsafe points z:
  *   sbo_pairs_prepare     compact the local S and Z, build the local z-side operands
@@ -188,7 +198,8 @@ int sbo_goose_target(sbo_ctx* ctx, double beta, const double* L /* G */, sbo_pai
  *                         candidate) into caller-owned DEVICE buffers  -> all-gather them (NCCL)
  *   sbo_pairs_import_dev  hand the concatenation of all ranks' rows back (n_total candidates)
  *   sbo_pairs_run_dev     result_dev: lipschitz uint8[(G-1)*n_total] hit flags | fantasy int32[n_total] counts
- *                         (goose: uint8[(G-1)*n_z_local], no exchange needed) -> all-reduce max / sum (NCCL)
+ *                         (goose: lipschitz uint8[(G-1)*n_z_local] | fantasy uint32[ceil(n_z_local/32)] hit words over the
+ *                         prepared, key-sorted unsafe slots; no exchange needed) -> all-reduce max / sum (NCCL)
  *   sbo_pairs_finish_dev  masks + arg-reductions on the local shard; the local candidates are rows
  *                         [offset, offset + n_x_local) of the reduced result.  `out` holds LOCAL optima with
  *                         GLOBAL indices; the caller reduces them across ranks (value, then lowest index).
@@ -213,7 +224,7 @@ int sbo_pairs_finish_dev(sbo_ctx* ctx, int goose, int64_t offset, const void* re
 int sbo_pairs_set_segments(sbo_ctx* ctx, int nranks, int rank, const int64_t* n_per_rank);
 int sbo_mask_export_dev(sbo_ctx* ctx, int mask_kind, int which, void* dst_dev, int64_t dst_words);
 int sbo_pairs_set_global_unsafe_dev(sbo_ctx* ctx, const void* gathered_words_dev, int64_t words_per_rank, int nranks);
-/* which = idx-1 (lipschitz/target: one mask per constraint) ; fantasy: which = 0 */
+/* which = idx-1 (lipschitz/target: one mask per constraint) ; fantasy (expander and target): which = 0 */
 #define SBO_MASK_EXPANDER 4
 #define SBO_MASK_TARGET   5
 
@@ -240,6 +251,11 @@ int sbo_comm_destroy(sbo_ctx* ctx);
 int sbo_safeopt_step_sharded(sbo_ctx* ctx, double beta, int mode, int precision, int unsafe_rule, const double* L /* G or NULL */,
                              sbo_step_result* out);
 int sbo_goose_step_sharded(sbo_ctx* ctx, double beta, int unsafe_rule, const double* L /* G or NULL */, sbo_step_result* out);
+/* the GoOSE step in either pair test (sbo_goose_step_sharded is the Lipschitz case).  Fantasy mode: the posterior keeps the V rows of
+ * `precision` and computes no gradient (L is ignored); every rank pairs all candidates with its own unsafe points, so the target set
+ * needs no result collective. */
+int sbo_goose_step_sharded_ex(sbo_ctx* ctx, double beta, int mode, int precision, int unsafe_rule, const double* L /* G or NULL */,
+                              sbo_step_result* out);
 
 /* ---- instrumentation ------------------------------------------------------------------------ */
 /* number of kernels this library launched on ctx since the last reset */
@@ -268,7 +284,7 @@ int sbo_refine_stats(sbo_ctx* ctx, int64_t* cells, int64_t* fp64_rows);
  *                        Cauchy-Schwarz keys of csrc/pairs.cu (k_key_x / k_key_z) and only tile pairs whose keys can meet
  *                        are evaluated; FP64 counts are unchanged | 0: every pair goes through the GEMM
  *   "prior_mean_zero"    1: zero prior mean for every GP at the next sbo_set_model (GP_Robust.py, StableOpt) | 0 (default) GP_Safe.py:331
- *   "fantasy_refine"     2 (default): the TF32 and TF32X3 fantasy expanders settle every pair inside their error bound in FP64
+ *   "fantasy_refine"     2 (default): the TF32 and TF32X3 fantasy expanders and GoOSE targets settle every pair inside their error bound in FP64
  *                        (the counts are the FP64 counts, at any grid size where the ambiguous pairs fit the list: fewer than 2^31
  *                        per shard) | 1: TF32X3 only | 0: decide on the tensor-core value
  *                        | 3: bounds mode -- no FP64 pass: the counts are the pairs the error bound settles as newly safe (a lower bound

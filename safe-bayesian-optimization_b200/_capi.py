@@ -84,6 +84,7 @@ SIGNATURES = {
     "sbo_argreduce": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _D, _I64, _D]),
     "sbo_expander": (C.c_int, [_P, C.c_int, C.c_int, C.c_double, _D, C.POINTER(PairResult), C.POINTER(C.c_int32)]),
     "sbo_goose_target": (C.c_int, [_P, C.c_double, _D, C.POINTER(PairResult)]),
+    "sbo_goose_target_ex": (C.c_int, [_P, C.c_int, C.c_int, C.c_double, _D, C.POINTER(PairResult)]),
     "sbo_set_shard_cyclic": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, _I64]),
     "sbo_pairs_prepare": (C.c_int, [_P, C.c_int, C.c_int, C.c_double, _D, C.POINTER(PairsInfo)]),
     "sbo_pairs_export_dev": (C.c_int, [_P, _P, _P]),
@@ -98,6 +99,7 @@ SIGNATURES = {
     "sbo_comm_destroy": (C.c_int, [_P]),
     "sbo_safeopt_step_sharded": (C.c_int, [_P, C.c_double, C.c_int, C.c_int, C.c_int, _D, C.POINTER(StepResult)]),
     "sbo_goose_step_sharded": (C.c_int, [_P, C.c_double, C.c_int, _D, C.POINTER(StepResult)]),
+    "sbo_goose_step_sharded_ex": (C.c_int, [_P, C.c_double, C.c_int, C.c_int, C.c_int, _D, C.POINTER(StepResult)]),
     "sbo_kernel_launches": (C.c_int64, [_P, C.c_int]),
     "sbo_mem_peak": (C.c_int64, [_P, C.c_int]),
     "sbo_phase_ms": (C.c_int, [_P, C.c_int, _D]),

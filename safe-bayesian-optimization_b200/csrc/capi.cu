@@ -105,7 +105,7 @@ int sbo_destroy(sbo_ctx* ctx) {
                     &ctx->kx, &ctx->lmax, &ctx->vall, &ctx->tile_bb, &ctx->nll_K, &ctx->nll_in, &ctx->m_safe, &ctx->m_unsafe, &ctx->m_min, &ctx->m_user, &ctx->m_exp,
                     &ctx->m_tgt, &ctx->partials, &ctx->result, &ctx->scan_a, &ctx->scan_b, &ctx->xs_idx, &ctx->zs_idx,
                     &ctx->xs_pay, &ctx->zs_pay, &ctx->hits, &ctx->counts, &ctx->pairctr, &ctx->imp_rows, &ctx->vx, &ctx->vz,
-                    &ctx->aux_x, &ctx->aux_z, &ctx->pp_x, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->pp_g, &ctx->tc_row, &ctx->tc_col, &ctx->tc_err, &ctx->exp_rows, &ctx->exp_v, &ctx->key_x, &ctx->key_z, &ctx->perm_x, &ctx->perm_z, &ctx->sort_ws, &ctx->tile_keys, &ctx->item_mask, &ctx->item_list, &ctx->gz_mask, &ctx->gz_idx, &ctx->gz_pay, &ctx->st_score, &ctx->st_mask, &ctx->tabs, &ctx->tc_stats, &ctx->amb_list, &ctx->amb_ctr, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts, &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_rows, &ctx->m_und, &ctx->amb_cell, &ctx->amb_hist})
+                    &ctx->aux_x, &ctx->aux_z, &ctx->pp_x, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->pp_g, &ctx->tc_row, &ctx->tc_col, &ctx->tc_err, &ctx->exp_rows, &ctx->exp_v, &ctx->key_x, &ctx->key_z, &ctx->perm_x, &ctx->perm_z, &ctx->sort_ws, &ctx->tile_keys, &ctx->item_mask, &ctx->item_list, &ctx->gz_mask, &ctx->gz_idx, &ctx->gz_pay, &ctx->st_score, &ctx->st_mask, &ctx->tabs, &ctx->tc_stats, &ctx->amb_list, &ctx->amb_ctr, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts, &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_rows, &ctx->m_und, &ctx->amb_cell, &ctx->amb_hist, &ctx->amb_tgt})
     free_buf(*b);
   ev_collect(ctx);
   for (cudaEvent_t e : ctx->evpool) cudaEventDestroy(e);
@@ -353,8 +353,14 @@ int sbo_expander(sbo_ctx* ctx, int mode, int precision, double beta, const doubl
 }
 
 int sbo_goose_target(sbo_ctx* ctx, double beta, const double* L, sbo_pair_result* out) {
+  return sbo_goose_target_ex(ctx, SBO_MODE_LIPSCHITZ, SBO_PREC_FP64, beta, L, out);
+}
+
+int sbo_goose_target_ex(sbo_ctx* ctx, int mode, int precision, double beta, const double* L, sbo_pair_result* out) {
   ENTER();
-  return pairs_lipschitz(ctx, true, beta, L, out);
+  if (mode == SBO_MODE_LIPSCHITZ) return pairs_lipschitz(ctx, true, beta, L, out);
+  if (mode == SBO_MODE_FANTASY) return pairs_goose_fantasy(ctx, precision, beta, out);
+  return sbo_fail(ctx, SBO_ERR_INVALID, "bad target mode");
 }
 
 int sbo_pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const double* L, sbo_pairs_info* info) {
@@ -453,7 +459,7 @@ int sbo_release(sbo_ctx* ctx, int what) {
     for (DevBuf* b : {&ctx->vx, &ctx->vz, &ctx->exp_v, &ctx->tc_row, &ctx->tc_col, &ctx->imp_rows}) { ctx->mem_now -= (int64_t)b->cap; free_buf(*b); }
     // workspaces of the FP64 refinement: the ambiguous-pair list, its points, rank maps, buckets and FP64 rows
     for (DevBuf* b : {&ctx->amb_list, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts,
-                      &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_cell, &ctx->amb_hist})
+                      &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_cell, &ctx->amb_hist, &ctx->amb_tgt})
       sbo_free(ctx, *b);
     ctx->ps = PairStage{};
   }

@@ -7,7 +7,8 @@
 //                reduced on the host: best value, lowest index on ties -> every rank gets the same answer
 //   broadcast    (grouped, one per rank) candidate rows / V rows written straight into the gathered buffer
 //   all-gather   unsafe bitmask (Lipschitz SafeOpt expander: N/8 bytes in total)
-//   all-reduce   per-candidate hit flags (max) / newly-safe counts (sum)
+//   all-reduce   per-candidate hit flags (max) / newly-safe counts (sum); none for the fantasy GoOSE target, whose
+//                verdict on an unsafe point is local (every rank pairs all candidates with its own unsafe points)
 // Decision rules: test/test_SafeOpt.py:144-158 and test/test_GoOSE.py:151-162 of the reference.
 #include "common.cuh"
 #include <dlfcn.h>
@@ -161,7 +162,7 @@ static int sharded_pairs(sbo_ctx* ctx, int mode, int precision, bool goose, doub
   // (4) run on the local shard, combine the per-candidate results
   const long long nzg = ctx->ps.nz_global;                     // >= 0: the pair stage runs over the all-gathered unsafe set
   const bool goose_global = goose && nzg >= 0;
-  const size_t res_b = fantasy ? sizeof(int) * (size_t)n_total
+  const size_t res_b = fantasy ? (goose ? sizeof(uint32_t) * (size_t)cdiv(info.n_z_local, 32) : sizeof(int) * (size_t)n_total)
                                : (size_t)nc * (size_t)(goose ? (goose_global ? nzg : info.n_z_local) : n_total);
   SBO_TRY(sbo_ensure(ctx, cm->result, (res_b ? res_b : 16) + (goose_global ? (size_t)nc * info.n_z_local + 16 : 0)));
   SBO_TRY(pairs_run(ctx, goose ? 1 : 0, cm->result.p));
@@ -205,7 +206,7 @@ static int sharded_pairs(sbo_ctx* ctx, int mode, int precision, bool goose, doub
     pr->n_hit += (int64_t)g[(size_t)r * nrec + 2 * SBO_MAX_G]; pr->pairs_evaluated += (int64_t)g[(size_t)r * nrec + 2 * SBO_MAX_G + 1];
     pr->n_ambiguous += (int64_t)g[(size_t)r * nrec + 2 * SBO_MAX_G + 2]; pr->n_refined_safe += (int64_t)g[(size_t)r * nrec + 2 * SBO_MAX_G + 3];
   }
-  reduce_arg(g, nrec, R, 2 * SBO_MAX_G + 4, true, &pr->undecided_best_value, &pr->undecided_best_idx);
+  reduce_arg(g, nrec, R, 2 * SBO_MAX_G + 4, !goose, &pr->undecided_best_value, &pr->undecided_best_idx);   // GoOSE: min lcb_0
   for (int r = 0; r < R; ++r) pr->n_undecided += (int64_t)g[(size_t)r * nrec + 2 * SBO_MAX_G + 6];
   pr->n_x = n_total; pr->n_z = nz_total; pr->pairs_algorithmic = n_total * nz_total * nc;
   if (big) SBO_TRY(sbo_release(ctx, 2));
@@ -305,16 +306,24 @@ int sbo_safeopt_step_sharded(sbo_ctx* ctx, double beta, int mode, int precision,
 }
 
 int sbo_goose_step_sharded(sbo_ctx* ctx, double beta, int unsafe_rule, const double* L, sbo_step_result* out) {
+  return sbo_goose_step_sharded_ex(ctx, beta, SBO_MODE_LIPSCHITZ, SBO_PREC_FP64, unsafe_rule, L, out);
+}
+
+int sbo_goose_step_sharded_ex(sbo_ctx* ctx, double beta, int mode, int precision, int unsafe_rule, const double* L, sbo_step_result* out) {
   if (!ctx) return sbo_fail(nullptr, SBO_ERR_INVALID, "null context");
   cudaSetDevice(ctx->device);
   SBO_REQUIRE(ctx->comm != nullptr, "sbo_goose_step_sharded: call sbo_comm_init first");
   SBO_REQUIRE(out != nullptr, "null result");
+  SBO_REQUIRE(mode == SBO_MODE_LIPSCHITZ || mode == SBO_MODE_FANTASY, "bad target mode");
   memset(out, 0, sizeof(*out));
   const int G = ctx->ms.G;
-  SBO_TRY(sharded_sets(ctx, beta, unsafe_rule, L ? 0 : 1, 0, nullptr, out));
+  const bool fantasy = mode == SBO_MODE_FANTASY;
+  // fantasy: V rows kept at the GEMM's precision and no gradient, as in sbo_safeopt_step_sharded
+  const int keep_v = fantasy ? (precision == SBO_PREC_FP64 ? 1 : (precision == SBO_PREC_TF32 ? 2 : 3)) : 0;
+  SBO_TRY(sharded_sets(ctx, beta, unsafe_rule, (!fantasy && !L) ? 1 : 0, keep_v, nullptr, out));
   double Lg[SBO_MAX_G];
   for (int i = 0; i < SBO_MAX_G; ++i) Lg[i] = L ? (i < G ? L[i] : 0.0) : out->L[G - 1];   // GoOSE.py:100
-  SBO_TRY(sharded_pairs(ctx, SBO_MODE_LIPSCHITZ, SBO_PREC_FP64, true, beta, Lg, &out->pairs));
+  SBO_TRY(sharded_pairs(ctx, mode, fantasy ? precision : SBO_PREC_FP64, true, beta, fantasy ? nullptr : Lg, &out->pairs));
   out->explore_idx = -1;
   if (out->sets.min_lcb0 <= out->pairs.best_value || out->pairs.best_idx < 0) {        // test_GoOSE.py:158-162
     out->x_new_idx = out->sets.min_lcb0_idx;

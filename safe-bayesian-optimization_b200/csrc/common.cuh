@@ -167,6 +167,7 @@ struct sbo_ctx {
   DevBuf key_x, key_z, perm_x, perm_z, sort_ws, tile_keys, item_mask, item_list;   // exact pruning of the fantasy expander
   DevBuf amb_list, amb_ctr, amb_mask, amb_xd, amb_zd, amb_rx, amb_rz, amb_pts, amb_vx, amb_vz, amb_rows, m_und;   // FP64 refinement of the split-TF32 expander
   DevBuf amb_cell, amb_hist;              // cell-wise refinement: the ambiguous list bucketed by cell, per-cell counters
+  DevBuf amb_tgt;                         // GoOSE target refinement: the listed pairs whose z is not yet in the target set
   int64_t refine_cells = 0, refine_rows = 0;   // last pair stage: cells of the FP64 refinement and FP64 rows computed (sbo_refine_stats)
   DevBuf st_score, st_mask;               // StableOpt: per-x_c worst-case score and robust-safe bitmask
   DevBuf gz_mask, gz_idx, gz_pay;         // all-gathered unsafe set of a sharded Lipschitz expander
@@ -263,5 +264,6 @@ int pairs_goose_localize(sbo_ctx* ctx, const void* hits_global, void* hits_local
 int pairs_set_global_unsafe(sbo_ctx* ctx, const void* gathered_words_dev, long long words_per_rank, int nranks);
 int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_dev, sbo_pair_result* out, int32_t* counts_host);
 int pairs_fantasy(sbo_ctx* ctx, int precision, double beta, sbo_pair_result* out, int32_t* counts_host);
+int pairs_goose_fantasy(sbo_ctx* ctx, int precision, double beta, sbo_pair_result* out);
 uint32_t* mask_ptr(sbo_ctx* ctx, int mask_kind, int which);
 long long mask_words(const sbo_ctx* ctx);

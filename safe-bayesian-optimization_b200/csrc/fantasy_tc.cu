@@ -49,6 +49,10 @@ struct Params {
   long long amb_cap;
   int* amb_rows;                   // bounds mode (fantasy_refine = 3): per-candidate number of ambiguous pairs, no list
   float e_abs, d_mu, d_t;          // absolute error terms of the FP32 epilogue (covariance, mean, variance side)
+  // GoOSE target (2-CTA kernel only; counts unused): bit z of hit_words is set when some valid candidate row makes column z
+  // safe; bounds mode sets bit z of amb_words instead of amb_rows when column z has a pair inside the error bound
+  uint32_t* hit_words;
+  uint32_t* amb_words;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -591,7 +595,7 @@ __device__ __forceinline__ bool item_coords2(const Params& p, long long item, in
   return xt < p.nxt;
 }
 
-template <int D4, int EW, bool REFINE>
+template <int D4, int EW, bool REFINE, bool TARGET>   // TARGET: GoOSE target epilogue (column OR, p.hit_words)
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
 k_fantasy_tc2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const Params p) {
   using C = Cfg2<D4>;
@@ -786,11 +790,30 @@ k_fantasy_tc2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         if (++slot == SLOTS) { slot = 0; sphase ^= 1; }
         if (++b == 2) { b = 0; bphase ^= 1; }
       }
-      int cnt = 0;
+      if (TARGET) {
+        // GoOSE target: column OR over the warp's 32 candidate rows, one atomicOr per 32-column word.  Padded rows and
+        // columns are zero operands and must never set a bit, so rows >= nx and columns >= nz are masked first.
+        const bool row_ok = xrow < p.nx;
 #pragma unroll
-      for (int h = 0; h < NCH; ++h) cnt += __popc(bits[h]);
-      if (xrow < p.nx && cnt) atomicAdd(p.counts + (p.row_perm ? p.row_perm[xrow] : xrow), cnt);
-      if (REFINE && xrow < p.nx) {
+        for (int h = 0; h < NCH; ++h) {
+          const long long zc0 = (long long)zt * BN + (half * NCH + h) * 32;
+          const uint32_t cm = zc0 + 32 <= p.nz ? 0xffffffffu : (zc0 >= p.nz ? 0u : (1u << (int)(p.nz - zc0)) - 1u);
+          const uint32_t hw = __reduce_or_sync(0xffffffffu, row_ok ? bits[h] & cm : 0u);
+          if (lane == 0 && hw) atomicOr(p.hit_words + (zc0 >> 5), hw);
+          if (REFINE && p.amb_words) {
+            const uint32_t amb = row_ok ? ~bits[h] & ~ubits[h] & cm : 0u;
+            const uint32_t aw = __reduce_or_sync(0xffffffffu, amb);
+            if (amb) atomicAdd(p.amb_count, (unsigned long long)__popc(amb));
+            if (lane == 0 && aw) atomicOr(p.amb_words + (zc0 >> 5), aw);
+          }
+        }
+      } else {
+        int cnt = 0;
+#pragma unroll
+        for (int h = 0; h < NCH; ++h) cnt += __popc(bits[h]);
+        if (xrow < p.nx && cnt) atomicAdd(p.counts + (p.row_perm ? p.row_perm[xrow] : xrow), cnt);
+      }
+      if (REFINE && xrow < p.nx && !(TARGET && p.amb_words)) {
 #pragma unroll
         for (int h = 0; h < NCH; ++h) {
           uint32_t amb = ~bits[h] & ~ubits[h];              // neither settled safe nor settled unsafe
@@ -938,9 +961,9 @@ static int launch(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx
   return SBO_OK;
 }
 
-struct RefineArgs { int2* list; unsigned long long* count; long long cap; float e_abs, d_mu, d_t; int* rows; };
+struct RefineArgs { int2* list; unsigned long long* count; long long cap; float e_abs, d_mu, d_t; int* rows; uint32_t* hit_words; uint32_t* amb_words; };
 
-template <int D4, int EW, bool REFINE>
+template <int D4, int EW, bool REFINE, bool TARGET>
 static int launch2(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx, long long nz, long long nxp, long long nzp,
                    const float* Vx, const float* Vz, const float* rowrec, const float* colrec, int* counts, int* err,
                    const long long* item_list, long long n_list, const int* row_perm, int gx, const RefineArgs& ra) {
@@ -963,19 +986,22 @@ static int launch2(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   p.sched_counter = (unsigned int*)(err + 1);
   p.item_list = item_list; p.row_perm = row_perm;
   p.amb_list = ra.list; p.amb_count = ra.count; p.amb_cap = ra.cap; p.amb_rows = ra.rows; p.e_abs = ra.e_abs; p.d_mu = ra.d_mu; p.d_t = ra.d_t;
+  p.hit_words = ra.hit_words; p.amb_words = ra.amb_words;
   if (p.n_items == 0) return SBO_OK;
-  SBO_CUDA((cudaFuncSetAttribute(k_fantasy_tc2<D4, EW, REFINE>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES)));
+  SBO_CUDA((cudaFuncSetAttribute(k_fantasy_tc2<D4, EW, REFINE, TARGET>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES)));
   const int grid = 2 * (int)((p.n_items < clusters) ? p.n_items : clusters);
-  k_fantasy_tc2<D4, EW, REFINE><<<grid, 128 + 32 * EW, C::SMEM_BYTES, ctx->stream>>>(tmA, tmB, p);
+  k_fantasy_tc2<D4, EW, REFINE, TARGET><<<grid, 128 + 32 * EW, C::SMEM_BYTES, ctx->stream>>>(tmA, tmB, p);
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }
 
 }  // namespace tc
 
-// keys of the exact pruning (pairs.cu): sorted key_x[nx] (max side), key_z[nz] (min side), slot -> counts row
+// keys of the exact pruning (pairs.cu): sorted key_x[nx] (max side), key_z[nz] (min side), slot -> counts row;
+// hit_words != null: GoOSE target (column OR into hit_words over the z slots; bounds mode: amb_words instead of amb_rows)
 struct FantasyPruneArgs { const double* key_x; const double* key_z; const int* row_perm; long long* items_run;
-                          int refine; int2* amb_list; unsigned long long* amb_count; long long amb_cap; int* amb_rows; };
+                          int refine; int2* amb_list; unsigned long long* amb_count; long long amb_cap; int* amb_rows;
+                          uint32_t* hit_words; uint32_t* amb_words; };
 // per tile of `tile` consecutive sorted entries: max (x side) or min (z side) of the keys
 __global__ void __launch_bounds__(256)
 k_tile_keys(long long n, int tile, int want_max, const double* __restrict__ key, double* __restrict__ out) {
@@ -1052,9 +1078,11 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   const double c1 = refine ? ((split ? 9.5367431640625e-07 : 9.7680091857910156e-04) + (fc.npad / 8) * 1.1920928955078125e-07) : 0.0;
   const double esc = refine ? sqrt(c1) : 0.0;
   tc::RefineArgs ra{};
+  const bool target = pr && pr->hit_words;
+  ra.hit_words = target ? pr->hit_words : nullptr;
   unsigned long long* stats = nullptr;
   if (refine) {
-    ra.list = pr->amb_list; ra.count = pr->amb_count; ra.cap = pr->amb_cap; ra.rows = pr->amb_rows;
+    ra.list = pr->amb_list; ra.count = pr->amb_count; ra.cap = pr->amb_cap; ra.rows = pr->amb_rows; ra.amb_words = pr->amb_words;
     SBO_TRY(sbo_ensure(ctx, ctx->tc_stats, 4 * sizeof(unsigned long long)));
     stats = (unsigned long long*)ctx->tc_stats.p;
     SBO_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), ctx->stream));
@@ -1095,6 +1123,7 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   int variant = (int)ctx->opt_fantasy_variant;
   if (variant < 0) variant = 5 | ((fc.npad <= 256 || D4 == 2) ? 2 : 0);
   if (refine) variant |= 7;        // the refining epilogue exists in the 2-CTA kernel only; it is heavier: 8 epilogue warps
+  if (target) variant |= 4;        // so does the column-OR epilogue of the GoOSE target
   // tile geometry of the chosen kernel and the raster of its work items
   const bool two = (variant & 4) != 0;
   const int tile_x = two ? 2 * tc::BM : tc::BM, tile_z = (two || (variant & 1)) ? 256 : 128;
@@ -1113,8 +1142,9 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   ev_end(ctx);            // record prep = phase 6
   ev_begin(ctx, 4);       // the GEMM kernel alone = phase 4 (closed by the caller)
 #define TC_LAUNCH(BN_, D4_, EW_) SBO_TRY((tc::launch<BN_, D4_, EW_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm)))
-#define TC_LAUNCH2(D4_, EW_) do { if (refine) SBO_TRY((tc::launch2<D4_, EW_, true>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm, gx, ra))); \
-                                 else SBO_TRY((tc::launch2<D4_, EW_, false>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm, gx, ra))); } while (0)
+#define TC_LAUNCH2R(D4_, EW_, R_, T_) SBO_TRY((tc::launch2<D4_, EW_, R_, T_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm, gx, ra)))
+#define TC_LAUNCH2(D4_, EW_) do { if (target) { if (refine) TC_LAUNCH2R(D4_, EW_, true, true); else TC_LAUNCH2R(D4_, EW_, false, true); } \
+                                  else if (refine) TC_LAUNCH2R(D4_, EW_, true, false); else TC_LAUNCH2R(D4_, EW_, false, false); } while (0)
   if (variant & 4) {            // 2-CTA pairs (cta_group::2), BN = 256
     if (D4 == 1) { if (variant & 2) TC_LAUNCH2(1, 8); else TC_LAUNCH2(1, 4); }
     else         { if (variant & 2) TC_LAUNCH2(2, 8); else TC_LAUNCH2(2, 4); }
@@ -1134,6 +1164,7 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
     }
   }
 #undef TC_LAUNCH2
+#undef TC_LAUNCH2R
 #undef TC_LAUNCH
   return SBO_OK;
 }

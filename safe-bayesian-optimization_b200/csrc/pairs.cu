@@ -620,17 +620,18 @@ k_union_count(int nc, const uint32_t* __restrict__ masks, long long nwords, unsi
 // =============================================================================================
 #define FB 64
 #define FK 16
-template <int D>
+template <int D, bool TARGET>   // TARGET: GoOSE target epilogue (column OR into hit_words)
 __global__ void __launch_bounds__(256)
 k_fantasy_f64(FantasyConsts fc, long long nx, long long nz, long long nxp, long long nzp,
               const double* __restrict__ Vx, const double* __restrict__ Vz,
               const double* __restrict__ xn, const double* __restrict__ ax, const double* __restrict__ bx,
               const double* __restrict__ zn, const double* __restrict__ mz, const double* __restrict__ sz,
               int* __restrict__ counts, const double* __restrict__ key_x, const double* __restrict__ key_z,
-              const int* __restrict__ row_perm, unsigned long long* __restrict__ pair_counter) {
+              const int* __restrict__ row_perm, unsigned long long* __restrict__ pair_counter, uint32_t* __restrict__ hit_words) {
   __shared__ double As[FK][FB + 1];   // z rows
   __shared__ double Bs[FK][FB + 1];   // x rows
   __shared__ int cnt[16][FB];
+  __shared__ uint32_t hw[FB / 32];    // GoOSE target: the block's z rows made safe by some valid x column
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
   const long long zb = (long long)blockIdx.x * FB, xb = (long long)blockIdx.y * FB;
   if (key_x) {   // exact pruning (see k_key_z): no pair of this block can become safe when min key_z > max key_x
@@ -650,6 +651,7 @@ k_fantasy_f64(FantasyConsts fc, long long nx, long long nz, long long nxp, long 
     if (!reach) return;
   }
   if (tid == 0 && pair_counter) atomicAdd(pair_counter, (unsigned long long)FB * FB);
+  if (TARGET && tid < FB / 32) hw[tid] = 0u;
   const int np = fc.npad;
   unsigned okmask = 0xffffu;   // bit i*4+j
   double zc[4][D], xc[4][D];
@@ -712,6 +714,20 @@ k_fantasy_f64(FantasyConsts fc, long long nx, long long nz, long long nxp, long 
       }
     }
   }
+  if (TARGET) {   // GoOSE target: OR over the valid x columns of every valid z row
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int r = ty * 4 + i;
+      bool any = false;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) any |= xb + tx * 4 + j < nx && ((okmask >> (i * 4 + j)) & 1u);
+      if (any && zb + r < nz) atomicOr(hw + (r >> 5), 1u << (r & 31));
+    }
+    __syncthreads();
+    if (tid < FB / 32 && hw[tid]) atomicOr(hit_words + (zb >> 5) + tid, hw[tid]);
+    return;
+  }
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     int cj = 0;
@@ -757,6 +773,7 @@ struct DmmaArgs {
   int* counts;
   const int* row_perm;
   const long long* item_list;
+  uint32_t* hit_words;          // GoOSE target: column OR over the candidates instead of counts
 };
 
 __device__ __forceinline__ void fd_cp16(void* smem, const void* gmem) {
@@ -767,7 +784,7 @@ __device__ __forceinline__ void fd_dmma(double& c0, double& c1, double a, double
                : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
-template <int D>
+template <int D, bool TARGET>   // TARGET: GoOSE target epilogue (column OR into a.hit_words)
 __global__ void __launch_bounds__(256, 2)
 k_fantasy_dmma(FantasyConsts fc, DmmaArgs a) {
   extern __shared__ __align__(16) double fsm[];
@@ -873,6 +890,22 @@ k_fantasy_dmma(FantasyConsts fc, DmmaArgs a) {
         }
     }
   }
+  if (TARGET) {
+    // GoOSE target: the warp's 32 z columns zb + wp*32 + (j*8 + 2*tig + e), OR over its valid x rows, one word per warp
+    uint32_t w = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      if (xb + wr * 32 + i * 8 + grp >= a.nx) continue;
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+#pragma unroll
+        for (int e = 0; e < 2; ++e)
+          if (((okbits >> ((i * 4 + j) * 2 + e)) & 1u) && zb + wp * 32 + j * 8 + 2 * tig + e < a.nz) w |= 1u << (j * 8 + 2 * tig + e);
+    }
+    w = __reduce_or_sync(0xffffffffu, w);
+    if (lane == 0 && w) atomicOr(a.hit_words + ((zb + wp * 32) >> 5), w);
+    return;
+  }
   // per candidate: newly-safe z of this tile = set bits of its row over valid columns, summed over the 4 lanes of a
   // quad (tig) here and over the two column warps by the atomics
 #pragma unroll
@@ -894,7 +927,8 @@ int fantasy_build_items(sbo_ctx* ctx, long long nx, long long nz, int tile_x, in
                         const double* key_z, const long long** item_list, long long* n_list);
 
 struct FantasyPruneArgs { const double* key_x; const double* key_z; const int* row_perm; long long* items_run;
-                          int refine; int2* amb_list; unsigned long long* amb_count; long long amb_cap; int* amb_rows; };
+                          int refine; int2* amb_list; unsigned long long* amb_count; long long amb_cap; int* amb_rows;
+                          uint32_t* hit_words; uint32_t* amb_words; };
 int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx, long long nz, long long nxp,
                    long long nzp, const float* Vx, const float* Vz, const double* aux_x, const double* aux_z, int* counts_c,
                    const FantasyPruneArgs* pr);
@@ -957,19 +991,23 @@ k_cell_scatter(long long n, const int2* __restrict__ list, CellPlan p, const int
 
 // one warp per ambiguous pair of list[0..n_amb).  Vx / Vz hold the FP64 rows of the ranks [x0, x0 + mx) / [z0, z0 + mz_)
 // (one cell: all ranks, offsets 0)
-template <int D>
+template <int D, bool TARGET>   // TARGET: GoOSE target (safe pairs set their z's bit in hit_words)
 __global__ void __launch_bounds__(256)
 k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list, long long nx, long long nz, long long mx, long long mz_,
                long long x0, long long z0, const int* __restrict__ rank_x, const int* __restrict__ rank_z,
                const double* __restrict__ Vx, const double* __restrict__ Vz,
                const double* __restrict__ xn, const double* __restrict__ ax, const double* __restrict__ bx,
                const double* __restrict__ zn, const double* __restrict__ mz, const double* __restrict__ sz,
-               int* __restrict__ counts, const int* __restrict__ row_perm, unsigned long long* __restrict__ n_safe) {
+               int* __restrict__ counts, const int* __restrict__ row_perm, unsigned long long* __restrict__ n_safe,
+               uint32_t* __restrict__ hit_words) {
   const long long w = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (w >= n_amb) return;
   const int lane = threadIdx.x & 31;
   const int2 e = list[w];
   const long long xi = e.x, zi = e.y;
+  const uint32_t zbit = 1u << (zi & 31);
+  // GoOSE target: a pair can only re-confirm a z another pair of this pass already added (warp-uniform skip)
+  if (TARGET && (*(volatile const uint32_t*)(hit_words + (zi >> 5)) & zbit)) return;
   const long long rx = rank_x[xi] - x0, rz = rank_z[zi] - z0;
   bool ok = true;
   for (int c = 0; c < fc.nc && ok; ++c) {
@@ -988,23 +1026,29 @@ k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list,
     ok = (mu - fc.beta * sqrt(fmax(s2, 0.0))) >= 0.0;
   }
   if (ok && lane == 0) {
-    atomicAdd(counts + (row_perm ? row_perm[xi] : xi), 1);
-    atomicAdd(n_safe, 1ULL);
+    if (TARGET) {   // n_safe counts points: exactly one atomicOr sees the bit of a newly added z clear
+      if (!(atomicOr(hit_words + (zi >> 5), zbit) & zbit)) atomicAdd(n_safe, 1ULL);
+    } else {
+      atomicAdd(counts + (row_perm ? row_perm[xi] : xi), 1);
+      atomicAdd(n_safe, 1ULL);
+    }
   }
 }
 
 static int launch_refine(sbo_ctx* ctx, const FantasyConsts& fc, long long n, const int2* list, long long nx, long long nz,
                          long long mx, long long mz_, long long x0, long long z0, const double* Vx, const double* Vz,
-                         int* counts, const int* row_perm) {
+                         int* counts, const int* row_perm, uint32_t* hit_words) {
   const int d = fc.d, nc = fc.nc;
   const double* xn = (const double*)ctx->aux_x.p; const double* ax = xn + (size_t)d * nx; const double* bx = ax + (size_t)nc * nx;
   const double* zn = (const double*)ctx->aux_z.p; const double* mz = zn + (size_t)d * nz; const double* sz = mz + (size_t)nc * nz;
   unsigned long long* nsafe = (unsigned long long*)ctx->amb_ctr.p + 1;
-#define RP(DD) k_refine_pairs<DD><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0, (const int*)ctx->amb_rx.p, \
-      (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe)
+#define RPT(DD, T) k_refine_pairs<DD, T><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0, (const int*)ctx->amb_rx.p, \
+      (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe, hit_words)
+#define RP(DD) do { if (hit_words) RPT(DD, true); else RPT(DD, false); } while (0)
   switch (d) { case 1: RP(1); break; case 2: RP(2); break; case 3: RP(3); break; case 4: RP(4); break;
                case 5: RP(5); break; case 6: RP(6); break; case 7: RP(7); break; default: RP(8); break; }
 #undef RP
+#undef RPT
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }
@@ -1043,14 +1087,27 @@ static bool plan_cells(const sbo_ctx* ctx, long long mx, long long mz, long long
   return false;
 }
 
-static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx, long long nz, int* counts, const int* row_perm) {
+// GoOSE target: the listed pairs whose z is not yet in the target set (the order of the kept pairs is arbitrary)
+__global__ void __launch_bounds__(256) k_amb_filter(long long n, const int2* __restrict__ list, const uint32_t* __restrict__ hit_words,
+                                                    int2* __restrict__ out, unsigned long long* __restrict__ n_out) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const int2 e = list[t];
+  if (!((hit_words[e.y >> 5] >> (e.y & 31)) & 1u)) out[atomicAdd(n_out, 1ULL)] = e;
+}
+
+// counts != null: SafeOpt expander (safe pairs are added to the candidates' counts).  hit_words != null: GoOSE target (safe
+// pairs set their z's bit; the list is first cut to the pairs whose z no settled pair reached, and n_refined_safe counts the
+// unsafe points the pass adds to the target set)
+static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx, long long nz, int* counts, const int* row_perm,
+                            uint32_t* hit_words) {
   PairStage& ps = ctx->ps;
   const ModelSpec& ms = ctx->ms;
   const int d = fc.d, nc = fc.nc;
   unsigned long long h[2] = {0, 0};
   SBO_CUDA(cudaMemcpyAsync(h, ctx->amb_ctr.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
   SBO_CUDA(cudaStreamSynchronize(ctx->stream));
-  const long long n_amb = (long long)h[0];
+  long long n_amb = (long long)h[0];
   const long long cap = (long long)(ctx->amb_list.cap / sizeof(int2));
   ps.n_ambiguous = n_amb; ps.n_refined_safe = 0;
   if (n_amb > cap)
@@ -1058,6 +1115,17 @@ static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx,
                                             std::to_string(cap) + " (use precision fp64, or option fantasy_refine = 0)");
   if (n_amb == 0) return SBO_OK;
   const int2* list = (const int2*)ctx->amb_list.p;
+  if (hit_words) {
+    SBO_TRY(sbo_ensure(ctx, ctx->amb_tgt, sizeof(int2) * (size_t)n_amb));
+    SBO_CUDA(cudaMemsetAsync(ctx->amb_ctr.p, 0, sizeof(unsigned long long), ctx->stream));
+    k_amb_filter<<<(unsigned)cdiv(n_amb, 256), 256, 0, ctx->stream>>>(n_amb, list, hit_words, (int2*)ctx->amb_tgt.p, (unsigned long long*)ctx->amb_ctr.p);
+    SBO_LAUNCH_CHECK();
+    SBO_CUDA(cudaMemcpyAsync(h, ctx->amb_ctr.p, sizeof(h[0]), cudaMemcpyDeviceToHost, ctx->stream));
+    SBO_CUDA(cudaStreamSynchronize(ctx->stream));
+    n_amb = (long long)h[0];
+    list = (const int2*)ctx->amb_tgt.p;
+    if (n_amb == 0) return SBO_OK;
+  }
   const long long wx = cdiv(nx, 32), wz = cdiv(nz, 32);
   SBO_TRY(sbo_ensure(ctx, ctx->amb_mask, sizeof(uint32_t) * (size_t)(wx + wz)));
   SBO_CUDA(cudaMemsetAsync(ctx->amb_mask.p, 0, sizeof(uint32_t) * (size_t)(wx + wz), ctx->stream));
@@ -1101,7 +1169,7 @@ static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx,
     }
     SBO_TRY(posterior_vrows_dev(ctx, mx, ptx, (double*)ctx->amb_vx.p));
     SBO_TRY(posterior_vrows_dev(ctx, mzd, ptz, (double*)ctx->amb_vz.p));
-    SBO_TRY(launch_refine(ctx, fc, n_amb, list, nx, nz, mx, mzd, 0, 0, (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, counts, row_perm));
+    SBO_TRY(launch_refine(ctx, fc, n_amb, list, nx, nz, mx, mzd, 0, 0, (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, counts, row_perm, hit_words));
     ctx->refine_cells = 1; ctx->refine_rows = mx + mzd;
   } else {
     CellPlan p{};
@@ -1155,7 +1223,7 @@ static int refine_ambiguous(sbo_ctx* ctx, const FantasyConsts& fc, long long nx,
         const long long x0 = p.z_outer ? q0 : r0, lx = p.z_outer ? len_i : len_o;
         const long long z0 = p.z_outer ? r0 : q0, lz = p.z_outer ? len_o : len_i;
         SBO_TRY(launch_refine(ctx, fc, cnt[(size_t)c], sorted + off[(size_t)c], nx, nz, lx, lz, x0, z0,
-                              (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, counts, row_perm));
+                              (const double*)ctx->amb_vx.p, (const double*)ctx->amb_vz.p, counts, row_perm, hit_words));
         ++cells;
       }
     }
@@ -1411,11 +1479,11 @@ int pairs_set_global_unsafe(sbo_ctx* ctx, const void* gathered_words_dev, long l
   return SBO_OK;
 }
 
-// result_dev: expander/lipschitz uint8[nc*n_total]; expander/fantasy int32[n_total]; goose: uint8[nc*nz_local]
+// result_dev: expander/lipschitz uint8[nc*n_total]; expander/fantasy int32[n_total]; goose/lipschitz uint8[nc*nz_local];
+// goose/fantasy uint32[ceil(nz_local/32)] hit words over the prepared (key-sorted) z slots
 int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
   PairStage& ps = ctx->ps;
   SBO_REQUIRE(ps.prepared && ps.imported, "sbo_pairs_run: prepare and import first");
-  SBO_REQUIRE(!goose || ps.mode == SBO_MODE_LIPSCHITZ, "the GoOSE target uses the Lipschitz pair test");
   const ModelSpec& ms = ctx->ms;
   const int nc = ms.G - 1, d = ctx->gs.d;
   const long long nx = ps.nx_total, nz = ps.nz_local;
@@ -1423,7 +1491,7 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
   ps.counted = false;
   ps.bounds = false;
   if (nc == 0) return SBO_OK;
-  const size_t res_bytes = (ps.mode == SBO_MODE_FANTASY) ? sizeof(int) * (size_t)nx
+  const size_t res_bytes = (ps.mode == SBO_MODE_FANTASY) ? (goose ? sizeof(uint32_t) * (size_t)cdiv(nz, 32) : sizeof(int) * (size_t)nx)
                                                          : (size_t)nc * (goose ? (ps.nz_global >= 0 ? ps.nz_global : nz) : nx);
   if (res_bytes) {
     SBO_REQUIRE(result_dev != nullptr, "null result buffer");
@@ -1469,7 +1537,8 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
     }
     const long long nxp = cdiv(nx, 256) * 256, nzp = cdiv(nz, 256) * 256;
     const double* zn = (const double*)ctx->aux_z.p; const double* mz = zn + (size_t)d * nz; const double* sz = mz + (size_t)nc * nz;
-    int* cnt = (int*)result_dev;
+    int* cnt = goose ? nullptr : (int*)result_dev;
+    uint32_t* hitw = goose ? (uint32_t*)result_dev : nullptr;    // GoOSE target: column OR instead of per-candidate counts
     const double* key_x = ps.sorted ? (const double*)ctx->key_x.p : nullptr;
     const double* key_z = ps.sorted ? (const double*)ctx->key_z.p : nullptr;
     const int* row_perm = ps.sorted ? (const int*)ctx->perm_x.p : nullptr;
@@ -1480,7 +1549,7 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
       da.nxt = (int)cdiv(nx, FD_BM); da.nzt = (int)cdiv(nz, FD_BN); da.gx = 32;
       da.Vx = (const double*)ctx->vx.p; da.Vz = (const double*)ctx->vz.p;
       da.xn = xn; da.ax = ax; da.bx = bx; da.zn = zn; da.mz = mz; da.sz = sz;
-      da.counts = cnt; da.row_perm = row_perm;
+      da.counts = cnt; da.row_perm = row_perm; da.hit_words = hitw;
       da.n_items = cdiv(da.nxt, da.gx) * da.gx * (long long)da.nzt;
       ev_begin(ctx, 6);
       if (key_x && key_z) SBO_TRY(fantasy_build_items(ctx, nx, nz, FD_BM, FD_BN, da.gx, key_x, key_z, &da.item_list, &da.n_items));
@@ -1490,11 +1559,13 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
       const size_t smem = sizeof(double) * ((size_t)FD_STAGES * FD_STAGE_D + (size_t)(FD_BM + FD_BN) * RC);
       ev_begin(ctx, 4);
       if (da.n_items > 0) {
-#define FDL(DD) do { SBO_CUDA(cudaFuncSetAttribute(k_fantasy_dmma<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-                     k_fantasy_dmma<DD><<<(unsigned)da.n_items, 256, smem, ctx->stream>>>(fc, da); } while (0)
+#define FDLT(DD, T) do { SBO_CUDA(cudaFuncSetAttribute(k_fantasy_dmma<DD, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+                        k_fantasy_dmma<DD, T><<<(unsigned)da.n_items, 256, smem, ctx->stream>>>(fc, da); } while (0)
+#define FDL(DD) do { if (hitw) FDLT(DD, true); else FDLT(DD, false); } while (0)
         switch (d) { case 1: FDL(1); break; case 2: FDL(2); break; case 3: FDL(3); break; case 4: FDL(4); break;
                      case 5: FDL(5); break; case 6: FDL(6); break; case 7: FDL(7); break; default: FDL(8); break; }
 #undef FDL
+#undef FDLT
         SBO_LAUNCH_CHECK();
       }
       ps.pairs_evaluated = da.n_items * (long long)FD_BM * FD_BN * nc;
@@ -1503,28 +1574,33 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
 
       SBO_REQUIRE(grid.y <= 65535, "too many candidates for the FP64 fantasy kernel");
       ev_begin(ctx, 4);
-#define FL(DD) k_fantasy_f64<DD><<<grid, 256, 0, ctx->stream>>>(fc, nx, nz, nxp, nzp, (const double*)ctx->vx.p, (const double*)ctx->vz.p, xn, ax, bx, zn, mz, sz, cnt, key_x, key_z, row_perm, ctr)
+#define FLT(DD, T) k_fantasy_f64<DD, T><<<grid, 256, 0, ctx->stream>>>(fc, nx, nz, nxp, nzp, (const double*)ctx->vx.p, (const double*)ctx->vz.p, xn, ax, bx, zn, mz, sz, cnt, key_x, key_z, row_perm, ctr, hitw)
+#define FL(DD) do { if (hitw) FLT(DD, true); else FLT(DD, false); } while (0)
       switch (d) { case 1: FL(1); break; case 2: FL(2); break; case 3: FL(3); break; case 4: FL(4); break;
                    case 5: FL(5); break; case 6: FL(6); break; case 7: FL(7); break; default: FL(8); break; }
 #undef FL
+#undef FLT
       SBO_LAUNCH_CHECK();
       ps.counted = true;          // pairs evaluated = ctr[0] * nc (read back in finish)
       ps.count_scale = nc;
     } else {   // record prep is logged as phase 6, the GEMM kernel as phase 4 (begun inside)
       long long run_pairs = nx * nz;
-      FantasyPruneArgs pr{key_x, key_z, row_perm, &run_pairs, 0, nullptr, nullptr, 0};
+      FantasyPruneArgs pr{key_x, key_z, row_perm, &run_pairs, 0, nullptr, nullptr, 0, nullptr, hitw, nullptr};
       const bool refine = (ps.precision == SBO_PREC_TF32X3 && ctx->opt_fantasy_refine >= 1) || (ps.precision == SBO_PREC_TF32 && ctx->opt_fantasy_refine >= 2);
       const bool bounds = refine && ctx->opt_fantasy_refine == 3;
       ps.bounds = bounds; ps.n_ambiguous = 0; ps.n_refined_safe = 0;
       if (bounds) {
         // bounds mode: no list and no FP64 pass.  counts = the pairs the error bound SETTLES as newly safe (a lower bound of the
-        // FP64 counts), amb_rows = per candidate the number of pairs it cannot settle (counts + amb_rows is an upper bound)
-        SBO_TRY(sbo_ensure(ctx, ctx->amb_rows, sizeof(int) * (size_t)nx));
-        SBO_CUDA(cudaMemsetAsync(ctx->amb_rows.p, 0, sizeof(int) * (size_t)nx, ctx->stream));
+        // FP64 counts), amb_rows = per candidate the number of pairs it cannot settle (counts + amb_rows is an upper bound).
+        // GoOSE target: the hit words hold the z with a settled pair, amb_rows the words of the z with a pair inside the bound
+        const size_t amb_b = goose ? sizeof(uint32_t) * (size_t)cdiv(nz, 32) : sizeof(int) * (size_t)nx;
+        SBO_TRY(sbo_ensure(ctx, ctx->amb_rows, amb_b));
+        SBO_CUDA(cudaMemsetAsync(ctx->amb_rows.p, 0, amb_b, ctx->stream));
         SBO_TRY(sbo_ensure(ctx, ctx->amb_ctr, 2 * sizeof(unsigned long long)));
         SBO_CUDA(cudaMemsetAsync(ctx->amb_ctr.p, 0, 2 * sizeof(unsigned long long), ctx->stream));
         pr.refine = 1; pr.amb_list = nullptr; pr.amb_cap = 0; pr.amb_count = (unsigned long long*)ctx->amb_ctr.p;
-        pr.amb_rows = (int*)ctx->amb_rows.p;
+        if (goose) pr.amb_words = (uint32_t*)ctx->amb_rows.p;
+        else pr.amb_rows = (int*)ctx->amb_rows.p;
       } else if (refine) {
         // list capacity: a 256th of the pairs, between 1 M and 32 M entries (C4: ~1 M ambiguous pairs of 3e10)
         long long cap = nx * nz / 256;
@@ -1562,7 +1638,7 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
         }
         ev_end(ctx);
         ev_begin(ctx, 7);
-        SBO_TRY(refine_ambiguous(ctx, fc, nx, nz, cnt, row_perm));
+        SBO_TRY(refine_ambiguous(ctx, fc, nx, nz, cnt, row_perm, hitw));
       }
     }
     ev_end(ctx);
@@ -1570,7 +1646,21 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
   return SBO_OK;
 }
 
-// result_dev: the (all-reduced) per-candidate results; the local candidates are rows [offset, offset+nx_local)
+// GoOSE fantasy target: hit bits over the prepared z slots -> grid-ordered target mask; bounds mode: slots with an ambiguous
+// pair and no settled one -> undecided mask
+__global__ void __launch_bounds__(256)
+k_slots_to_mask(long long n, const long long* __restrict__ idx, const uint32_t* __restrict__ hit, const uint32_t* __restrict__ amb,
+                uint32_t* __restrict__ mask, uint32_t* __restrict__ und) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const long long p = idx[t];
+  const uint32_t bit = 1u << (t & 31);
+  if (hit[t >> 5] & bit) atomicOr(mask + (p >> 5), 1u << (p & 31));
+  else if (amb && (amb[t >> 5] & bit)) atomicOr(und + (p >> 5), 1u << (p & 31));
+}
+
+// result_dev: the (all-reduced) per-candidate results; the local candidates are rows [offset, offset+nx_local).
+// GoOSE fantasy target: the local hit words of pairs_run (no reduction needed: every rank paired all candidates)
 int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_dev, sbo_pair_result* out, int32_t* counts_host) {
   PairStage& ps = ctx->ps;
   SBO_REQUIRE(ps.prepared && ps.imported, "sbo_pairs_finish: run the pair stage first");
@@ -1580,6 +1670,7 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
   const long long count = ctx->gs.count, nw = mask_words(ctx);
   const long long nx = ps.nx_local, nz = ps.nz_local, nxt = ps.nx_total;
   const bool fantasy = ps.mode == SBO_MODE_FANTASY;
+  const bool counted = fantasy && !goose;              // per-candidate newly-safe counts (fantasy expander)
   SBO_REQUIRE(goose || (offset >= 0 && offset + nx <= nxt), "local candidate slice out of range");
   memset(out, 0, sizeof(*out));
   out->best_idx = -1;
@@ -1592,7 +1683,7 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
   SBO_TRY(sbo_ensure(ctx, mbuf, sizeof(uint32_t) * (size_t)(nc > 0 ? nc : 1) * nw));
   SBO_CUDA(cudaMemsetAsync(mbuf.p, 0, sizeof(uint32_t) * (size_t)(nc > 0 ? nc : 1) * nw, ctx->stream));
   SBO_TRY(sbo_ensure(ctx, ctx->pairctr, 2 * sizeof(unsigned long long)));
-  if (fantasy) {
+  if (counted) {
     SBO_TRY(sbo_ensure(ctx, ctx->counts, sizeof(int) * (size_t)count));
     SBO_CUDA(cudaMemsetAsync(ctx->counts.p, 0, sizeof(int) * (size_t)count, ctx->stream));
   }
@@ -1604,7 +1695,14 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
   if (have) {
     ev_begin(ctx, 6);
     const long long* idx = (const long long*)(goose ? ctx->zs_idx.p : ctx->xs_idx.p);
-    if (fantasy)
+    if (bounds) {
+      SBO_TRY(sbo_ensure(ctx, ctx->m_und, sizeof(uint32_t) * (size_t)nw));
+      SBO_CUDA(cudaMemsetAsync(ctx->m_und.p, 0, sizeof(uint32_t) * (size_t)nw, ctx->stream));
+    }
+    if (fantasy && goose)
+      k_slots_to_mask<<<(unsigned)cdiv(nz, 256), 256, 0, ctx->stream>>>(nz, idx, (const uint32_t*)result_dev, bounds ? (const uint32_t*)ctx->amb_rows.p : nullptr,
+                                                                       (uint32_t*)mbuf.p, (uint32_t*)ctx->m_und.p);
+    else if (fantasy)
       k_counts_scatter<<<(unsigned)cdiv(nx, 256), 256, 0, ctx->stream>>>(nx, offset, idx, (const int*)result_dev, (int*)ctx->counts.p, (uint32_t*)mbuf.p);
     else
       k_hits_to_mask<<<(unsigned)cdiv(nloc, 256), 256, 0, ctx->stream>>>(nc, nloc, goose ? nz : nxt, goose ? 0 : offset, idx,
@@ -1617,11 +1715,12 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
     SBO_CUDA(cudaMemcpyAsync(h, ctr, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
     if (bounds) {
       // amb_rows holds the (all-reduced, sbo_*_step_sharded) per-candidate ambiguous-pair counts in the layout of result_dev
-      SBO_TRY(sbo_ensure(ctx, ctx->m_und, sizeof(uint32_t) * (size_t)nw));
-      SBO_CUDA(cudaMemsetAsync(ctx->m_und.p, 0, sizeof(uint32_t) * (size_t)nw, ctx->stream));
-      k_undecided_mask<<<(unsigned)cdiv(nx, 256), 256, 0, ctx->stream>>>(nx, offset, idx, (const int*)result_dev, (const int*)ctx->amb_rows.p,
-                                                                          (int*)ctx->counts.p, (uint32_t*)ctx->m_und.p);
-      SBO_LAUNCH_CHECK();
+      // (GoOSE target: the undecided mask was built above from the local ambiguous words)
+      if (!goose) {
+        k_undecided_mask<<<(unsigned)cdiv(nx, 256), 256, 0, ctx->stream>>>(nx, offset, idx, (const int*)result_dev, (const int*)ctx->amb_rows.p,
+                                                                            (int*)ctx->counts.p, (uint32_t*)ctx->m_und.p);
+        SBO_LAUNCH_CHECK();
+      }
       SBO_CUDA(cudaMemsetAsync(ctr + 1, 0, sizeof(unsigned long long), ctx->stream));
       k_union_count<<<(unsigned)cdiv(nw, 256), 256, 0, ctx->stream>>>(1, (const uint32_t*)ctx->m_und.p, nw, ctr + 1);
       SBO_LAUNCH_CHECK();
@@ -1630,7 +1729,7 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
     ev_end(ctx);
   }
   if (counts_host) {
-    if (fantasy) SBO_CUDA(cudaMemcpyAsync(counts_host, ctx->counts.p, sizeof(int32_t) * (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
+    if (counted) SBO_CUDA(cudaMemcpyAsync(counts_host, ctx->counts.p, sizeof(int32_t) * (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
     else memset(counts_host, 0, sizeof(int32_t) * (size_t)count);
   }
   SBO_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1638,7 +1737,7 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
   out->n_hit = (int64_t)h[1];
   out->n_ambiguous = ps.n_ambiguous; out->n_refined_safe = ps.n_refined_safe;
   out->n_undecided = bounds ? (int64_t)h_und : 0;
-  out->undecided_best_idx = -1; out->undecided_best_value = -INFINITY;
+  out->undecided_best_idx = -1; out->undecided_best_value = goose ? INFINITY : -INFINITY;
   if (ps.counted) out->pairs_evaluated = (int64_t)h[0] * ps.count_scale;
   else out->pairs_evaluated = ps.pairs_evaluated;
   if (out->pairs_evaluated > out->pairs_algorithmic) out->pairs_evaluated = out->pairs_algorithmic;
@@ -1657,7 +1756,8 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
     }
   }
   if (bounds && out->n_undecided > 0) {
-    SBO_TRY(argreduce_run(ctx, SBO_ARGMAX_VAR0, (const uint32_t*)ctx->m_und.p, nullptr, &out->undecided_best_idx, &out->undecided_best_value));
+    SBO_TRY(argreduce_run(ctx, goose ? SBO_ARGMIN_LCB0 : SBO_ARGMAX_VAR0, (const uint32_t*)ctx->m_und.p, nullptr, &out->undecided_best_idx,
+                          &out->undecided_best_value));
     acc5 += ctx->phase_ms[5];
   }
   ctx->phase_ms[5] = keep5 + acc5;
@@ -1678,7 +1778,8 @@ static int pairs_single(sbo_ctx* ctx, int mode, int precision, bool goose, doubl
   if (mode == SBO_MODE_FANTASY) SBO_TRY(sbo_ensure(ctx, ctx->exp_v, (size_t)(nx > 0 ? nx : 1) * info.vrow_bytes));
   SBO_TRY(pairs_export(ctx, ctx->exp_rows.p, ctx->exp_v.p));
   SBO_TRY(pairs_import(ctx, nx, ctx->exp_rows.p, ctx->exp_v.p));
-  const size_t res_bytes = (mode == SBO_MODE_FANTASY) ? sizeof(int) * (size_t)nx : (size_t)(nc > 0 ? nc : 1) * (goose ? nz : nx);
+  const size_t res_bytes = (mode == SBO_MODE_FANTASY) ? (goose ? sizeof(uint32_t) * (size_t)cdiv(nz, 32) : sizeof(int) * (size_t)nx)
+                                                     : (size_t)(nc > 0 ? nc : 1) * (goose ? nz : nx);
   SBO_TRY(sbo_ensure(ctx, ctx->hits, res_bytes));
   SBO_TRY(pairs_run(ctx, goose ? 1 : 0, ctx->hits.p));
   return pairs_finish(ctx, goose ? 1 : 0, 0, ctx->hits.p, out, counts_host);
@@ -1691,4 +1792,8 @@ int pairs_lipschitz(sbo_ctx* ctx, bool goose, double beta, const double* L, sbo_
 
 int pairs_fantasy(sbo_ctx* ctx, int precision, double beta, sbo_pair_result* out, int32_t* counts_host) {
   return pairs_single(ctx, SBO_MODE_FANTASY, precision, false, beta, nullptr, out, counts_host);
+}
+
+int pairs_goose_fantasy(sbo_ctx* ctx, int precision, double beta, sbo_pair_result* out) {
+  return pairs_single(ctx, SBO_MODE_FANTASY, precision, true, beta, nullptr, out, nullptr);
 }

@@ -308,12 +308,16 @@ class GridEngine:
             out["counts"] = counts
         return out
 
-    def goose_target(self, beta, L):
+    def goose_target(self, beta, L=None, mode=capi.MODE_LIPSCHITZ, precision=capi.PREC_FP64):
+        """GoOSE target set (SBO_MASK_TARGET) and its argmin lcb_0: Lipschitz pair test (L required) or fantasy test."""
         r = capi.PairResult()
-        Lc = _f64(L)
-        if Lc.shape[0] != self.G:
-            raise ValueError("L must have one entry per GP")
-        self._ck(self._lib.sbo_goose_target(self._h, float(beta), capi.dptr(Lc), C.byref(r)))
+        Lp = None
+        if mode == capi.MODE_LIPSCHITZ or L is not None:
+            Lc = _f64(L)
+            if Lc.ndim != 1 or Lc.shape[0] != self.G:
+                raise ValueError("L must have one entry per GP")
+            Lp = capi.dptr(Lc)
+        self._ck(self._lib.sbo_goose_target_ex(self._h, int(mode), int(precision), float(beta), Lp, C.byref(r)))
         return self._pair_dict(r)
 
     # -- staged pair driver (multi-GPU; tensors are torch CUDA tensors or anything with data_ptr()) --------
@@ -402,12 +406,14 @@ class GridEngine:
                                                     int(prec), int(unsafe_rule), Lp, C.byref(r)))
         return self._step_dict(r, False)
 
-    def goose_step_sharded(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True):
+    def goose_step_sharded(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, mode="lipschitz", precision="fp64"):
         if upload:
             self.set_model(ds)
+        prec, _ = capi.PRECISIONS[precision]
         r = capi.StepResult()
         Lp = capi.dptr(_f64(L)) if L is not None else None
-        self._ck(self._lib.sbo_goose_step_sharded(self._h, float(beta), int(unsafe_rule), Lp, C.byref(r)))
+        self._ck(self._lib.sbo_goose_step_sharded_ex(self._h, float(beta), capi.MODE_FANTASY if mode == "fantasy" else capi.MODE_LIPSCHITZ,
+                                                     int(prec), int(unsafe_rule), Lp, C.byref(r)))
         return self._step_dict(r, True)
 
     # -- whole steps (drivers' decision rules) ------------------------------------------------
@@ -438,18 +444,24 @@ class GridEngine:
         out["x_new_idx"] = s["minimizer_idx"] if out["minimizer_std"] > out["expander_std"] else ex["best_idx"]
         return out
 
-    def goose_step(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True):
-        """Decision rule of test/test_GoOSE.py:151-162."""
+    def goose_step(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, mode="lipschitz", precision="fp64"):
+        """Decision rule of test/test_GoOSE.py:151-162.  mode="fantasy": the target set comes from the fantasy pair test
+        (GP update with y_i = ucb_i(x)) at `precision`; L is not used."""
         if upload:
             self.set_model(ds)
-        self.posterior(with_grad=L is None, keep_v=0, fetch=False)
+        fantasy = mode == "fantasy"
+        prec, kv = capi.PRECISIONS[precision]
+        self.posterior(with_grad=not fantasy and L is None, keep_v=kv if fantasy else 0, fetch=False)
         s = self.sets_pass1(beta, unsafe_rule)
         out = dict(s)
-        if L is None:
-            Lg = self.lipschitz()
-            L = np.full(self.G, Lg[self.G - 1])           # GoOSE.py:100
-            out["L"] = Lg
-        tg = self.goose_target(beta, L)
+        if fantasy:
+            tg = self.goose_target(beta, None, capi.MODE_FANTASY, prec)
+        else:
+            if L is None:
+                Lg = self.lipschitz()
+                L = np.full(self.G, Lg[self.G - 1])       # GoOSE.py:100
+                out["L"] = Lg
+            tg = self.goose_target(beta, L)
         out["target"] = tg
         out["target_idx"], out["target_lcb"] = tg["best_idx"], tg["best_value"]
         if s["min_lcb0"] <= tg["best_value"] or tg["best_idx"] < 0:

@@ -1,8 +1,10 @@
 """Drop-in mirror of the reference's ``models/GoOSE.py`` (class ``BO``), restated on a dense grid.
 
 ``minimize_obj_lcb`` / ``Target`` / ``explore_safeset`` (GoOSE.py:63-119) each become one masked
-arg-reduction (plus, for ``Target``, the Lipschitz pair kernel with the reduction over the safe side)
-of the CUDA grid pipeline.  Same constructor and return values as the reference.
+arg-reduction (plus, for ``Target``, the pair kernel with the reduction over the safe side) of the CUDA
+grid pipeline.  Same constructor and return values as the reference; ``expander_mode='fantasy'`` (with
+``precision`` 'fp64' | 'tf32' | 'tf32x3') replaces the Lipschitz reachability test of ``Target`` by the
+fantasy test of the SafeOpt expander: z is reachable if the GP update with y_i = ucb_i(x) makes it safe.
 """
 from __future__ import annotations
 
@@ -13,9 +15,10 @@ from .SafeOpt import BO as _GridBO
 
 
 class BO(_GridBO):
-    def __init__(self, plant_system, bound, b, grid_points_per_dim=None, unsafe_rule='all', device=0):
+    def __init__(self, plant_system, bound, b, grid_points_per_dim=None, unsafe_rule='all', device=0,
+                 expander_mode='lipschitz', precision='fp64'):
         _GridBO.__init__(self, plant_system, bound, b, grid_points_per_dim=grid_points_per_dim,
-                         expander_mode='lipschitz', precision='fp64', unsafe_rule=unsafe_rule, device=device)
+                         expander_mode=expander_mode, precision=precision, unsafe_rule=unsafe_rule, device=device)
         # GoOSE.py:22-25 -- kept for API compatibility (SciPy constraint objects over lcb_i >= 0)
         self.safe_set_cons = [NonlinearConstraint(lambda x, i=i: self.lcb(x, i), 0., np.inf)
                               for i in range(1, self.n_fun)]
@@ -30,8 +33,12 @@ class BO(_GridBO):
         Empty target set -> (nan, +inf) so the driver's ``min_safe_lcb <= target_lcb`` picks the safe minimiser."""
         st = self._ensure_step()
         if "target" not in st:
-            L = np.full(self.n_fun, st["L"][self.n_fun - 1])       # GoOSE.py:100: leaked i = n_fun-1
-            st["target"] = self.engine.goose_target(self.b, L)
+            capi = self._capi()
+            if self.expander_mode == 'fantasy':
+                st["target"] = self.engine.goose_target(self.b, None, capi.MODE_FANTASY, capi.PRECISIONS[self.precision][0])
+            else:
+                L = np.full(self.n_fun, st["L"][self.n_fun - 1])   # GoOSE.py:100: leaked i = n_fun-1
+                st["target"] = self.engine.goose_target(self.b, L)
         tg = st["target"]
         if tg["best_idx"] < 0:
             return self._x(-1), np.inf

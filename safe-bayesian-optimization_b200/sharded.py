@@ -7,7 +7,8 @@ this module only inserts the collectives (``torch.distributed``: NCCL on GPUs, g
   broadcasts      the candidates' rows (+ V rows in fantasy mode), one block per rank straight into the gathered
                   buffer (an all-gather with uneven blocks): every rank pairs ALL candidates x in S with ITS OWN
                   unsafe points z
-  all-reduce      per-candidate hit flags (max) / newly-safe counts (sum)
+  all-reduce      per-candidate hit flags (max) / newly-safe counts (sum); none for the fantasy GoOSE target, whose
+                  verdict on an unsafe point is local
   all-gather      local optima (value, global index) -> deterministic reduction, lowest index on ties
 
 The engine is any object with the GridEngine staged-pair interface, so the orchestration is testable on CPU
@@ -168,7 +169,7 @@ def _pairs(eng, mode, prec, beta, L, goose, device, group, want_counts=False):
     n_all = gather_scalars([nx], device, group)[:, 0].astype(np.int64)
     n_total, offset = int(n_all.sum()), int(n_all[:rank].sum())
     fantasy = mode == capi.MODE_FANTASY
-    if fantasy and world > 1 and getattr(eng, "options", {}).get("fantasy_refine") == 3:
+    if fantasy and not goose and world > 1 and getattr(eng, "options", {}).get("fantasy_refine") == 3:
         raise ValueError("fantasy_refine = 3 (bounds mode) on several ranks needs the library communicator: "
                          "init_comm() / orchestrator='library' (the per-candidate undecided counts are combined there)")
     if not fantasy and world > 1 and hasattr(eng, "pairs_set_segments"):
@@ -211,7 +212,9 @@ def _pairs(eng, mode, prec, beta, L, goose, device, group, want_counts=False):
             torch.cuda.empty_cache()         # hand the gathered copy back before the GEMM workspaces are sized
     tr.mark("import")
     nc = eng.G - 1
-    if goose:
+    if goose and fantasy:                  # hit words over this rank's prepared unsafe slots
+        result = torch.zeros(max((nz + 31) // 32, 1), dtype=torch.int32, device=device)
+    elif goose:
         result = torch.zeros(max(nc * nz, 1), dtype=torch.uint8, device=device)
     elif fantasy:
         result = torch.zeros(max(n_total, 1), dtype=torch.int32, device=device)
@@ -239,6 +242,10 @@ def _pairs(eng, mode, prec, beta, L, goose, device, group, want_counts=False):
     out = {"best_idx": bi, "best_value": bv, "per_idx": per_idx, "per_value": per_value, "n_x": n_total,
            "n_z": int(tot[0]), "n_hit": int(tot[1]), "pairs_evaluated": int(tot[2]),
            "pairs_algorithmic": n_total * int(tot[0]) * nc, "n_ambiguous": int(tot[3]), "n_refined_safe": int(tot[4]), "local": loc}
+    if goose and fantasy:                  # bounds mode: the undecided unsafe points are local too
+        (uv, ui), = reduce_arg([(loc.get("undecided_best_value", np.inf), loc.get("undecided_best_idx", -1))], device, False, group)
+        out.update({"n_undecided": int(gather_scalars([loc.get("n_undecided", 0)], device, group).sum()),
+                    "undecided_best_idx": ui, "undecided_best_value": uv})
     return out
 
 
@@ -269,16 +276,23 @@ def safeopt_step(eng, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=
     return out
 
 
-def goose_step(eng, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, device=None, group=None, coords=None):
-    """test/test_GoOSE.py:151-162 on a sharded grid."""
+def goose_step(eng, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, device=None, group=None, coords=None,
+               mode="lipschitz", precision="fp64"):
+    """test/test_GoOSE.py:151-162 on a sharded grid.  mode="fantasy": candidate and V rows are exchanged as in the
+    SafeOpt fantasy step, then every rank decides its own unsafe points (no result all-reduce)."""
     if getattr(eng, "comm_ready", False) and group is None:
-        return eng.goose_step_sharded(ds, beta, unsafe_rule=unsafe_rule, L=L, upload=upload)
+        return eng.goose_step_sharded(ds, beta, unsafe_rule=unsafe_rule, L=L, upload=upload, mode=mode, precision=precision)
     device = torch.device("cuda", eng.device) if device is None else device
-    out = _posterior_and_sets(eng, ds, beta, unsafe_rule, with_grad=L is None, keep_v=0, upload=upload, device=device,
-                              group=group, need_pass2=False)
-    if L is None:
-        L = np.full(eng.G, out["L"][eng.G - 1])                  # GoOSE.py:100
-    tg = _pairs(eng, capi.MODE_LIPSCHITZ, capi.PREC_FP64, beta, L, True, device, group)
+    fantasy = mode == "fantasy"
+    prec, kv = capi.PRECISIONS[precision]
+    out = _posterior_and_sets(eng, ds, beta, unsafe_rule, with_grad=(not fantasy and L is None), keep_v=kv if fantasy else 0,
+                              upload=upload, device=device, group=group, need_pass2=False)
+    if fantasy:
+        tg = _pairs(eng, capi.MODE_FANTASY, prec, beta, None, True, device, group)
+    else:
+        if L is None:
+            L = np.full(eng.G, out["L"][eng.G - 1])              # GoOSE.py:100
+        tg = _pairs(eng, capi.MODE_LIPSCHITZ, capi.PREC_FP64, beta, L, True, device, group)
     out["target"] = tg
     out["target_idx"], out["target_lcb"] = tg["best_idx"], tg["best_value"]
     if out["min_lcb0"] <= tg["best_value"] or tg["best_idx"] < 0:
