@@ -49,6 +49,14 @@ enum sbo_status {
 enum sbo_unsafe_rule { SBO_UNSAFE_ALL = 0, SBO_UNSAFE_ANY = 1 };
 
 enum sbo_expander_mode { SBO_MODE_LIPSCHITZ = 0, SBO_MODE_FANTASY = 1 };
+
+/* covariance function of a model (sbo_set_model_ex, sbo_nll_batch_ex).  With the scaled squared distance
+ * s = sum_k (x_k - x'_k)^2 / ell_k of the ARD hyper-parameters:
+ *   SE        k = sf2 exp(-s/2)                      (GP_Safe.py:98-120, the reference's 'RBF')
+ *   MATERN32  k = sf2 (1 + t) exp(-t),        t = sqrt(3 s)
+ *   MATERN52  k = sf2 (1 + t + t^2/3) exp(-t), t = sqrt(5 s)
+ * Every GP of a model uses the same kernel; k(x, x) = sf2 for all three. */
+enum sbo_kernel { SBO_KERNEL_SE = 0, SBO_KERNEL_MATERN32 = 1, SBO_KERNEL_MATERN52 = 2 };
 enum sbo_precision { SBO_PREC_FP64 = 0, SBO_PREC_TF32 = 1, SBO_PREC_TF32X3 = 2 };
 
 /* score selectors for sbo_argreduce */
@@ -79,6 +87,15 @@ int sbo_set_model(sbo_ctx* ctx, int n, int d, int G,
                   const double* X_mean, const double* X_std,
                   const double* Y_mean, const double* Y_std,
                   const double* hyp);
+/* sbo_set_model with the covariance function `kernel` (enum sbo_kernel) in place of the SE kernel: K_i = k_i(X, X) + (sn2 +
+ * eps_f32) I with the same hyper-parameter layout.  sbo_set_model is the SBO_KERNEL_SE case.  The kernel stays part of the
+ * installed model: sbo_append_sample, the posterior, the sets, every pair test and the sharded steps use it.  The separable
+ * options "posterior_tables" and "posterior_fused" exist for the SE kernel only and are ignored for the others. */
+int sbo_set_model_ex(sbo_ctx* ctx, int kernel, int n, int d, int G,
+                     const double* X_norm, const double* Y_norm,
+                     const double* X_mean, const double* X_std,
+                     const double* Y_mean, const double* Y_std,
+                     const double* hyp);
 /* One more observation at FIXED hyper-parameters and FIXED normalisation (SURVEY.md section 8f row 1): x_norm_new[d],
  * y_norm_new[G] in the normalised units of the installed model.  Rank-1 update of the factor on the device -- new row of
  * L, of W = L^-1 and a refreshed alpha, O(n^2) -- instead of the rebuild + O(n^3) inverse of GP.add_sample
@@ -272,9 +289,9 @@ int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms);
 int sbo_refine_stats(sbo_ctx* ctx, int64_t* cells, int64_t* fp64_rows);
 /* tuning / diagnosis options (defaults reproduce the documented behaviour; none changes a result):
  *   "posterior_variant"  1 (default) FP64 tensor cores (DMMA) | 0 FP64 SIMT register tiles
- *   "posterior_tables"   1: on meshgrids the cross-covariance kernel multiplies separable SE-ARD factor tables instead of calling
+ *   "posterior_tables"   1 (SE kernel only): on meshgrids the cross-covariance kernel multiplies separable SE-ARD factor tables instead of calling
  *                        exp() per entry (same values to ~1e-16 relative; measured slower, 13.5 vs 9.0 ms at C4) | 0 (default)
- *   "posterior_fused"    1: meshgrids use separable SE-ARD factor tables; the cross-covariance is generated inside the solve
+ *   "posterior_fused"    1 (SE kernel only): meshgrids use separable SE-ARD factor tables; the cross-covariance is generated inside the solve
  *                        kernel's shared-memory stage and never stored (C4: 12 MB of DRAM traffic instead of 33.6 GB, 52.5 ms
  *                        instead of 40.0 ms) | 0 (default): cross-covariance kernel + scratch + solve
  *   "posterior_chunk_mb" size of the cross-covariance tile one posterior chunk keeps between its two kernels in MB (default 1024; 24-96 keeps it L2 resident but measured slower at C4)
@@ -305,6 +322,10 @@ int sbo_set_option(sbo_ctx* ctx, const char* name, int64_t value);
  * 1/2 log sf2, 1/2 log sn2) as GP_Safe.py:180-182, nll[P] out; a K_p that is not positive definite gives +inf.
  * Does not touch the model installed by sbo_set_model. */
 int sbo_nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll);
+/* sbo_nll_batch with K_p = k_p(X, X) + (sn2 + 1e-8) I of the covariance function `kernel` (enum sbo_kernel); sbo_nll_batch is the
+ * SBO_KERNEL_SE case. */
+int sbo_nll_batch_ex(sbo_ctx* ctx, int kernel, int n, int d, const double* X_norm, const double* y, int P, const double* hyp,
+                     double* nll);
 
 /* give device workspaces back to the driver (large grids: the V rows of the fantasy expander are n x count per
  * constraint -- 51 GB per rank at C5).  what = 1: the per-point V rows kept by sbo_posterior(keep_v) (call after

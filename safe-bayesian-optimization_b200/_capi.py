@@ -21,6 +21,8 @@ PREC_FP64, PREC_TF32, PREC_TF32X3 = 0, 1, 2
 PRECISIONS = {"fp64": (0, 1), "tf32": (1, 2), "tf32x3": (2, 3)}
 ARGMAX_VAR0, ARGMIN_LCB0, ARGMIN_UCB0, ARGMIN_DIST = 0, 1, 2, 3
 MASK_SAFE, MASK_MIN, MASK_UNSAFE, MASK_USER, MASK_EXPANDER, MASK_TARGET = 0, 1, 2, 3, 4, 5
+# covariance function name (models/GP_Safe.GP kernel argument) -> enum sbo_kernel
+KERNELS = {"RBF": 0, "Matern32": 1, "Matern52": 2}
 PHASES = ("model", "crosscov", "solve", "sets", "pairs", "argreduce", "pair_prep", "refine")
 
 
@@ -62,6 +64,7 @@ SIGNATURES = {
     "sbo_set_stream": (C.c_int, [_P, _P]),
     "sbo_version": (C.c_int, []),
     "sbo_set_model": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _D, _D, _D, _D, _D, _D, _D]),
+    "sbo_set_model_ex": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _D, _D, _D, _D, _D, _D, _D]),
     "sbo_get_model": (C.c_int, [_P, _D, _D, _D]),
     "sbo_append_sample": (C.c_int, [_P, _D, _D]),
     "sbo_stable_minmax": (C.c_int, [_P, C.c_int, C.c_int, C.c_double, _I64, _D, _I64, _D]),
@@ -107,6 +110,7 @@ SIGNATURES = {
     "sbo_set_option": (C.c_int, [_P, C.c_char_p, C.c_int64]),
     "sbo_release": (C.c_int, [_P, C.c_int]),
     "sbo_nll_batch": (C.c_int, [_P, C.c_int, C.c_int, _D, _D, C.c_int, _D, _D]),
+    "sbo_nll_batch_ex": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _D, _D, C.c_int, _D, _D]),
 }
 
 _lib = None

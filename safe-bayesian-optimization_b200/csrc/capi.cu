@@ -129,11 +129,16 @@ int sbo_set_stream(sbo_ctx* ctx, void* cuda_stream) {
   return SBO_OK;
 }
 
-int sbo_set_model(sbo_ctx* ctx, int n, int d, int G, const double* X_norm, const double* Y_norm, const double* X_mean,
-                  const double* X_std, const double* Y_mean, const double* Y_std, const double* hyp) {
+int sbo_set_model_ex(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_norm, const double* Y_norm,
+                     const double* X_mean, const double* X_std, const double* Y_mean, const double* Y_std, const double* hyp) {
   ENTER();
   ctx->have_model = false;
-  return model_upload(ctx, n, d, G, X_norm, Y_norm, X_mean, X_std, Y_mean, Y_std, hyp);
+  return model_upload(ctx, kernel, n, d, G, X_norm, Y_norm, X_mean, X_std, Y_mean, Y_std, hyp);
+}
+
+int sbo_set_model(sbo_ctx* ctx, int n, int d, int G, const double* X_norm, const double* Y_norm, const double* X_mean,
+                  const double* X_std, const double* Y_mean, const double* Y_std, const double* hyp) {
+  return sbo_set_model_ex(ctx, SBO_KERNEL_SE, n, d, G, X_norm, Y_norm, X_mean, X_std, Y_mean, Y_std, hyp);
 }
 
 int sbo_get_model(sbo_ctx* ctx, double* L, double* W, double* alpha) {
@@ -435,9 +440,14 @@ int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms) {
   return SBO_OK;
 }
 
-int sbo_nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll) {
+int sbo_nll_batch_ex(sbo_ctx* ctx, int kernel, int n, int d, const double* X_norm, const double* y, int P, const double* hyp,
+                     double* nll) {
   ENTER();
-  return nll_batch(ctx, n, d, X_norm, y, P, hyp, nll);
+  return nll_batch(ctx, kernel, n, d, X_norm, y, P, hyp, nll);
+}
+
+int sbo_nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll) {
+  return sbo_nll_batch_ex(ctx, SBO_KERNEL_SE, n, d, X_norm, y, P, hyp, nll);
 }
 
 int sbo_append_sample(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_new) {

@@ -28,6 +28,7 @@ struct GridSpec {
 struct ModelSpec {
   int n, npad, d, G;
   int g0;                   // posterior kernels process GPs g0 .. G-1 (0 except for the constraint-only FP64 rows of the refinement)
+  int kernel;               // enum sbo_kernel: the covariance function of every GP of the model
   const double* Xn;         // [npad][d], rows >= n are zero
   const double* alpha;      // [G][npad]
   const double* W;          // [G][npad][npad]  lower-triangular L^-1, zero elsewhere
@@ -40,6 +41,7 @@ struct ModelSpec {
 // constants of the fantasy expander (constraint GPs only: entry c is GP c+1)
 struct FantasyConsts {
   int nc, d, npad;
+  int kernel;               // enum sbo_kernel (ModelSpec::kernel)
   double beta;
   double sf2[SBO_MAX_G - 1], sn2[SBO_MAX_G - 1];
   double inv_ell[SBO_MAX_G - 1][SBO_MAX_D];
@@ -81,6 +83,103 @@ __device__ __forceinline__ double lcb_of(double mean, double var, double beta) {
 }
 __device__ __forceinline__ double ucb_of(double mean, double var, double beta) {
   return __dadd_rn(mean, __dmul_rn(beta, sqrt(var)));
+}
+
+// ---- packed FP32 (FFMA2 / FMUL2 / FADD2 on sm_100a): two z columns per instruction in the tensor-core epilogue ----
+__device__ __forceinline__ float ex2_approx(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+__device__ __forceinline__ float sqrt_approx(float x) {
+  float y;
+  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+__device__ __forceinline__ uint64_t pk2(float lo, float hi) {
+  uint64_t r;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+  return r;
+}
+__device__ __forceinline__ void upk2(uint64_t v, float& lo, float& hi) {
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
+}
+__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
+  uint64_t r;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
+  return r;
+}
+__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
+  uint64_t r;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
+  uint64_t r;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+  return r;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Covariance functions (enum sbo_kernel).  Every kernel site is templated on one of two classes, so an SE model runs the
+// code it always ran and Matern 3/2 and 5/2 share one instantiation (their order is a run-time constant).  With the
+// scaled squared distance  s = sum_k (x_k - x'_k)^2 / ell_k:
+//   value(s, sf2) = k                    SE: sf2 exp(-s/2)      MATERN: sf2 (1 + t + q t^2) exp(-t),  t = sqrt(c s)
+//   phi(s, sf2)   = -2 dk/ds              SE: k                  MATERN: c sf2 ((1 - 2q) + q t) exp(-t)
+// (Matern 3/2: c = 3, q = 0; 5/2: c = 5, q = 1/3), so that  dk/dx_k = -phi (x_k - x'_k) / ell_k  for every kernel.
+// The tensor-core epilogue (fantasy_tc.cu) gets the exponent e from its FP32 records and evaluates k in packed FP32:
+//   SE: e = log2 k, k = 2^e.   MATERN: e = -c s (records scaled by rec_scale() = c), k = sf2 P(t) 2^(-t log2 e), t = sqrt(max(-e, 0)).
+// ---------------------------------------------------------------------------------------------
+struct SE {
+  static constexpr bool kIsSE = true;
+  __device__ __host__ explicit SE(int) {}
+  __device__ __forceinline__ double value(double s, double sf2) const { return sf2 * exp(-0.5 * s); }
+  __device__ __forceinline__ double phi(double s, double sf2) const { return sf2 * exp(-0.5 * s); }
+  // two columns at once from the packed exponent e; sf2 is already part of e
+  __device__ __forceinline__ uint64_t value_f32x2(uint64_t e, uint64_t /*sf2x2*/) const {
+    float e0, e1;
+    upk2(e, e0, e1);
+    return pk2(ex2_approx(e0), ex2_approx(e1));
+  }
+};
+struct MATERN {
+  static constexpr bool kIsSE = false;
+  double c, q;
+  __device__ __host__ explicit MATERN(int kernel)
+      : c(kernel == SBO_KERNEL_MATERN32 ? 3.0 : 5.0), q(kernel == SBO_KERNEL_MATERN32 ? 0.0 : 1.0 / 3.0) {}
+  __device__ __forceinline__ double value(double s, double sf2) const {
+    const double t = sqrt(c * s);
+    return sf2 * fma(fma(q, t, 1.0), t, 1.0) * exp(-t);
+  }
+  __device__ __forceinline__ double phi(double s, double sf2) const {
+    const double t = sqrt(c * s);
+    return c * sf2 * fma(q, t, 1.0 - 2.0 * q) * exp(-t);
+  }
+  // e = -c s of two columns (clamped at 0: the expanded square can round below it); sf2x2 = (sf2, sf2)
+  __device__ __forceinline__ uint64_t value_f32x2(uint64_t e, uint64_t sf2x2) const {
+    float e0, e1;
+    upk2(e, e0, e1);
+    const uint64_t t = pk2(sqrt_approx(fmaxf(-e0, 0.f)), sqrt_approx(fmaxf(-e1, 0.f)));
+    const float nl = -1.4426950408889634f, qf = (float)q;
+    float y0, y1;
+    upk2(mul2(t, pk2(nl, nl)), y0, y1);
+    const uint64_t ex = pk2(ex2_approx(y0), ex2_approx(y1));
+    const uint64_t P = fma2(fma2(pk2(qf, qf), t, pk2(1.f, 1.f)), t, pk2(1.f, 1.f));
+    return mul2(mul2(P, sf2x2), ex);
+  }
+};
+// scale of the squared-distance terms of the FP32 records: SE log2(e)/2 (e = log2 k), MATERN c (e = -c s)
+static inline double kernel_rec_scale(int kernel) {
+  return kernel == SBO_KERNEL_SE ? 0.5 * 1.4426950408889634 : (kernel == SBO_KERNEL_MATERN32 ? 3.0 : 5.0);
+}
+static inline bool kernel_valid(int kernel) {
+  return kernel == SBO_KERNEL_SE || kernel == SBO_KERNEL_MATERN32 || kernel == SBO_KERNEL_MATERN52;
+}
+// host: f(SE{}) or f(MATERN{kernel}) -- f launches the instantiation of its kernel class
+template <class F>
+static inline void with_kernel(int kernel, F&& f) {
+  if (kernel == SBO_KERNEL_SE) f(SE(kernel));
+  else f(MATERN(kernel));
 }
 
 // (value, index) pairs with lowest-index tie-break
@@ -238,13 +337,13 @@ void ev_collect(sbo_ctx* ctx);            // (after a stream sync) add all logge
 static inline long long cdiv(long long a, long long b) { return (a + b - 1) / b; }
 
 // implemented across the .cu files
-int model_upload(sbo_ctx* ctx, int n, int d, int G, const double* X_norm, const double* Y_norm,
+int model_upload(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_norm, const double* Y_norm,
                  const double* X_mean, const double* X_std, const double* Y_mean, const double* Y_std,
                  const double* hyp);
 int model_append(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_new);
 int ball_mask(sbo_ctx* ctx, int mask_kind, const double* x0, double r);
 int stable_minmax(sbo_ctx* ctx, int n_controlled, int fun_kind, double beta, int64_t* xc_idx, double* value, int64_t* n_robust_safe, double* score_host);
-int nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll);
+int nll_batch(sbo_ctx* ctx, int kernel, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll);
 int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v);
 int posterior_vrows_dev(sbo_ctx* ctx, long long m, const double* pts_dev, double* vout);
 void posterior_vrows_scratch(const sbo_ctx* ctx, long long m, size_t* mv_bytes, size_t* k_bytes);

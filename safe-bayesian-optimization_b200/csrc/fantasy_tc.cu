@@ -3,7 +3,8 @@
 //
 //   for every candidate x (rows, MMA M = 128) and every unsafe z (columns, MMA N = BN) and every constraint GP c:
 //       acc  = v_x . v_z                         tcgen05.mma kind::tf32, FP32 accumulator in TMEM, K = npad
-//       cov  = k_c(z,x) - acc                    SE-ARD kernel recomputed in the epilogue (ex2.approx)
+//       cov  = k_c(z,x) - acc                    covariance recomputed in the epilogue (SE: ex2.approx; Matern:
+//                                                sqrt.approx + ex2.approx + polynomial, common.cuh)
 //       mu'  = m_z + cov * a_x ,  s2' = s_z - cov^2 * b_x     (rank-1 fantasy update, normalised units)
 //       ok  &= mu' >= 0  &&  mu'^2 >= beta^2 * s2'            (<=> mu' - beta*sqrt(max(s2',0)) >= 0)
 //   g(x) = popcount over z of ok  -> atomicAdd per candidate.
@@ -53,6 +54,8 @@ struct Params {
   // safe; bounds mode sets bit z of amb_words instead of amb_rows when column z has a pair inside the error bound
   uint32_t* hit_words;
   uint32_t* amb_words;
+  int kernel;                      // enum sbo_kernel; Matern: sf2 of every constraint (SE carries it in the row records)
+  float ksf2[SBO_MAX_G - 1];
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -129,37 +132,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* r) {
       : "r"(taddr)
       : "memory");
 }
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
-// ---- packed FP32 (FFMA2 / FMUL2 / FADD2 on sm_100a): two z columns per instruction in the epilogue ----
-__device__ __forceinline__ uint64_t pk2(float lo, float hi) {
-  uint64_t r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ void upk2(uint64_t v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
-  uint64_t r;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-  return r;
-}
-__device__ __forceinline__ uint64_t mul2(uint64_t a, uint64_t b) {
-  uint64_t r;
-  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
-  uint64_t r;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-  return r;
-}
-
 // w |= bit  iff  mu >= 0 and mu^2 >= t   (two FSETP chained through the predicate + one predicated LOP3)
 __device__ __forceinline__ void set_bit_if_safe(uint32_t& w, float mu, float mm, float t, uint32_t bit) {
   asm("{\n\t.reg .pred p;\n\t"
@@ -174,6 +146,7 @@ __device__ __forceinline__ void set_bit_if_safe(uint32_t& w, float mu, float mm,
 template <int D4>
 struct RowConsts {
   uint64_t xx[4 * D4], Cx, ax, nbx, ex;      // ex: sqrt(c1)*|v_x| (refinement band), duplicated like the others
+  uint64_t kf;                               // Matern: (sf2_c, sf2_c); unused by SE
   __device__ __forceinline__ void load(const float* __restrict__ rowrec_row) {
     const float4* rr = reinterpret_cast<const float4*>(rowrec_row);
 #pragma unroll
@@ -189,9 +162,11 @@ struct RowConsts {
 // One 32-column chunk of the fused epilogue for one candidate row: acc[32] = v_x . v_z from TMEM, `rec` = the 16
 // pair-interleaved column records of the chunk in shared memory ((4*D4+4) float2 per column pair:
 // z_k pairs, -Bz pair, m_z pair, s'_z pair, pad).  Same operations in the same order as the scalar form
-// (e = (Cx - Bz) + sum xx_k z_k; cov = exp2(e) - acc; mu = cov*a + m; t = s' - cov^2 b'), two columns per FFMA2.
-template <int D4>
-__device__ __forceinline__ uint32_t epilogue_chunk(const uint32_t (&acc)[32], const uint64_t* __restrict__ rec, const RowConsts<D4>& rc) {
+// (e = (Cx - Bz) + sum xx_k z_k; cov = k(e) - acc; mu = cov*a + m; t = s' - cov^2 b'), two columns per FFMA2.
+// k(e) is KC::value_f32x2 (common.cuh): exp2(e) for SE, sf2 P(t) exp(-t) with t = sqrt(-e) for Matern.
+template <int D4, class KC>
+__device__ __forceinline__ uint32_t epilogue_chunk(const uint32_t (&acc)[32], const uint64_t* __restrict__ rec, const RowConsts<D4>& rc,
+                                                   const KC& kc) {
   constexpr int RS = 4 * D4 + 4;
   const uint64_t minus1 = pk2(-1.f, -1.f);
   uint32_t w = 0;
@@ -201,9 +176,7 @@ __device__ __forceinline__ uint32_t epilogue_chunk(const uint32_t (&acc)[32], co
     uint64_t e = add2(rc.Cx, p[4 * D4]);
 #pragma unroll
     for (int k = 0; k < 4 * D4; ++k) e = fma2(rc.xx[k], p[k], e);
-    float e0, e1;
-    upk2(e, e0, e1);
-    const uint64_t ex = pk2(ex2_approx(e0), ex2_approx(e1));
+    const uint64_t ex = kc.value_f32x2(e, rc.kf);
     const uint64_t a2 = pk2(__uint_as_float(acc[2 * jp]), __uint_as_float(acc[2 * jp + 1]));
     const uint64_t cov = fma2(a2, minus1, ex);
     const uint64_t mu = fma2(cov, rc.ax, p[4 * D4 + 1]);
@@ -226,9 +199,10 @@ __device__ __forceinline__ uint32_t epilogue_chunk(const uint32_t (&acc)[32], co
 //   S (settled safe)    <=  cov - E >= 0 (monotone branch) and f(cov - E) >= 0 evaluated PESSIMISTICALLY (-d_mu, +d_t);
 //                           only needed where U fails: whole warps skip it (almost every pair is settled unsafe).
 // Everything else is AMBIGUOUS and goes to the FP64 re-evaluation (pairs.cu refine_ambiguous).
-template <int D4>
+template <int D4, class KC>
 __device__ __forceinline__ void epilogue_chunk_refine(const uint32_t (&acc)[32], const uint64_t* __restrict__ rec, const RowConsts<D4>& rc,
-                                                      uint64_t e_abs2, uint64_t d_mu2, uint64_t d_t2, uint32_t& S, uint32_t& U) {
+                                                      const KC& kc, uint64_t e_abs2, uint64_t d_mu2, uint64_t d_t2, uint32_t& S,
+                                                      uint32_t& U) {
   constexpr int RS = 4 * D4 + 4;
   const uint64_t minus1 = pk2(-1.f, -1.f);
   uint32_t wup = 0, wsf = 0;
@@ -238,9 +212,7 @@ __device__ __forceinline__ void epilogue_chunk_refine(const uint32_t (&acc)[32],
     uint64_t e = add2(rc.Cx, p[4 * D4]);
 #pragma unroll
     for (int k = 0; k < 4 * D4; ++k) e = fma2(rc.xx[k], p[k], e);
-    float e0, e1;
-    upk2(e, e0, e1);
-    const uint64_t ex = pk2(ex2_approx(e0), ex2_approx(e1));
+    const uint64_t ex = kc.value_f32x2(e, rc.kf);
     const uint64_t a2 = pk2(__uint_as_float(acc[2 * jp]), __uint_as_float(acc[2 * jp + 1]));
     const uint64_t cov = fma2(a2, minus1, ex);
     const uint64_t E = fma2(rc.ex, p[4 * D4 + 3], e_abs2);                // ex*ez + e_abs
@@ -476,7 +448,7 @@ k_fantasy_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           uint32_t r[32];
           tmem_ld32(taddr + h * 32, r);
           asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-          bits[h] &= epilogue_chunk<D4>(r, cb + (size_t)h * 16 * RS, rc);
+          bits[h] &= epilogue_chunk<D4>(r, cb + (size_t)h * 16 * RS, rc, SE(SBO_KERNEL_SE));
         }
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         __syncwarp();
@@ -595,7 +567,7 @@ __device__ __forceinline__ bool item_coords2(const Params& p, long long item, in
   return xt < p.nxt;
 }
 
-template <int D4, int EW, bool REFINE, bool TARGET>   // TARGET: GoOSE target epilogue (column OR, p.hit_words)
+template <int D4, int EW, bool REFINE, bool TARGET, class KC>   // TARGET: GoOSE target epilogue (column OR, p.hit_words); KC: covariance function
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
 k_fantasy_tc2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const Params p) {
   using C = Cfg2<D4>;
@@ -762,9 +734,11 @@ k_fantasy_tc2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
       for (int h = 0; h < NCH; ++h) { bits[h] = 0xffffffffu; ubits[h] = 0u; }
       const uint64_t e_abs2 = pk2(p.e_abs, p.e_abs), d_mu2 = pk2(p.d_mu, p.d_mu), d_t2 = pk2(p.d_t, p.d_t);
+      const KC kc(p.kernel);
       for (int c = 0; c < p.nc; ++c) {
         RowConsts<D4> rc;
         rc.load(p.rowrec + ((size_t)c * p.nxp + xrow) * RS);
+        if (!KC::kIsSE) rc.kf = pk2(p.ksf2[c], p.ksf2[c]);
         mbar_wait(bar_cfull(b), bphase, p.err, 5);
         mbar_wait_cl(bar_tfull(slot), sphase, p.err, 6);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -778,10 +752,10 @@ k_fantasy_tc2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
           asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
           if (REFINE) {
             uint32_t S, U;
-            epilogue_chunk_refine<D4>(r, cb + (size_t)h * 16 * RS, rc, e_abs2, d_mu2, d_t2, S, U);
+            epilogue_chunk_refine<D4>(r, cb + (size_t)h * 16 * RS, rc, kc, e_abs2, d_mu2, d_t2, S, U);
             bits[h] &= S; ubits[h] |= U;
           } else {
-            bits[h] &= epilogue_chunk<D4>(r, cb + (size_t)h * 16 * RS, rc);
+            bits[h] &= epilogue_chunk<D4>(r, cb + (size_t)h * 16 * RS, rc, kc);
           }
         }
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -844,13 +818,15 @@ k_fantasy_tc2(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 }
 
 // ---------------------------------------------------------------------------------------------
-// FP32 record builders.  h = log2(e)/2 so that  k_c(z,x) = exp2(Cx - Bz + sum_k xx_k z_k)
-//   row (candidate x):  xx_k = 2 h w_ck x_k ; Cx = log2 sf2_c - h sum_k w_ck x_k^2 ; a = beta*sigma/(sigma^2+sn2) ;
+// FP32 record builders.  e = Cx - Bz + sum_k xx_k z_k = l - h s_c(z,x)  with  s_c = sum_k w_ck (z_k - x_k)^2:
+//   SE:     h = log2(e)/2, l = log2 sf2_c, so that  k_c(z,x) = exp2(e)
+//   MATERN: h = c (3 or 5), l = 0, so that  e = -c s = -t^2  (sf2_c is the per-constraint constant Params::ksf2)
+//   row (candidate x):  xx_k = 2 h w_ck x_k ; Cx = l - h sum_k w_ck x_k^2 ; a = beta*sigma/(sigma^2+sn2) ;
 //                       b' = beta^2/(sigma^2+sn2)
 //   col (unsafe z):     z_k ; -Bz, Bz = h sum_k w_ck z_k^2 ; m_z = mean/Ystd ; s'_z = beta^2 var/Ystd^2
 //                       (stored pair-interleaved: two adjacent columns form packed f32x2 operands)
 // ---------------------------------------------------------------------------------------------
-template <int D4>
+template <int D4, class KC>
 __global__ void __launch_bounds__(256)
 k_tc_records(FantasyConsts fc, long long n, long long npadrows, int is_row, const double* __restrict__ coords,
              const double* __restrict__ a, const double* __restrict__ b, float* __restrict__ rec, double esc,
@@ -868,7 +844,7 @@ k_tc_records(FantasyConsts fc, long long n, long long npadrows, int is_row, cons
     if (!is_row) o[(4 * D4 + 1) * st] = -1e30f;         // padded z columns can never become safe
     return;
   }
-  const double h = 0.5 * 1.4426950408889634;
+  const double h = KC::kIsSE ? 0.5 * 1.4426950408889634 : MATERN(fc.kernel).c;
   double q = 0.0;
   for (int k = 0; k < 4 * D4; ++k) {
     const double x = (k < fc.d) ? coords[(size_t)k * n + t] : 0.0;
@@ -893,7 +869,7 @@ k_tc_records(FantasyConsts fc, long long n, long long npadrows, int is_row, cons
     }
   }
   if (is_row) {
-    o[4 * D4] = (float)(log2(fc.sf2[c]) - h * q);
+    o[4 * D4] = (float)((KC::kIsSE ? log2(fc.sf2[c]) : 0.0) - h * q);
     o[4 * D4 + 1] = (float)av;
     o[4 * D4 + 2] = (float)(fc.beta * fc.beta * bv);
   } else {
@@ -963,7 +939,7 @@ static int launch(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx
 
 struct RefineArgs { int2* list; unsigned long long* count; long long cap; float e_abs, d_mu, d_t; int* rows; uint32_t* hit_words; uint32_t* amb_words; };
 
-template <int D4, int EW, bool REFINE, bool TARGET>
+template <int D4, int EW, bool REFINE, bool TARGET, class KC>
 static int launch2(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx, long long nz, long long nxp, long long nzp,
                    const float* Vx, const float* Vz, const float* rowrec, const float* colrec, int* counts, int* err,
                    const long long* item_list, long long n_list, const int* row_perm, int gx, const RefineArgs& ra) {
@@ -987,10 +963,12 @@ static int launch2(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   p.item_list = item_list; p.row_perm = row_perm;
   p.amb_list = ra.list; p.amb_count = ra.count; p.amb_cap = ra.cap; p.amb_rows = ra.rows; p.e_abs = ra.e_abs; p.d_mu = ra.d_mu; p.d_t = ra.d_t;
   p.hit_words = ra.hit_words; p.amb_words = ra.amb_words;
+  p.kernel = fc.kernel;
+  for (int c = 0; c < fc.nc; ++c) p.ksf2[c] = (float)fc.sf2[c];
   if (p.n_items == 0) return SBO_OK;
-  SBO_CUDA((cudaFuncSetAttribute(k_fantasy_tc2<D4, EW, REFINE, TARGET>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES)));
+  SBO_CUDA((cudaFuncSetAttribute(k_fantasy_tc2<D4, EW, REFINE, TARGET, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES)));
   const int grid = 2 * (int)((p.n_items < clusters) ? p.n_items : clusters);
-  k_fantasy_tc2<D4, EW, REFINE, TARGET><<<grid, 128 + 32 * EW, C::SMEM_BYTES, ctx->stream>>>(tmA, tmB, p);
+  k_fantasy_tc2<D4, EW, REFINE, TARGET, KC><<<grid, 128 + 32 * EW, C::SMEM_BYTES, ctx->stream>>>(tmA, tmB, p);
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }
@@ -1088,31 +1066,45 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
     SBO_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), ctx->stream));
   }
   ev_begin(ctx, 6);
-  if (D4 == 1) {
-    tc::k_tc_records<1><<<dim3((unsigned)cdiv(nxp, 256), nc), 256, 0, ctx->stream>>>(fc, nx, nxp, 1, xn, ax, bx, rowrec, esc, stats);
-    SBO_LAUNCH_CHECK();
-    tc::k_tc_records<1><<<dim3((unsigned)cdiv(nzp, 256), nc), 256, 0, ctx->stream>>>(fc, nz, nzp, 0, zn, mz, sz, colrec, esc, stats);
-    SBO_LAUNCH_CHECK();
-  } else {
-    tc::k_tc_records<2><<<dim3((unsigned)cdiv(nxp, 256), nc), 256, 0, ctx->stream>>>(fc, nx, nxp, 1, xn, ax, bx, rowrec, esc, stats);
-    SBO_LAUNCH_CHECK();
-    tc::k_tc_records<2><<<dim3((unsigned)cdiv(nzp, 256), nc), 256, 0, ctx->stream>>>(fc, nz, nzp, 0, zn, mz, sz, colrec, esc, stats);
-    SBO_LAUNCH_CHECK();
-  }
+  const bool se = fc.kernel == SBO_KERNEL_SE;
+#define TC_REC(D4_, KC_) do { \
+    tc::k_tc_records<D4_, KC_><<<dim3((unsigned)cdiv(nxp, 256), nc), 256, 0, ctx->stream>>>(fc, nx, nxp, 1, xn, ax, bx, rowrec, esc, stats); \
+    SBO_LAUNCH_CHECK(); \
+    tc::k_tc_records<D4_, KC_><<<dim3((unsigned)cdiv(nzp, 256), nc), 256, 0, ctx->stream>>>(fc, nz, nzp, 0, zn, mz, sz, colrec, esc, stats); \
+    SBO_LAUNCH_CHECK(); } while (0)
+  if (D4 == 1) { if (se) TC_REC(1, SE); else TC_REC(1, MATERN); }
+  else         { if (se) TC_REC(2, SE); else TC_REC(2, MATERN); }
+#undef TC_REC
   if (refine) {
     // absolute error terms of the FP32 epilogue from the data (one small read-back):
     //   exponent  e = (Cx - Bz) + sum xx_k z_k : 12*D4+3 roundings (inputs and FMAs) of magnitudes <= T = |log2 sf2| + 2h(Ax + Az),
     //             k = ex2.approx(e) (2 ulp), cov = k - acc (1 rounding of <= 2 sf2)             -> e_abs
     //   mean      mu' = cov*a + m : two roundings of <= |m|max + beta*sqrt(sf2) (a*|cov| <= beta*sigma_z)   -> d_mu
     //   variance  t = s' - cov^2 b', compared with mu'^2 near mu'^2 ~ t <= beta^2 (s_z + sf2)     -> d_t
+    // Matern (records scaled by c, e = -c s <= 0, k = sf2 P(t) exp(-t) with t = sqrt(max(-e, 0))):
+    //   exponent  the same 12*D4+3 roundings, of magnitudes <= T = c (Ax + Az) (no log2 sf2 term).  |dk/de| = |dk/ds| / c
+    //             <= kappa sf2 / 2 with kappa = max_t ((1-2q) + q t) e^-t = 1 (3/2) or 1/3 (5/2), and the clamp at 0 only
+    //             moves e towards the true value: error in k <= kappa/2 sf2 u (12*D4+3) T
+    //   value     with t = sqrt(-e) exact, the FP32 evaluation adds at most 17.3 u sf2, taken as 32 u sf2: sqrt.approx
+    //             (<= 8 u relative in t; t |dk/dt| = sf2 t^2 ((1-2q) + q t) e^-t <= 0.61 sf2 -> 4.9 u), the argument -t log2(e)
+    //             (2 u relative -> ln2 * 2u t log2(e) relative in k; t P(t) e^-t <= 1.2 -> 2.4 u), ex2.approx (4 u),
+    //             the polynomial (3 u), the two products (2 u) and sf2 in FP32 (1 u): every t^j e^-t is bounded
+    //   cov = k - acc: one rounding of <= 2 sf2                                                   -> e_abs
     double st[4];
     SBO_CUDA(cudaMemcpyAsync(st, stats, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     SBO_CUDA(cudaStreamSynchronize(ctx->stream));
     double sf2max = 0.0, lsf = 0.0;
     for (int c = 0; c < nc; ++c) { sf2max = fmax(sf2max, fc.sf2[c]); lsf = fmax(lsf, fabs(log2(fc.sf2[c]))); }
     const double h = 0.5 * 1.4426950408889634, u = 5.9604644775390625e-08;           // u = 2^-24
-    const double T = lsf + 2.0 * h * (st[0] + st[1]);
-    ra.e_abs = (float)(sf2max * (0.6931471805599453 * u * (12 * D4 + 3) * T * 1.05 + 8.0 * u) + 4.0 * u * sf2max);
+    if (se) {
+      const double T = lsf + 2.0 * h * (st[0] + st[1]);
+      ra.e_abs = (float)(sf2max * (0.6931471805599453 * u * (12 * D4 + 3) * T * 1.05 + 8.0 * u) + 4.0 * u * sf2max);
+    } else {
+      const MATERN mk(fc.kernel);
+      const double kappa = mk.q > 0.0 ? 1.0 / 3.0 : 1.0;
+      const double T = mk.c * (st[0] + st[1]);
+      ra.e_abs = (float)(sf2max * (0.5 * kappa * u * (12 * D4 + 3) * T * 1.05 + 32.0 * u) + 4.0 * u * sf2max);
+    }
     ra.d_mu = (float)(4.0 * u * (st[2] + fc.beta * sqrt(sf2max)) + 1e-9);
     ra.d_t = (float)(8.0 * u * fc.beta * fc.beta * (st[3] + sf2max) + 1e-9);
   }
@@ -1124,6 +1116,7 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   if (variant < 0) variant = 5 | ((fc.npad <= 256 || D4 == 2) ? 2 : 0);
   if (refine) variant |= 7;        // the refining epilogue exists in the 2-CTA kernel only; it is heavier: 8 epilogue warps
   if (target) variant |= 4;        // so does the column-OR epilogue of the GoOSE target
+  if (!se) variant |= 4;           // and the Matern epilogue
   // tile geometry of the chosen kernel and the raster of its work items
   const bool two = (variant & 4) != 0;
   const int tile_x = two ? 2 * tc::BM : tc::BM, tile_z = (two || (variant & 1)) ? 256 : 128;
@@ -1142,7 +1135,8 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   ev_end(ctx);            // record prep = phase 6
   ev_begin(ctx, 4);       // the GEMM kernel alone = phase 4 (closed by the caller)
 #define TC_LAUNCH(BN_, D4_, EW_) SBO_TRY((tc::launch<BN_, D4_, EW_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm)))
-#define TC_LAUNCH2R(D4_, EW_, R_, T_) SBO_TRY((tc::launch2<D4_, EW_, R_, T_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm, gx, ra)))
+#define TC_LAUNCH2K(D4_, EW_, R_, T_, K_) SBO_TRY((tc::launch2<D4_, EW_, R_, T_, K_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm, gx, ra)))
+#define TC_LAUNCH2R(D4_, EW_, R_, T_) do { if (se) TC_LAUNCH2K(D4_, EW_, R_, T_, SE); else TC_LAUNCH2K(D4_, EW_, R_, T_, MATERN); } while (0)
 #define TC_LAUNCH2(D4_, EW_) do { if (target) { if (refine) TC_LAUNCH2R(D4_, EW_, true, true); else TC_LAUNCH2R(D4_, EW_, false, true); } \
                                   else if (refine) TC_LAUNCH2R(D4_, EW_, true, false); else TC_LAUNCH2R(D4_, EW_, false, false); } while (0)
   if (variant & 4) {            // 2-CTA pairs (cta_group::2), BN = 256
@@ -1165,6 +1159,7 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   }
 #undef TC_LAUNCH2
 #undef TC_LAUNCH2R
+#undef TC_LAUNCH2K
 #undef TC_LAUNCH
   return SBO_OK;
 }

@@ -1,4 +1,4 @@
-// model.cu -- model upload: K_i = sf2*exp(-1/2 dist) + (sn2+eps_f32) I, blocked Cholesky K = L L^T,
+// model.cu -- model upload: K_i = k_i(X, X) + (sn2+eps_f32) I (SE or Matern, common.cuh), blocked Cholesky K = L L^T,
 // W = L^-1 (lower-triangular inverse) and alpha = K^-1 (Y_i - m0_i), all FP64 on the device.
 // Replaces the host-side jnp.linalg.inv(Kopt) of models/GP_Safe.py:226-232 for the grid path.
 #include "common.cuh"
@@ -8,7 +8,9 @@
 #define NB 32   // factorisation block size
 
 // K[g][r][c], padded to npad: identity on the padded diagonal so the padded matrix stays SPD.
+template <class KC>
 __global__ void k_build_K(ModelSpec ms, double* __restrict__ K) {
+  const KC kc(ms.kernel);
   const int g = blockIdx.z;
   const int r = blockIdx.y * blockDim.y + threadIdx.y;
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -20,7 +22,7 @@ __global__ void k_build_K(ModelSpec ms, double* __restrict__ K) {
       const double df = ms.Xn[r * ms.d + k] - ms.Xn[c * ms.d + k];
       s += df * df * ms.inv_ell[g][k];
     }
-    v = ms.sf2[g] * exp(-0.5 * s);
+    v = kc.value(s, ms.sf2[g]);
     if (r == c) v += ms.sn2[g];
   } else {
     v = (r == c) ? 1.0 : 0.0;
@@ -170,18 +172,19 @@ __global__ void __launch_bounds__(256) k_alpha(ModelSpec ms, const double* __res
   }
 }
 
-int model_upload(sbo_ctx* ctx, int n, int d, int G, const double* X_norm, const double* Y_norm,
+int model_upload(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_norm, const double* Y_norm,
                  const double* X_mean, const double* X_std, const double* Y_mean, const double* Y_std,
                  const double* hyp) {
   SBO_REQUIRE(n >= 1 && n <= 16384, "n out of range");
   SBO_REQUIRE(d >= 1 && d <= SBO_MAX_D, "d out of range (1..8)");
   SBO_REQUIRE(G >= 1 && G <= SBO_MAX_G, "G out of range (1..8)");
   SBO_REQUIRE(X_norm && Y_norm && X_mean && X_std && Y_mean && Y_std && hyp, "null model pointer");
+  SBO_REQUIRE(kernel_valid(kernel), "unknown kernel (SBO_KERNEL_SE, SBO_KERNEL_MATERN32 or SBO_KERNEL_MATERN52)");
   ev_reset(ctx, 0);
   ev_begin(ctx, 0);
   ModelSpec& ms = ctx->ms;
   memset(&ms, 0, sizeof(ms));
-  ms.n = n; ms.d = d; ms.G = G;
+  ms.n = n; ms.d = d; ms.G = G; ms.kernel = kernel;
   ms.npad = (int)(cdiv(n, 128) * 128);   // multiple of the 128-row blocks of the DMMA solve kernel
   const int np = ms.npad;
   for (int k = 0; k < d; ++k) { ms.Xmean[k] = X_mean[k]; ms.Xstd[k] = X_std[k]; }
@@ -212,7 +215,7 @@ int model_upload(sbo_ctx* ctx, int n, int d, int G, const double* X_norm, const 
 
   {
     dim3 b(16, 16), g((unsigned)cdiv(np, 16), (unsigned)cdiv(np, 16), (unsigned)G);
-    k_build_K<<<g, b, 0, ctx->stream>>>(ms, K);
+    with_kernel(kernel, [&](auto kc) { k_build_K<decltype(kc)><<<g, b, 0, ctx->stream>>>(ms, K); });
     SBO_LAUNCH_CHECK();
   }
   const int nblk = np / NB;
@@ -258,8 +261,10 @@ int model_upload(sbo_ctx* ctx, int n, int d, int G, const double* X_norm, const 
 //   W' = L'^-1 = [[W, 0], [-(l^T W)/l_nn, 1/l_nn]] ,  alpha' = W'^T W' (y' - m0)            -- O(n^2) per GP.
 // One CTA per GP; rows n of the padded L and W (identity rows until now) are overwritten in place.
 // =============================================================================================
+template <class KC>
 __global__ void __launch_bounds__(256) k_append_row(ModelSpec ms, int n_old, double* __restrict__ Lm, double* __restrict__ Wm,
                                                     double* __restrict__ scratch, int* __restrict__ info) {
+  const KC kc(ms.kernel);
   __shared__ double red[8];
   __shared__ double s_lnn;
   const int g = blockIdx.x, np = ms.npad, d = ms.d;
@@ -272,7 +277,7 @@ __global__ void __launch_bounds__(256) k_append_row(ModelSpec ms, int n_old, dou
   for (int j = threadIdx.x; j < n_old; j += blockDim.x) {
     double s = 0.0;
     for (int k = 0; k < d; ++k) { const double df = ms.Xn[(size_t)j * d + k] - xnew[k]; s += df * df * ms.inv_ell[g][k]; }
-    kv[j] = ms.sf2[g] * exp(-0.5 * s);
+    kv[j] = kc.value(s, ms.sf2[g]);
   }
   __syncthreads();
   double part = 0.0;
@@ -350,7 +355,9 @@ int model_append(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_ne
   ctx->Yn = nY;
   SBO_TRY(sbo_ensure(ctx, ctx->pp_k, sizeof(double) * (size_t)G * 2 * np));
   SBO_CUDA(cudaMemsetAsync(ctx->info.p, 0, sizeof(int) * SBO_MAX_G, ctx->stream));
-  k_append_row<<<G, 256, 0, ctx->stream>>>(ms, n, (double*)ctx->Kmat.p, (double*)ctx->W.p, (double*)ctx->pp_k.p, (int*)ctx->info.p);
+  with_kernel(ms.kernel, [&](auto kc) {
+    k_append_row<decltype(kc)><<<G, 256, 0, ctx->stream>>>(ms, n, (double*)ctx->Kmat.p, (double*)ctx->W.p, (double*)ctx->pp_k.p, (int*)ctx->info.p);
+  });
   SBO_LAUNCH_CHECK();
   ms.n = n + 1;
   k_alpha<<<G, 256, 0, ctx->stream>>>(ms, (const double*)ctx->Yn.p, (double*)ctx->alpha.p + (size_t)G * np, (double*)ctx->alpha.p);
@@ -371,15 +378,17 @@ int model_append(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_ne
 
 // =============================================================================================
 // Batched negative log-likelihood for the hyper-parameter fit (SURVEY.md section 8f row 2).
-//   GP.negative_loglikelihood (models/GP_Safe.py:169-192):  K = sf2*exp(-1/2 dist) + (sn2 + 1e-8) I,
+//   GP.negative_loglikelihood (models/GP_Safe.py:169-192):  K = k(X, X) + (sn2 + 1e-8) I,
 //   NLL = y^T K^-1 y + log det K = |L^-1 y|^2 + 2 sum log L_ii   with K = L L^T.
 // The reference evaluates it once per DE individual on the host (GP_Safe.py:224); here a whole DE population
 // (P hyper-parameter vectors) is factorised in one batch with the blocked-Cholesky kernels above (batch index in the
 // place of the GP index).
 // =============================================================================================
 // hyp[p][0..d) = 1/2 log ell_k, hyp[p][d] = 1/2 log sf2, hyp[p][d+1] = 1/2 log sn2      (GP_Safe.py:180-182)
-__global__ void k_build_K_pop(int n, int npad, int d, const double* __restrict__ Xn, const double* __restrict__ hyp,
+template <class KC>
+__global__ void k_build_K_pop(int kernel, int n, int npad, int d, const double* __restrict__ Xn, const double* __restrict__ hyp,
                               double* __restrict__ K) {
+  const KC kc(kernel);
   const int p = blockIdx.z;
   const int r = blockIdx.y * blockDim.y + threadIdx.y;
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -392,7 +401,7 @@ __global__ void k_build_K_pop(int n, int npad, int d, const double* __restrict__
       const double df = Xn[r * d + k] - Xn[c * d + k];
       s += df * df / exp(2.0 * h[k]);
     }
-    v = exp(2.0 * h[d]) * exp(-0.5 * s);
+    v = kc.value(s, exp(2.0 * h[d]));
     if (r == c) v += exp(2.0 * h[d + 1]) + 1e-8;                       // GP_Safe.py:184
   } else {
     v = (r == c) ? 1.0 : 0.0;
@@ -445,11 +454,12 @@ __global__ void __launch_bounds__(256) k_nll_finish(int n, int npad, const doubl
   }
 }
 
-int nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll) {
+int nll_batch(sbo_ctx* ctx, int kernel, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll) {
   SBO_REQUIRE(n >= 1 && n <= 8192, "n out of range");
   SBO_REQUIRE(d >= 1 && d <= SBO_MAX_D, "d out of range (1..8)");
   SBO_REQUIRE(P >= 1 && P <= 65535, "population size out of range (1..65535)");
   SBO_REQUIRE(X_norm && y && hyp && nll, "null pointer");
+  SBO_REQUIRE(kernel_valid(kernel), "unknown kernel (SBO_KERNEL_SE, SBO_KERNEL_MATERN32 or SBO_KERNEL_MATERN52)");
   const int np = (int)(cdiv(n, NB) * NB);
   const size_t kbytes = sizeof(double) * (size_t)P * np * np;
   SBO_TRY(sbo_ensure(ctx, ctx->nll_K, kbytes));
@@ -466,7 +476,7 @@ int nll_batch(sbo_ctx* ctx, int n, int d, const double* X_norm, const double* y,
   double* K = (double*)ctx->nll_K.p;
   {
     dim3 b(16, 16), g((unsigned)cdiv(np, 16), (unsigned)cdiv(np, 16), (unsigned)P);
-    k_build_K_pop<<<g, b, 0, ctx->stream>>>(n, np, d, Xd, hd, K);
+    with_kernel(kernel, [&](auto kc) { k_build_K_pop<decltype(kc)><<<g, b, 0, ctx->stream>>>(kernel, n, np, d, Xd, hd, K); });
     SBO_LAUNCH_CHECK();
   }
   const int nblk = np / NB;

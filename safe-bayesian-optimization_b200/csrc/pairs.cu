@@ -620,7 +620,7 @@ k_union_count(int nc, const uint32_t* __restrict__ masks, long long nwords, unsi
 // =============================================================================================
 #define FB 64
 #define FK 16
-template <int D, bool TARGET>   // TARGET: GoOSE target epilogue (column OR into hit_words)
+template <int D, bool TARGET, class KC>   // TARGET: GoOSE target epilogue (column OR into hit_words); KC: covariance function
 __global__ void __launch_bounds__(256)
 k_fantasy_f64(FantasyConsts fc, long long nx, long long nz, long long nxp, long long nzp,
               const double* __restrict__ Vx, const double* __restrict__ Vz,
@@ -632,6 +632,7 @@ k_fantasy_f64(FantasyConsts fc, long long nx, long long nz, long long nxp, long 
   __shared__ double Bs[FK][FB + 1];   // x rows
   __shared__ int cnt[16][FB];
   __shared__ uint32_t hw[FB / 32];    // GoOSE target: the block's z rows made safe by some valid x column
+  const KC kc(fc.kernel);
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
   const long long zb = (long long)blockIdx.x * FB, xb = (long long)blockIdx.y * FB;
   if (key_x) {   // exact pruning (see k_key_z): no pair of this block can become safe when min key_z > max key_x
@@ -706,7 +707,7 @@ k_fantasy_f64(FantasyConsts fc, long long nx, long long nz, long long nxp, long 
         double s = 0.0;
 #pragma unroll
         for (int k = 0; k < D; ++k) { const double df = zc[i][k] - xc[j][k]; s += df * df * fc.inv_ell[c][k]; }
-        const double cc = fc.sf2[c] * exp(-0.5 * s) - acc[i][j];
+        const double cc = kc.value(s, fc.sf2[c]) - acc[i][j];
         const double mu = m_z + cc * a_x;
         const double s2 = s_z - cc * cc * b_x;
         const bool ok = (mu - fc.beta * sqrt(fmax(s2, 0.0))) >= 0.0;
@@ -784,10 +785,11 @@ __device__ __forceinline__ void fd_dmma(double& c0, double& c1, double a, double
                : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
-template <int D, bool TARGET>   // TARGET: GoOSE target epilogue (column OR into a.hit_words)
+template <int D, bool TARGET, class KC>   // TARGET: GoOSE target epilogue (column OR into a.hit_words); KC: covariance function
 __global__ void __launch_bounds__(256, 2)
 k_fantasy_dmma(FantasyConsts fc, DmmaArgs a) {
   extern __shared__ __align__(16) double fsm[];
+  const KC kc(fc.kernel);
   const int RC = D + 2 * fc.nc;                       // constants per row / column: xn[D] | a[nc] | b[nc]  (zn | m | s)
   double* rowc = fsm + FD_STAGES * FD_STAGE_D;        // [FD_BM][RC]
   double* colc = rowc + FD_BM * RC;                   // [FD_BN][RC]
@@ -883,7 +885,7 @@ k_fantasy_dmma(FantasyConsts fc, DmmaArgs a) {
           double s = 0.0;
 #pragma unroll
           for (int k = 0; k < D; ++k) { const double df = cz[k] - rx[k]; s += df * df * fc.inv_ell[c][k]; }
-          const double cc = sf2 * exp(-0.5 * s) - acc[i][j][e];
+          const double cc = kc.value(s, sf2) - acc[i][j][e];
           const double mu = cz[D + c] + cc * a_x;
           const double s2 = cz[D + nc + c] - cc * cc * b_x;
           if (!((mu - beta * sqrt(fmax(s2, 0.0))) >= 0.0)) okbits &= ~(1u << ((i * 4 + j) * 2 + e));
@@ -991,7 +993,7 @@ k_cell_scatter(long long n, const int2* __restrict__ list, CellPlan p, const int
 
 // one warp per ambiguous pair of list[0..n_amb).  Vx / Vz hold the FP64 rows of the ranks [x0, x0 + mx) / [z0, z0 + mz_)
 // (one cell: all ranks, offsets 0)
-template <int D, bool TARGET>   // TARGET: GoOSE target (safe pairs set their z's bit in hit_words)
+template <int D, bool TARGET, class KC>   // TARGET: GoOSE target (safe pairs set their z's bit in hit_words); KC: covariance function
 __global__ void __launch_bounds__(256)
 k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list, long long nx, long long nz, long long mx, long long mz_,
                long long x0, long long z0, const int* __restrict__ rank_x, const int* __restrict__ rank_z,
@@ -1002,6 +1004,7 @@ k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list,
                uint32_t* __restrict__ hit_words) {
   const long long w = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (w >= n_amb) return;
+  const KC kc(fc.kernel);
   const int lane = threadIdx.x & 31;
   const int2 e = list[w];
   const long long xi = e.x, zi = e.y;
@@ -1020,7 +1023,7 @@ k_refine_pairs(FantasyConsts fc, long long n_amb, const int2* __restrict__ list,
     double s = 0.0;
 #pragma unroll
     for (int k = 0; k < D; ++k) { const double df = zn[(size_t)k * nz + zi] - xn[(size_t)k * nx + xi]; s += df * df * fc.inv_ell[c][k]; }
-    const double cc = fc.sf2[c] * exp(-0.5 * s) - acc;
+    const double cc = kc.value(s, fc.sf2[c]) - acc;
     const double mu = mz[(size_t)c * nz + zi] + cc * ax[(size_t)c * nx + xi];
     const double s2 = sz[(size_t)c * nz + zi] - cc * cc * bx[(size_t)c * nx + xi];
     ok = (mu - fc.beta * sqrt(fmax(s2, 0.0))) >= 0.0;
@@ -1042,8 +1045,8 @@ static int launch_refine(sbo_ctx* ctx, const FantasyConsts& fc, long long n, con
   const double* xn = (const double*)ctx->aux_x.p; const double* ax = xn + (size_t)d * nx; const double* bx = ax + (size_t)nc * nx;
   const double* zn = (const double*)ctx->aux_z.p; const double* mz = zn + (size_t)d * nz; const double* sz = mz + (size_t)nc * nz;
   unsigned long long* nsafe = (unsigned long long*)ctx->amb_ctr.p + 1;
-#define RPT(DD, T) k_refine_pairs<DD, T><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0, (const int*)ctx->amb_rx.p, \
-      (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe, hit_words)
+#define RPT(DD, T) with_kernel(fc.kernel, [&](auto kc) { k_refine_pairs<DD, T, decltype(kc)><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0, (const int*)ctx->amb_rx.p, \
+      (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe, hit_words); })
 #define RP(DD) do { if (hit_words) RPT(DD, true); else RPT(DD, false); } while (0)
   switch (d) { case 1: RP(1); break; case 2: RP(2); break; case 3: RP(3); break; case 4: RP(4); break;
                case 5: RP(5); break; case 6: RP(6); break; case 7: RP(7); break; default: RP(8); break; }
@@ -1530,7 +1533,7 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
     ps.counted = true;
   } else {
     FantasyConsts fc{};
-    fc.nc = nc; fc.d = d; fc.npad = ms.npad; fc.beta = ps.beta;
+    fc.nc = nc; fc.d = d; fc.npad = ms.npad; fc.kernel = ms.kernel; fc.beta = ps.beta;
     for (int c = 0; c < nc; ++c) {
       fc.sf2[c] = ms.sf2[c + 1]; fc.sn2[c] = ms.sn2[c + 1];
       for (int k = 0; k < d; ++k) fc.inv_ell[c][k] = ms.inv_ell[c + 1][k];
@@ -1559,13 +1562,15 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
       const size_t smem = sizeof(double) * ((size_t)FD_STAGES * FD_STAGE_D + (size_t)(FD_BM + FD_BN) * RC);
       ev_begin(ctx, 4);
       if (da.n_items > 0) {
-#define FDLT(DD, T) do { SBO_CUDA(cudaFuncSetAttribute(k_fantasy_dmma<DD, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-                        k_fantasy_dmma<DD, T><<<(unsigned)da.n_items, 256, smem, ctx->stream>>>(fc, da); } while (0)
+#define FDLK(DD, T, K) do { SBO_CUDA(cudaFuncSetAttribute(k_fantasy_dmma<DD, T, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+                           k_fantasy_dmma<DD, T, K><<<(unsigned)da.n_items, 256, smem, ctx->stream>>>(fc, da); } while (0)
+#define FDLT(DD, T) do { if (fc.kernel == SBO_KERNEL_SE) FDLK(DD, T, SE); else FDLK(DD, T, MATERN); } while (0)
 #define FDL(DD) do { if (hitw) FDLT(DD, true); else FDLT(DD, false); } while (0)
         switch (d) { case 1: FDL(1); break; case 2: FDL(2); break; case 3: FDL(3); break; case 4: FDL(4); break;
                      case 5: FDL(5); break; case 6: FDL(6); break; case 7: FDL(7); break; default: FDL(8); break; }
 #undef FDL
 #undef FDLT
+#undef FDLK
         SBO_LAUNCH_CHECK();
       }
       ps.pairs_evaluated = da.n_items * (long long)FD_BM * FD_BN * nc;
@@ -1574,7 +1579,7 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
 
       SBO_REQUIRE(grid.y <= 65535, "too many candidates for the FP64 fantasy kernel");
       ev_begin(ctx, 4);
-#define FLT(DD, T) k_fantasy_f64<DD, T><<<grid, 256, 0, ctx->stream>>>(fc, nx, nz, nxp, nzp, (const double*)ctx->vx.p, (const double*)ctx->vz.p, xn, ax, bx, zn, mz, sz, cnt, key_x, key_z, row_perm, ctr, hitw)
+#define FLT(DD, T) with_kernel(fc.kernel, [&](auto kc) { k_fantasy_f64<DD, T, decltype(kc)><<<grid, 256, 0, ctx->stream>>>(fc, nx, nz, nxp, nzp, (const double*)ctx->vx.p, (const double*)ctx->vz.p, xn, ax, bx, zn, mz, sz, cnt, key_x, key_z, row_perm, ctr, hitw); })
 #define FL(DD) do { if (hitw) FLT(DD, true); else FLT(DD, false); } while (0)
       switch (d) { case 1: FL(1); break; case 2: FL(2); break; case 3: FL(3); break; case 4: FL(4); break;
                    case 5: FL(5); break; case 6: FL(6); break; case 7: FL(7); break; default: FL(8); break; }

@@ -1,6 +1,6 @@
 // posterior.cu -- GP posterior over the candidate grid (models/GP_Safe.py:310-352 vmapped, as in
 // test/test_SafeOpt.py:324-338), trsm form:
-//   k_j   = sf2 * exp(-1/2 sum_k (Xn_jk - xn_k)^2 / ell_k)                 (K1a, fused SE-ARD cross-covariance)
+//   k_j   = k(s_j),  s_j = sum_k (Xn_jk - xn_k)^2 / ell_k  (SE or Matern)  (K1a, fused ARD cross-covariance)
 //   mean  = (m0 + k . alpha) * Ystd + Ymean                                 (K1a epilogue)
 //   grad  = d mean / d x (analytic), L_i = max_p ||grad||_inf               (K1c, optional)
 //   v     = W k  (W = L^-1 lower triangular),  var = max(0, sf2 - |v|^2) * Ystd^2   (K1b)
@@ -52,7 +52,7 @@ k_build_tables(ModelSpec ms, GridSpec gs, TabSpec ts, double* __restrict__ tab) 
 // ---------------------------------------------------------------------------------------------
 // K1a: cross-covariance tile -> Kx scratch [G][npad][P] (points contiguous), mean, optional gradient
 // ---------------------------------------------------------------------------------------------
-template <int D>
+template <int D, class KC>
 __global__ void __launch_bounds__(XC_THREADS)
 k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __restrict__ Kx,
            double* __restrict__ mean_out, long long out_ld, double* __restrict__ gradmax,
@@ -60,6 +60,7 @@ k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __
   __shared__ double Xs[XC_JT * D];
   __shared__ double As[XC_JT];
   __shared__ double red[XC_THREADS / 32];
+  const KC kc(ms.kernel);
   const int g = blockIdx.y + ms.g0;
   const int pl = blockIdx.x * XC_THREADS + threadIdx.x;
   const bool in_chunk = pl < P;
@@ -113,13 +114,14 @@ k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __
 #pragma unroll
             for (int k = 1; k < D; ++k) kv *= __ldg(trow[k] + (size_t)(j0 + j) * ts.pts[k]);
           } else {
-            kv = sf2 * exp(-0.5 * s);                                            // GP_Safe.py:165-166
+            kv = kc.value(s, sf2);                                               // GP_Safe.py:165-166
           }
           const double w = As[j] * kv;
           acc += w;
           if (want_grad) {
+            const double wg = KC::kIsSE ? w : As[j] * kc.phi(s, sf2);           // dk/dx_k = -phi df_k / ell_k (SE: phi = k)
 #pragma unroll
-            for (int k = 0; k < D; ++k) gk[k] += w * df[k];
+            for (int k = 0; k < D; ++k) gk[k] += wg * df[k];
           }
         }
         if (Kx) kcol[(size_t)(j0 + j) * P] = kv;
@@ -561,8 +563,10 @@ static void launch_crosscov(sbo_ctx* ctx, const GridSpec& gs, long long p0, int 
   const int g0 = ctx->post_g0;
   ModelSpec msl = ctx->ms; msl.g0 = g0;
   dim3 grid((unsigned)cdiv(P, XC_THREADS), (unsigned)(ctx->ms.G - g0));
-  k_crosscov<D><<<grid, XC_THREADS, 0, ctx->stream>>>(msl, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax,
-                                                      grad_out, grad_gp, ts);
+  with_kernel(msl.kernel, [&](auto kc) {
+    k_crosscov<D, decltype(kc)><<<grid, XC_THREADS, 0, ctx->stream>>>(msl, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax,
+                                                                      grad_out, grad_gp, ts);
+  });
 }
 
 static int crosscov_dispatch(sbo_ctx* ctx, const GridSpec& gs, long long p0, int P, int valid, double* Kx,
@@ -685,7 +689,9 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   SBO_TRY(sbo_ensure(ctx, ctx->var, sizeof(double) * (size_t)ms.G * count));
   SBO_TRY(sbo_ensure(ctx, ctx->lmax, sizeof(double) * SBO_MAX_G));
   // meshgrid + DMMA variant: fused path, no cross-covariance scratch at all (one "chunk" = the whole shard)
-  const bool fused = ctx->gs.kind == 1 && ctx->opt_posterior_variant == 1 && ctx->opt_posterior_fused;
+  // the separable factor tables exist for the SE kernel only: a Matern model ignores "posterior_fused" / "posterior_tables"
+  const bool separable = ctx->gs.kind == 1 && ms.kernel == SBO_KERNEL_SE;
+  const bool fused = separable && ctx->opt_posterior_variant == 1 && ctx->opt_posterior_fused;
   const long long P = fused ? cdiv(count, 128) * 128 : chunk_points(ctx, ms, count);
   if (!fused) SBO_TRY(sbo_ensure(ctx, ctx->kx, sizeof(double) * (size_t)ms.G * ms.npad * P));
   ctx->keep_v = 0;
@@ -698,7 +704,7 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   // meshgrids: the cross-covariance kernel takes its kernel values from the separable factor tables (d loads + d-1
   // multiplies instead of an FP64 exp per entry) whether or not the solve is fused
   TabSpec ts{};
-  if (ctx->gs.kind == 1 && (fused || ctx->opt_posterior_tables)) {
+  if (separable && (fused || ctx->opt_posterior_tables)) {
     ev_begin(ctx, 1);
     SBO_TRY(build_tables(ctx, &ts));
     ev_end(ctx);

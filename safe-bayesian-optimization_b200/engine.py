@@ -21,6 +21,13 @@ def _f64(a):
     return np.ascontiguousarray(np.asarray(a, dtype=np.float64))
 
 
+def kernel_id(kernel):
+    """enum sbo_kernel of a covariance function name ('RBF', 'Matern32', 'Matern52')."""
+    if kernel not in capi.KERNELS:
+        raise ValueError(f"unknown kernel {kernel!r}: expected one of {', '.join(capi.KERNELS)}")
+    return capi.KERNELS[kernel]
+
+
 def unpack_bits(words, count):
     """uint32 little-endian bit words -> bool array of length count."""
     b = np.unpackbits(np.ascontiguousarray(words).view(np.uint8), bitorder="little")
@@ -105,16 +112,18 @@ class GridEngine:
         return out
 
     # -- model ------------------------------------------------------------------------------
-    def set_model(self, ds):
-        """Upload ``inference_datasets`` (models/GP_Safe.py:236-245).  invKopt is not needed."""
+    def set_model(self, ds, kernel="RBF"):
+        """Upload ``inference_datasets`` (models/GP_Safe.py:236-245) with the covariance function ``kernel`` ('RBF',
+        'Matern32' or 'Matern52').  invKopt is not needed."""
+        kid = kernel_id(kernel)
         Xn, Yn, hyp = _f64(ds["X_norm"]), _f64(ds["Y_norm"]), _f64(ds["hypopt"])
         n, d = Xn.shape
         G = Yn.shape[1]
         if hyp.shape != (d + 2, G):
             raise ValueError("ERROR W and X_norm dimension should be same")   # GP_Safe.py:134-135
         xm, xs, ym, ys = _f64(ds["X_mean"]), _f64(ds["X_std"]), _f64(ds["Y_mean"]), _f64(ds["Y_std"])
-        self._ck(self._lib.sbo_set_model(self._h, n, d, G, capi.dptr(Xn), capi.dptr(Yn), capi.dptr(xm), capi.dptr(xs),
-                                         capi.dptr(ym), capi.dptr(ys), capi.dptr(hyp)))
+        self._ck(self._lib.sbo_set_model_ex(self._h, kid, n, d, G, capi.dptr(Xn), capi.dptr(Yn), capi.dptr(xm), capi.dptr(xs),
+                                            capi.dptr(ym), capi.dptr(ys), capi.dptr(hyp)))
         self.n, self.d, self.G = n, d, G
 
     def append_sample(self, x_norm_new, y_norm_new):
@@ -136,14 +145,15 @@ class GridEngine:
         self._ck(self._lib.sbo_stable_minmax(self._h, int(n_controlled), kind, float(beta), C.byref(idx), C.byref(val), C.byref(cnt), sp))
         return (idx.value, val.value, cnt.value, sc) if want_scores else (idx.value, val.value, cnt.value)
 
-    def nll_batch(self, X_norm, y, hyp_pop):
+    def nll_batch(self, X_norm, y, hyp_pop, kernel="RBF"):
         """GP.negative_loglikelihood (GP_Safe.py:169-192) for a population: hyp_pop (P, d+2) -> nll (P,)."""
+        kid = kernel_id(kernel)
         Xn, yv, hp = _f64(X_norm), _f64(y).reshape(-1), _f64(hyp_pop)
         n, d = Xn.shape
         if hp.ndim != 2 or hp.shape[1] != d + 2 or yv.shape[0] != n:
             raise ValueError("hyp_pop must be (P, d+2) and y (n,)")
         out = np.empty(hp.shape[0])
-        self._ck(self._lib.sbo_nll_batch(self._h, n, d, capi.dptr(Xn), capi.dptr(yv), hp.shape[0], capi.dptr(hp), capi.dptr(out)))
+        self._ck(self._lib.sbo_nll_batch_ex(self._h, kid, n, d, capi.dptr(Xn), capi.dptr(yv), hp.shape[0], capi.dptr(hp), capi.dptr(out)))
         return out
 
     def get_model(self):
@@ -394,11 +404,12 @@ class GridEngine:
             out["minimizer_std"] = float(np.sqrt(out["minimizer_var"])) if out["minimizer_idx"] >= 0 else 0.0
         return out
 
-    def safeopt_step_sharded(self, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True):
+    def safeopt_step_sharded(self, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True,
+                             kernel="RBF"):
         """One SafeOpt step on a grid sharded over the ranks of the library's communicator (sbo_comm_init); the
         collectives run inside the library.  Every rank returns the same global result."""
         if upload:
-            self.set_model(ds)
+            self.set_model(ds, kernel)
         prec, _ = capi.PRECISIONS[precision]
         r = capi.StepResult()
         Lp = capi.dptr(_f64(L)) if L is not None else None
@@ -406,9 +417,10 @@ class GridEngine:
                                                     int(prec), int(unsafe_rule), Lp, C.byref(r)))
         return self._step_dict(r, False)
 
-    def goose_step_sharded(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, mode="lipschitz", precision="fp64"):
+    def goose_step_sharded(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, mode="lipschitz", precision="fp64",
+                           kernel="RBF"):
         if upload:
-            self.set_model(ds)
+            self.set_model(ds, kernel)
         prec, _ = capi.PRECISIONS[precision]
         r = capi.StepResult()
         Lp = capi.dptr(_f64(L)) if L is not None else None
@@ -418,11 +430,11 @@ class GridEngine:
 
     # -- whole steps (drivers' decision rules) ------------------------------------------------
     def safeopt_step(self, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=capi.UNSAFE_ALL, L=None,
-                     upload=True):
+                     upload=True, kernel="RBF"):
         """model upload -> posterior -> sets -> L -> expander pairs -> arg-reductions -> x_new.
         Decision rule of test/test_SafeOpt.py:144-158.  Returns a dict of scalars/indices."""
         if upload:
-            self.set_model(ds)
+            self.set_model(ds, kernel)
         fantasy = mode == "fantasy"
         prec, kv = capi.PRECISIONS[precision]
         keep_v = kv if fantasy else 0
@@ -444,11 +456,12 @@ class GridEngine:
         out["x_new_idx"] = s["minimizer_idx"] if out["minimizer_std"] > out["expander_std"] else ex["best_idx"]
         return out
 
-    def goose_step(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, mode="lipschitz", precision="fp64"):
+    def goose_step(self, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, mode="lipschitz", precision="fp64",
+                   kernel="RBF"):
         """Decision rule of test/test_GoOSE.py:151-162.  mode="fantasy": the target set comes from the fantasy pair test
         (GP update with y_i = ucb_i(x)) at `precision`; L is not used."""
         if upload:
-            self.set_model(ds)
+            self.set_model(ds, kernel)
         fantasy = mode == "fantasy"
         prec, kv = capi.PRECISIONS[precision]
         self.posterior(with_grad=not fantasy and L is None, keep_v=kv if fantasy else 0, fetch=False)

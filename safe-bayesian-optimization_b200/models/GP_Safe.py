@@ -15,6 +15,8 @@ from scipy.optimize import differential_evolution
 from ._boot import package
 
 _EPS_F32 = float(np.finfo(np.float32).eps)
+# covariance functions: the reference's 'RBF' (squared exponential) and, additively, Matern 3/2 and 5/2
+KERNELS = ('RBF', 'Matern32', 'Matern52')
 
 
 class GP:
@@ -43,7 +45,7 @@ class GP:
         key = (id(ds), self._version if ds is self.inference_datasets else None,
                id(ds.get("hypopt")), id(ds.get("X_norm")))
         if self._uploaded != key:
-            self.engine.set_model(ds)
+            self.engine.set_model(ds, self.kernel)
             self._uploaded = key
             self._on_model_changed()
 
@@ -80,12 +82,18 @@ class GP:
         return -2 * np.dot(Xa, Ya.T) + np.sum(Xa ** 2, axis=1)[:, None] + np.sum(Ya ** 2, axis=1)
 
     def Cov_mat(self, kernel, X_norm, Y_norm, W, sf2):
-        """GP_Safe.py:122-143."""
+        """GP_Safe.py:122-143.  s = squared distance scaled by W;  'RBF': sf2 exp(-s/2),  'Matern32': sf2 (1 + t) exp(-t)
+        with t = sqrt(3 s),  'Matern52': sf2 (1 + t + t^2/3) exp(-t) with t = sqrt(5 s)."""
         if W.shape[0] != X_norm.shape[1]:
             raise ValueError('ERROR W and X_norm dimension should be same')
-        elif kernel != 'RBF':
+        elif kernel not in KERNELS:
             raise ValueError('ERROR no kernel with name ', kernel)
-        return sf2 * np.exp(-0.5 * self.squared_seuclidean_jax(X_norm, Y_norm, W))
+        s = self.squared_seuclidean_jax(X_norm, Y_norm, W)
+        if kernel == 'RBF':
+            return sf2 * np.exp(-0.5 * s)
+        t = np.sqrt((3.0 if kernel == 'Matern32' else 5.0) * np.maximum(s, 0.0))   # the expanded square can round below 0
+        poly = 1.0 + t if kernel == 'Matern32' else 1.0 + t + t * t / 3.0
+        return sf2 * poly * np.exp(-t)
 
     def calc_Cov_mat(self, kernel, X_norm, x_norm, ell, sf2):
         """GP_Safe.py:146-167."""
@@ -119,7 +127,7 @@ class GP:
                 # GPU factorises the S covariance matrices in one batch; 'deferred' updating is what vectorised
                 # evaluation implies, so the search path (not the objective) differs from the reference's
                 yi = np.ascontiguousarray(Y_norm[:, i])
-                res = differential_evolution(lambda H: self.engine.nll_batch(X_norm, yi, np.atleast_2d(H.T)),
+                res = differential_evolution(lambda H: self.engine.nll_batch(X_norm, yi, np.atleast_2d(H.T), self.kernel),
                                              bounds=bounds, vectorized=True, updating='deferred', **kw)
             else:
                 res = differential_evolution(self.negative_loglikelihood, args=(X_norm, Y_norm[:, i:i + 1]),
@@ -155,9 +163,10 @@ class GP:
 
     # ------------------------------------------------------------------ initialisation / update
     def GP_initialization(self, X, Y, kernel, multi_hyper, var_out=True, hypopt=None):
-        """GP_Safe.py:251-277.  ``hypopt`` (additive, optional) skips the fit."""
+        """GP_Safe.py:251-277.  ``kernel``: 'RBF' as in the reference, or (additive) 'Matern32' / 'Matern52'.
+        ``hypopt`` (additive, optional) skips the fit."""
         self.X, self.Y, self.kernel = np.asarray(X, dtype=np.float64), np.asarray(Y, dtype=np.float64), kernel
-        if kernel != 'RBF':
+        if kernel not in KERNELS:
             raise ValueError('ERROR no kernel with name ', kernel)
         self.n_point, self.nx_dim = self.X.shape[0], self.X.shape[1]
         self.ny_dim = self.Y.shape[1]

@@ -134,9 +134,12 @@ def first_best(per_value, per_idx, maximize):
 # ---------------------------------------------------------------------------------------------
 # stages shared by the SafeOpt and GoOSE steps
 # ---------------------------------------------------------------------------------------------
-def _posterior_and_sets(eng, ds, beta, unsafe_rule, with_grad, keep_v, upload, device, group, need_pass2=True):
+def _posterior_and_sets(eng, ds, beta, unsafe_rule, with_grad, keep_v, upload, device, group, need_pass2=True, kernel="RBF"):
     if upload:
-        eng.set_model(ds)
+        if kernel == "RBF":
+            eng.set_model(ds)             # the one-argument form keeps engines that only know the SE kernel usable here
+        else:
+            eng.set_model(ds, kernel)
     eng.posterior(with_grad=with_grad, keep_v=keep_v, fetch=False)
     s1 = eng.sets_pass1(beta, unsafe_rule)
     (min_ucb0, min_ucb0_idx), (min_lcb0, min_lcb0_idx) = reduce_arg(
@@ -253,15 +256,16 @@ def _pairs(eng, mode, prec, beta, L, goose, device, group, want_counts=False):
 # whole steps (same decision rules as GridEngine.safeopt_step / goose_step)
 # ---------------------------------------------------------------------------------------------
 def safeopt_step(eng, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True,
-                 device=None, group=None):
+                 device=None, group=None, kernel="RBF"):
     """test/test_SafeOpt.py:144-158 on a sharded grid.  Every rank returns the same global result."""
     if getattr(eng, "comm_ready", False) and group is None:
-        return eng.safeopt_step_sharded(ds, beta, mode=mode, precision=precision, unsafe_rule=unsafe_rule, L=L, upload=upload)
+        return eng.safeopt_step_sharded(ds, beta, mode=mode, precision=precision, unsafe_rule=unsafe_rule, L=L, upload=upload,
+                                        kernel=kernel)
     device = torch.device("cuda", eng.device) if device is None else device
     fantasy = mode == "fantasy"
     prec, kv = capi.PRECISIONS[precision]
     out = _posterior_and_sets(eng, ds, beta, unsafe_rule, with_grad=(not fantasy and L is None),
-                              keep_v=kv if fantasy else 0, upload=upload, device=device, group=group)
+                              keep_v=kv if fantasy else 0, upload=upload, device=device, group=group, kernel=kernel)
     out["minimizer_std"] = float(np.sqrt(out["minimizer_var"])) if out["minimizer_idx"] >= 0 else 0.0
     if fantasy:
         ex = _pairs(eng, capi.MODE_FANTASY, prec, beta, None, False, device, group)
@@ -277,16 +281,17 @@ def safeopt_step(eng, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=
 
 
 def goose_step(eng, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, device=None, group=None, coords=None,
-               mode="lipschitz", precision="fp64"):
+               mode="lipschitz", precision="fp64", kernel="RBF"):
     """test/test_GoOSE.py:151-162 on a sharded grid.  mode="fantasy": candidate and V rows are exchanged as in the
     SafeOpt fantasy step, then every rank decides its own unsafe points (no result all-reduce)."""
     if getattr(eng, "comm_ready", False) and group is None:
-        return eng.goose_step_sharded(ds, beta, unsafe_rule=unsafe_rule, L=L, upload=upload, mode=mode, precision=precision)
+        return eng.goose_step_sharded(ds, beta, unsafe_rule=unsafe_rule, L=L, upload=upload, mode=mode, precision=precision,
+                                      kernel=kernel)
     device = torch.device("cuda", eng.device) if device is None else device
     fantasy = mode == "fantasy"
     prec, kv = capi.PRECISIONS[precision]
     out = _posterior_and_sets(eng, ds, beta, unsafe_rule, with_grad=(not fantasy and L is None), keep_v=kv if fantasy else 0,
-                              upload=upload, device=device, group=group, need_pass2=False)
+                              upload=upload, device=device, group=group, need_pass2=False, kernel=kernel)
     if fantasy:
         tg = _pairs(eng, capi.MODE_FANTASY, prec, beta, None, True, device, group)
     else:
