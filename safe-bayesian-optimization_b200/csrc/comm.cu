@@ -292,7 +292,7 @@ int sbo_safeopt_step_sharded(sbo_ctx* ctx, double beta, int mode, int precision,
   memset(out, 0, sizeof(*out));
   const int G = ctx->ms.G;
   const bool fantasy = mode == SBO_MODE_FANTASY;
-  const int keep_v = fantasy ? (precision == SBO_PREC_FP64 ? 1 : (precision == SBO_PREC_TF32 ? 2 : 3)) : 0;
+  const int keep_v = fantasy ? keep_v_of(precision) : 0;
   sbo_sets_result s2;
   SBO_TRY(sharded_sets(ctx, beta, unsafe_rule, (!fantasy && !L) ? 1 : 0, keep_v, &s2, out));
   double Lg[SBO_MAX_G];
@@ -319,7 +319,7 @@ int sbo_goose_step_sharded_ex(sbo_ctx* ctx, double beta, int mode, int precision
   const int G = ctx->ms.G;
   const bool fantasy = mode == SBO_MODE_FANTASY;
   // fantasy: V rows kept at the GEMM's precision and no gradient, as in sbo_safeopt_step_sharded
-  const int keep_v = fantasy ? (precision == SBO_PREC_FP64 ? 1 : (precision == SBO_PREC_TF32 ? 2 : 3)) : 0;
+  const int keep_v = fantasy ? keep_v_of(precision) : 0;
   SBO_TRY(sharded_sets(ctx, beta, unsafe_rule, (!fantasy && !L) ? 1 : 0, keep_v, nullptr, out));
   double Lg[SBO_MAX_G];
   for (int i = 0; i < SBO_MAX_G; ++i) Lg[i] = L ? (i < G ? L[i] : 0.0) : out->L[G - 1];   // GoOSE.py:100

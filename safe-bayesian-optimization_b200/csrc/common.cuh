@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string>
+#include <type_traits>
 #include <vector>
 #include "../../include/sbo_b200.h"
 
@@ -175,11 +176,31 @@ static inline double kernel_rec_scale(int kernel) {
 static inline bool kernel_valid(int kernel) {
   return kernel == SBO_KERNEL_SE || kernel == SBO_KERNEL_MATERN32 || kernel == SBO_KERNEL_MATERN52;
 }
-// host: f(SE{}) or f(MATERN{kernel}) -- f launches the instantiation of its kernel class
+// Host-side compile-time dispatch: each helper calls f with a value that names one template argument and returns what
+// f returns, so nested calls select one kernel instantiation and can hand back an SBO status.
+// f(SE{}) or f(MATERN{kernel}) -- f launches the instantiation of its kernel class
 template <class F>
-static inline void with_kernel(int kernel, F&& f) {
-  if (kernel == SBO_KERNEL_SE) f(SE(kernel));
-  else f(MATERN(kernel));
+static inline auto with_kernel(int kernel, F&& f) {
+  if (kernel == SBO_KERNEL_SE) return f(SE(kernel));
+  return f(MATERN(kernel));
+}
+// f(std::integral_constant<int, v>{}) for v in [LO, HI]; any other v takes HI (callers validate v)
+template <int LO, int HI, class F>
+static inline auto with_int(int v, F&& f) {
+  if constexpr (LO < HI) {
+    if (v != LO) return with_int<LO + 1, HI>(v, f);
+  }
+  return f(std::integral_constant<int, LO>{});
+}
+// f(std::true_type{}) or f(std::false_type{})
+template <class F>
+static inline auto with_flag(bool b, F&& f) {
+  if (b) return f(std::true_type{});
+  return f(std::false_type{});
+}
+// keep_v of the posterior whose V rows the fantasy pair test of this precision reads
+static inline int keep_v_of(int precision) {
+  return precision == SBO_PREC_FP64 ? 1 : (precision == SBO_PREC_TF32 ? 2 : 3);
 }
 
 // (value, index) pairs with lowest-index tie-break

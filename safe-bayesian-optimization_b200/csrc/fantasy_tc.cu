@@ -908,28 +908,10 @@ static int make_map(sbo_ctx* ctx, CUtensorMap* map, const float* base, int rowle
   return SBO_OK;
 }
 
+// the attribute is per device and cheap: set before every launch (a process may hold contexts on several GPUs)
 template <int BN, int D4, int EW>
-static int launch(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx, long long nz, long long nxp, long long nzp,
-                  const float* Vx, const float* Vz, const float* rowrec, const float* colrec, int* counts, int* err,
-                  const long long* item_list, long long n_list, const int* row_perm) {
+static int launch(sbo_ctx* ctx, const CUtensorMap& tmA, const CUtensorMap& tmB, const Params& p, int sms) {
   using C = Cfg<BN, D4>;
-  CUtensorMap tmA, tmB;
-  const int rowlen = split ? 2 * fc.npad : fc.npad;
-  SBO_TRY(make_map(ctx, &tmA, Vx, rowlen, nxp, fc.nc, BM));
-  SBO_TRY(make_map(ctx, &tmB, Vz, rowlen, nzp, fc.nc, BN));
-  Params p{};
-  p.nc = fc.nc; p.nkb = fc.npad / BK; p.kblocks = split ? 3 * p.nkb : p.nkb; p.npad = fc.npad; p.split = split;
-  p.nx = nx; p.nz = nz; p.nxp = nxp; p.nzp = nzp;
-  p.nxt = (int)cdiv(nx, BM); p.nzt = (int)cdiv(nz, BN);
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
-  p.n_items = item_list ? n_list : cdiv(p.nxt, GX) * GX * (long long)p.nzt;
-  SBO_REQUIRE(p.n_items < 2000000000LL, "too many tile pairs for one launch");
-  p.rowrec = rowrec; p.colrec = colrec; p.counts = counts; p.err = err;
-  p.sched_counter = (unsigned int*)(err + 1);
-  p.item_list = item_list; p.row_perm = row_perm;
-  if (p.n_items == 0) return SBO_OK;
-  // per device and cheap: set before every launch (a process may hold contexts on several GPUs)
   SBO_CUDA(cudaFuncSetAttribute(k_fantasy_tc<BN, D4, EW>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
   const int grid = (int)((p.n_items < sms) ? p.n_items : sms);
   k_fantasy_tc<BN, D4, EW><<<grid, 128 + 32 * EW, C::SMEM_BYTES, ctx->stream>>>(tmA, tmB, p);
@@ -937,35 +919,10 @@ static int launch(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx
   return SBO_OK;
 }
 
-struct RefineArgs { int2* list; unsigned long long* count; long long cap; float e_abs, d_mu, d_t; int* rows; uint32_t* hit_words; uint32_t* amb_words; };
-
 template <int D4, int EW, bool REFINE, bool TARGET, class KC>
-static int launch2(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long nx, long long nz, long long nxp, long long nzp,
-                   const float* Vx, const float* Vz, const float* rowrec, const float* colrec, int* counts, int* err,
-                   const long long* item_list, long long n_list, const int* row_perm, int gx, const RefineArgs& ra) {
+static int launch2(sbo_ctx* ctx, const CUtensorMap& tmA, const CUtensorMap& tmB, const Params& p, int sms) {
   using C = Cfg2<D4>;
-  CUtensorMap tmA, tmB;
-  const int rowlen = split ? 2 * fc.npad : fc.npad;
-  SBO_TRY(make_map(ctx, &tmA, Vx, rowlen, nxp, fc.nc, BM));
-  SBO_TRY(make_map(ctx, &tmB, Vz, rowlen, nzp, fc.nc, C::BN / 2));
-  Params p{};
-  p.nc = fc.nc; p.nkb = fc.npad / BK; p.kblocks = split ? 3 * p.nkb : p.nkb; p.npad = fc.npad; p.split = split;
-  p.nx = nx; p.nz = nz; p.nxp = nxp; p.nzp = nzp;
-  p.nxt = (int)cdiv(nx, 2 * BM); p.nzt = (int)cdiv(nz, C::BN);
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device);
   const int clusters = sms / 2;
-  p.gx = gx;
-  p.n_items = item_list ? n_list : cdiv(p.nxt, p.gx) * p.gx * (long long)p.nzt;
-  SBO_REQUIRE(p.n_items < 2000000000LL, "too many tile pairs for one launch");
-  p.rowrec = rowrec; p.colrec = colrec; p.counts = counts; p.err = err;
-  p.sched_counter = (unsigned int*)(err + 1);
-  p.item_list = item_list; p.row_perm = row_perm;
-  p.amb_list = ra.list; p.amb_count = ra.count; p.amb_cap = ra.cap; p.amb_rows = ra.rows; p.e_abs = ra.e_abs; p.d_mu = ra.d_mu; p.d_t = ra.d_t;
-  p.hit_words = ra.hit_words; p.amb_words = ra.amb_words;
-  p.kernel = fc.kernel;
-  for (int c = 0; c < fc.nc; ++c) p.ksf2[c] = (float)fc.sf2[c];
-  if (p.n_items == 0) return SBO_OK;
   SBO_CUDA((cudaFuncSetAttribute(k_fantasy_tc2<D4, EW, REFINE, TARGET, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES)));
   const int grid = 2 * (int)((p.n_items < clusters) ? p.n_items : clusters);
   k_fantasy_tc2<D4, EW, REFINE, TARGET, KC><<<grid, 128 + 32 * EW, C::SMEM_BYTES, ctx->stream>>>(tmA, tmB, p);
@@ -1055,26 +1012,25 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   const bool refine = pr && pr->refine;
   const double c1 = refine ? ((split ? 9.5367431640625e-07 : 9.7680091857910156e-04) + (fc.npad / 8) * 1.1920928955078125e-07) : 0.0;
   const double esc = refine ? sqrt(c1) : 0.0;
-  tc::RefineArgs ra{};
+  tc::Params p{};
   const bool target = pr && pr->hit_words;
-  ra.hit_words = target ? pr->hit_words : nullptr;
+  p.hit_words = target ? pr->hit_words : nullptr;
   unsigned long long* stats = nullptr;
   if (refine) {
-    ra.list = pr->amb_list; ra.count = pr->amb_count; ra.cap = pr->amb_cap; ra.rows = pr->amb_rows; ra.amb_words = pr->amb_words;
+    p.amb_list = pr->amb_list; p.amb_count = pr->amb_count; p.amb_cap = pr->amb_cap; p.amb_rows = pr->amb_rows; p.amb_words = pr->amb_words;
     SBO_TRY(sbo_ensure(ctx, ctx->tc_stats, 4 * sizeof(unsigned long long)));
     stats = (unsigned long long*)ctx->tc_stats.p;
     SBO_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), ctx->stream));
   }
   ev_begin(ctx, 6);
   const bool se = fc.kernel == SBO_KERNEL_SE;
-#define TC_REC(D4_, KC_) do { \
-    tc::k_tc_records<D4_, KC_><<<dim3((unsigned)cdiv(nxp, 256), nc), 256, 0, ctx->stream>>>(fc, nx, nxp, 1, xn, ax, bx, rowrec, esc, stats); \
-    SBO_LAUNCH_CHECK(); \
-    tc::k_tc_records<D4_, KC_><<<dim3((unsigned)cdiv(nzp, 256), nc), 256, 0, ctx->stream>>>(fc, nz, nzp, 0, zn, mz, sz, colrec, esc, stats); \
-    SBO_LAUNCH_CHECK(); } while (0)
-  if (D4 == 1) { if (se) TC_REC(1, SE); else TC_REC(1, MATERN); }
-  else         { if (se) TC_REC(2, SE); else TC_REC(2, MATERN); }
-#undef TC_REC
+  SBO_TRY((with_int<1, 2>(D4, [&](auto d4) { return with_kernel(fc.kernel, [&](auto kc) -> int {
+    tc::k_tc_records<d4, decltype(kc)><<<dim3((unsigned)cdiv(nxp, 256), nc), 256, 0, ctx->stream>>>(fc, nx, nxp, 1, xn, ax, bx, rowrec, esc, stats);
+    SBO_LAUNCH_CHECK();
+    tc::k_tc_records<d4, decltype(kc)><<<dim3((unsigned)cdiv(nzp, 256), nc), 256, 0, ctx->stream>>>(fc, nz, nzp, 0, zn, mz, sz, colrec, esc, stats);
+    SBO_LAUNCH_CHECK();
+    return SBO_OK;
+  }); })));
   if (refine) {
     // absolute error terms of the FP32 epilogue from the data (one small read-back):
     //   exponent  e = (Cx - Bz) + sum xx_k z_k : 12*D4+3 roundings (inputs and FMAs) of magnitudes <= T = |log2 sf2| + 2h(Ax + Az),
@@ -1098,15 +1054,15 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
     const double h = 0.5 * 1.4426950408889634, u = 5.9604644775390625e-08;           // u = 2^-24
     if (se) {
       const double T = lsf + 2.0 * h * (st[0] + st[1]);
-      ra.e_abs = (float)(sf2max * (0.6931471805599453 * u * (12 * D4 + 3) * T * 1.05 + 8.0 * u) + 4.0 * u * sf2max);
+      p.e_abs = (float)(sf2max * (0.6931471805599453 * u * (12 * D4 + 3) * T * 1.05 + 8.0 * u) + 4.0 * u * sf2max);
     } else {
       const MATERN mk(fc.kernel);
       const double kappa = mk.q > 0.0 ? 1.0 / 3.0 : 1.0;
       const double T = mk.c * (st[0] + st[1]);
-      ra.e_abs = (float)(sf2max * (0.5 * kappa * u * (12 * D4 + 3) * T * 1.05 + 32.0 * u) + 4.0 * u * sf2max);
+      p.e_abs = (float)(sf2max * (0.5 * kappa * u * (12 * D4 + 3) * T * 1.05 + 32.0 * u) + 4.0 * u * sf2max);
     }
-    ra.d_mu = (float)(4.0 * u * (st[2] + fc.beta * sqrt(sf2max)) + 1e-9);
-    ra.d_t = (float)(8.0 * u * fc.beta * fc.beta * (st[3] + sf2max) + 1e-9);
+    p.d_mu = (float)(4.0 * u * (st[2] + fc.beta * sqrt(sf2max)) + 1e-9);
+    p.d_t = (float)(8.0 * u * fc.beta * fc.beta * (st[3] + sf2max) + 1e-9);
   }
   int* err = (int*)ctx->tc_err.p;
   // variant: bit 0: BN = 256, bit 1: 8 epilogue warps, bit 2: 2-CTA pairs (cta_group::2, 256 x 256 tile pairs);
@@ -1134,32 +1090,25 @@ int fantasy_tc_run(sbo_ctx* ctx, const FantasyConsts& fc, int split, long long n
   if (pr && pr->items_run) *pr->items_run = n_list * (long long)tile_x * tile_z;   // pairs per constraint actually evaluated
   ev_end(ctx);            // record prep = phase 6
   ev_begin(ctx, 4);       // the GEMM kernel alone = phase 4 (closed by the caller)
-#define TC_LAUNCH(BN_, D4_, EW_) SBO_TRY((tc::launch<BN_, D4_, EW_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm)))
-#define TC_LAUNCH2K(D4_, EW_, R_, T_, K_) SBO_TRY((tc::launch2<D4_, EW_, R_, T_, K_>(ctx, fc, split, nx, nz, nxp, nzp, Vx, Vz, rowrec, colrec, counts_c, err, item_list, n_list, row_perm, gx, ra)))
-#define TC_LAUNCH2R(D4_, EW_, R_, T_) do { if (se) TC_LAUNCH2K(D4_, EW_, R_, T_, SE); else TC_LAUNCH2K(D4_, EW_, R_, T_, MATERN); } while (0)
-#define TC_LAUNCH2(D4_, EW_) do { if (target) { if (refine) TC_LAUNCH2R(D4_, EW_, true, true); else TC_LAUNCH2R(D4_, EW_, false, true); } \
-                                  else if (refine) TC_LAUNCH2R(D4_, EW_, true, false); else TC_LAUNCH2R(D4_, EW_, false, false); } while (0)
-  if (variant & 4) {            // 2-CTA pairs (cta_group::2), BN = 256
-    if (D4 == 1) { if (variant & 2) TC_LAUNCH2(1, 8); else TC_LAUNCH2(1, 4); }
-    else         { if (variant & 2) TC_LAUNCH2(2, 8); else TC_LAUNCH2(2, 4); }
-  } else if (D4 == 1) {
-    switch (variant & 3) {
-      case 0: TC_LAUNCH(128, 1, 4); break;
-      case 1: TC_LAUNCH(256, 1, 4); break;
-      case 2: TC_LAUNCH(128, 1, 8); break;
-      default: TC_LAUNCH(256, 1, 8); break;
-    }
-  } else {
-    switch (variant & 3) {
-      case 0: TC_LAUNCH(128, 2, 4); break;
-      case 1: TC_LAUNCH(256, 2, 4); break;
-      case 2: TC_LAUNCH(128, 2, 8); break;
-      default: TC_LAUNCH(256, 2, 8); break;
-    }
-  }
-#undef TC_LAUNCH2
-#undef TC_LAUNCH2R
-#undef TC_LAUNCH2K
-#undef TC_LAUNCH
-  return SBO_OK;
+  // the TMA maps and the work of both kernels; a 2-CTA pair stages half of its z tile in each CTA
+  CUtensorMap tmA, tmB;
+  const int rowlen = split ? 2 * fc.npad : fc.npad;
+  SBO_TRY(tc::make_map(ctx, &tmA, Vx, rowlen, nxp, nc, tc::BM));
+  SBO_TRY(tc::make_map(ctx, &tmB, Vz, rowlen, nzp, nc, two ? tile_z / 2 : tile_z));
+  p.nc = nc; p.nkb = fc.npad / tc::BK; p.kblocks = split ? 3 * p.nkb : p.nkb; p.npad = fc.npad; p.split = split;
+  p.nx = nx; p.nz = nz; p.nxp = nxp; p.nzp = nzp;
+  p.nxt = nxt; p.nzt = nzt; p.gx = gx; p.n_items = n_list;
+  p.rowrec = rowrec; p.colrec = colrec; p.counts = counts_c; p.err = err;
+  p.sched_counter = (unsigned int*)(err + 1);
+  p.item_list = item_list; p.row_perm = row_perm;
+  p.kernel = fc.kernel;
+  for (int c = 0; c < nc; ++c) p.ksf2[c] = (float)fc.sf2[c];
+  if (p.n_items == 0) return SBO_OK;
+  return with_int<1, 2>(D4, [&](auto d4) { return with_flag(variant & 2, [&](auto ew8) {
+    if (two)            // 2-CTA pairs (cta_group::2), BN = 256
+      return with_flag(refine, [&](auto r) { return with_flag(target, [&](auto t) { return with_kernel(fc.kernel, [&](auto kc) {
+        return tc::launch2<d4, (ew8 ? 8 : 4), r, t, decltype(kc)>(ctx, tmA, tmB, p, sms);
+      }); }); });
+    return with_flag(variant & 1, [&](auto bn256) { return tc::launch<(bn256 ? 256 : 128), d4, (ew8 ? 8 : 4)>(ctx, tmA, tmB, p, sms); });
+  }); });
 }

@@ -1045,13 +1045,10 @@ static int launch_refine(sbo_ctx* ctx, const FantasyConsts& fc, long long n, con
   const double* xn = (const double*)ctx->aux_x.p; const double* ax = xn + (size_t)d * nx; const double* bx = ax + (size_t)nc * nx;
   const double* zn = (const double*)ctx->aux_z.p; const double* mz = zn + (size_t)d * nz; const double* sz = mz + (size_t)nc * nz;
   unsigned long long* nsafe = (unsigned long long*)ctx->amb_ctr.p + 1;
-#define RPT(DD, T) with_kernel(fc.kernel, [&](auto kc) { k_refine_pairs<DD, T, decltype(kc)><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0, (const int*)ctx->amb_rx.p, \
-      (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe, hit_words); })
-#define RP(DD) do { if (hit_words) RPT(DD, true); else RPT(DD, false); } while (0)
-  switch (d) { case 1: RP(1); break; case 2: RP(2); break; case 3: RP(3); break; case 4: RP(4); break;
-               case 5: RP(5); break; case 6: RP(6); break; case 7: RP(7); break; default: RP(8); break; }
-#undef RP
-#undef RPT
+  with_int<1, SBO_MAX_D>(d, [&](auto D) { with_flag(hit_words != nullptr, [&](auto T) { with_kernel(fc.kernel, [&](auto kc) {
+    k_refine_pairs<D, T, decltype(kc)><<<(unsigned)cdiv(n, 8), 256, 0, ctx->stream>>>(fc, n, list, nx, nz, mx, mz_, x0, z0,
+        (const int*)ctx->amb_rx.p, (const int*)ctx->amb_rz.p, Vx, Vz, xn, ax, bx, zn, mz, sz, counts, row_perm, nsafe, hit_words);
+  }); }); });
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }
@@ -1266,7 +1263,7 @@ int pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const doub
   } else {
     SBO_REQUIRE(nc >= 1, "fantasy expander needs at least one constraint GP");
     SBO_REQUIRE(precision == SBO_PREC_FP64 || precision == SBO_PREC_TF32 || precision == SBO_PREC_TF32X3, "bad precision");
-    SBO_REQUIRE(ctx->keep_v == (precision == SBO_PREC_FP64 ? 1 : (precision == SBO_PREC_TF32 ? 2 : 3)),
+    SBO_REQUIRE(ctx->keep_v == keep_v_of(precision),
                 "fantasy expander: run sbo_posterior with keep_v = 1 (FP64), 2 (TF32) or 3 (TF32x3) first");
   }
   ev_reset(ctx, 4); ev_reset(ctx, 6); ev_reset(ctx, 7);
@@ -1522,12 +1519,9 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
     unsigned char* hits = (unsigned char*)result_dev;
     if (nzr == 0) return SBO_OK;
     ev_begin(ctx, 4);
-#define LP(DD) SBO_TRY(launch_pairs<DD>(ctx, goose, pc, nx, nzr, xc, ucb, thr, zc, hits, ctr, stride, off, out_pos))
-    switch (d) {
-      case 1: LP(1); break; case 2: LP(2); break; case 3: LP(3); break; case 4: LP(4); break;
-      case 5: LP(5); break; case 6: LP(6); break; case 7: LP(7); break; default: LP(8); break;
-    }
-#undef LP
+    SBO_TRY((with_int<1, SBO_MAX_D>(d, [&](auto D) {
+      return launch_pairs<D>(ctx, goose, pc, nx, nzr, xc, ucb, thr, zc, hits, ctr, stride, off, out_pos);
+    })));
     SBO_LAUNCH_CHECK();
     ev_end(ctx);
     ps.counted = true;
@@ -1562,15 +1556,12 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
       const size_t smem = sizeof(double) * ((size_t)FD_STAGES * FD_STAGE_D + (size_t)(FD_BM + FD_BN) * RC);
       ev_begin(ctx, 4);
       if (da.n_items > 0) {
-#define FDLK(DD, T, K) do { SBO_CUDA(cudaFuncSetAttribute(k_fantasy_dmma<DD, T, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-                           k_fantasy_dmma<DD, T, K><<<(unsigned)da.n_items, 256, smem, ctx->stream>>>(fc, da); } while (0)
-#define FDLT(DD, T) do { if (fc.kernel == SBO_KERNEL_SE) FDLK(DD, T, SE); else FDLK(DD, T, MATERN); } while (0)
-#define FDL(DD) do { if (hitw) FDLT(DD, true); else FDLT(DD, false); } while (0)
-        switch (d) { case 1: FDL(1); break; case 2: FDL(2); break; case 3: FDL(3); break; case 4: FDL(4); break;
-                     case 5: FDL(5); break; case 6: FDL(6); break; case 7: FDL(7); break; default: FDL(8); break; }
-#undef FDL
-#undef FDLT
-#undef FDLK
+        SBO_TRY((with_int<1, SBO_MAX_D>(d, [&](auto D) { return with_flag(hitw != nullptr, [&](auto T) {
+          return with_kernel(fc.kernel, [&](auto kc) -> int {
+            SBO_CUDA(cudaFuncSetAttribute(k_fantasy_dmma<D, T, decltype(kc)>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            k_fantasy_dmma<D, T, decltype(kc)><<<(unsigned)da.n_items, 256, smem, ctx->stream>>>(fc, da);
+            return SBO_OK;
+          }); }); })));
         SBO_LAUNCH_CHECK();
       }
       ps.pairs_evaluated = da.n_items * (long long)FD_BM * FD_BN * nc;
@@ -1579,12 +1570,10 @@ int pairs_run(sbo_ctx* ctx, int goose, void* result_dev) {
 
       SBO_REQUIRE(grid.y <= 65535, "too many candidates for the FP64 fantasy kernel");
       ev_begin(ctx, 4);
-#define FLT(DD, T) with_kernel(fc.kernel, [&](auto kc) { k_fantasy_f64<DD, T, decltype(kc)><<<grid, 256, 0, ctx->stream>>>(fc, nx, nz, nxp, nzp, (const double*)ctx->vx.p, (const double*)ctx->vz.p, xn, ax, bx, zn, mz, sz, cnt, key_x, key_z, row_perm, ctr, hitw); })
-#define FL(DD) do { if (hitw) FLT(DD, true); else FLT(DD, false); } while (0)
-      switch (d) { case 1: FL(1); break; case 2: FL(2); break; case 3: FL(3); break; case 4: FL(4); break;
-                   case 5: FL(5); break; case 6: FL(6); break; case 7: FL(7); break; default: FL(8); break; }
-#undef FL
-#undef FLT
+      with_int<1, SBO_MAX_D>(d, [&](auto D) { with_flag(hitw != nullptr, [&](auto T) { with_kernel(fc.kernel, [&](auto kc) {
+        k_fantasy_f64<D, T, decltype(kc)><<<grid, 256, 0, ctx->stream>>>(fc, nx, nz, nxp, nzp, (const double*)ctx->vx.p,
+            (const double*)ctx->vz.p, xn, ax, bx, zn, mz, sz, cnt, key_x, key_z, row_perm, ctr, hitw);
+      }); }); });
       SBO_LAUNCH_CHECK();
       ps.counted = true;          // pairs evaluated = ctr[0] * nc (read back in finish)
       ps.count_scale = nc;

@@ -557,31 +557,16 @@ k_solve_fused(ModelSpec ms, GridSpec gs, TabSpec ts, int EMIT, long long p0, int
 // ---------------------------------------------------------------------------------------------
 // host drivers
 // ---------------------------------------------------------------------------------------------
-template <int D>
-static void launch_crosscov(sbo_ctx* ctx, const GridSpec& gs, long long p0, int P, int valid, double* Kx,
-                            double* mean_out, long long out_ld, double* gradmax, double* grad_out, int grad_gp, const TabSpec& ts) {
-  const int g0 = ctx->post_g0;
-  ModelSpec msl = ctx->ms; msl.g0 = g0;
-  dim3 grid((unsigned)cdiv(P, XC_THREADS), (unsigned)(ctx->ms.G - g0));
-  with_kernel(msl.kernel, [&](auto kc) {
-    k_crosscov<D, decltype(kc)><<<grid, XC_THREADS, 0, ctx->stream>>>(msl, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax,
-                                                                      grad_out, grad_gp, ts);
-  });
-}
-
 static int crosscov_dispatch(sbo_ctx* ctx, const GridSpec& gs, long long p0, int P, int valid, double* Kx,
                              double* mean_out, long long out_ld, double* gradmax, double* grad_out, int grad_gp,
                              const TabSpec& ts = TabSpec{}) {
-  switch (ctx->ms.d) {
-    case 1: launch_crosscov<1>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    case 2: launch_crosscov<2>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    case 3: launch_crosscov<3>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    case 4: launch_crosscov<4>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    case 5: launch_crosscov<5>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    case 6: launch_crosscov<6>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    case 7: launch_crosscov<7>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-    default: launch_crosscov<8>(ctx, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax, grad_out, grad_gp, ts); break;
-  }
+  const int g0 = ctx->post_g0;
+  ModelSpec msl = ctx->ms; msl.g0 = g0;
+  dim3 grid((unsigned)cdiv(P, XC_THREADS), (unsigned)(ctx->ms.G - g0));
+  with_int<1, SBO_MAX_D>(msl.d, [&](auto D) { with_kernel(msl.kernel, [&](auto kc) {
+    k_crosscov<D, decltype(kc)><<<grid, XC_THREADS, 0, ctx->stream>>>(msl, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax,
+                                                                      grad_out, grad_gp, ts);
+  }); });
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }
@@ -590,29 +575,20 @@ static int solve_dispatch(sbo_ctx* ctx, const double* Kx, int P, long long p0, i
                           long long out_ld, int keep_v, void* vall, long long v_count) {
   const int g0 = ctx->post_g0;
   ModelSpec msl = ctx->ms; msl.g0 = g0;
-  if (ctx->opt_posterior_variant == 1) {   // FP64 tensor-core (DMMA) kernel
-    dim3 grid((unsigned)(P / DV_BP), (unsigned)(ctx->ms.G - g0));
-    // the attribute is per device and a process may hold contexts on several GPUs: set it before every launch
-    SBO_CUDA(cudaFuncSetAttribute(k_solve_var_dmma<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM));
-    SBO_CUDA(cudaFuncSetAttribute(k_solve_var_dmma<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM));
-    SBO_CUDA(cudaFuncSetAttribute(k_solve_var_dmma<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM));
-    SBO_CUDA(cudaFuncSetAttribute(k_solve_var_dmma<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM));
-    if (keep_v == 1) k_solve_var_dmma<1><<<grid, 256, DV_SMEM, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, vall, v_count);
-    else if (keep_v == 2) k_solve_var_dmma<2><<<grid, 256, DV_SMEM, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, vall, v_count);
-    else if (keep_v == 3) k_solve_var_dmma<3><<<grid, 256, DV_SMEM, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, vall, v_count);
-    else k_solve_var_dmma<0><<<grid, 256, DV_SMEM, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, nullptr, 0);
-    SBO_LAUNCH_CHECK();
+  SBO_TRY((with_int<0, 3>(keep_v, [&](auto EMIT) -> int {
+    void* v = EMIT ? vall : nullptr;
+    const long long vc = EMIT ? v_count : 0;
+    if (ctx->opt_posterior_variant == 1) {   // FP64 tensor-core (DMMA) kernel
+      dim3 grid((unsigned)(P / DV_BP), (unsigned)(ctx->ms.G - g0));
+      // the attribute is per device and a process may hold contexts on several GPUs: set it before every launch
+      SBO_CUDA(cudaFuncSetAttribute(k_solve_var_dmma<EMIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM));
+      k_solve_var_dmma<EMIT><<<grid, 256, DV_SMEM, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, v, vc);
+    } else {
+      dim3 grid((unsigned)(P / PB_BP), (unsigned)(ctx->ms.G - g0));
+      k_solve_var<EMIT><<<grid, 256, 0, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, v, vc);
+    }
     return SBO_OK;
-  }
-  dim3 grid((unsigned)(P / PB_BP), (unsigned)(ctx->ms.G - g0));
-  if (keep_v == 1)
-    k_solve_var<1><<<grid, 256, 0, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, vall, v_count);
-  else if (keep_v == 2)
-    k_solve_var<2><<<grid, 256, 0, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, vall, v_count);
-  else if (keep_v == 3)
-    k_solve_var<3><<<grid, 256, 0, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, vall, v_count);
-  else
-    k_solve_var<0><<<grid, 256, 0, ctx->stream>>>(msl, Kx, P, p0, valid, var_out, out_ld, nullptr, 0);
+  })));
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }
@@ -635,25 +611,14 @@ static int build_tables(sbo_ctx* ctx, TabSpec* ts) {
   return SBO_OK;
 }
 
-template <int D>
-static void launch_fused(sbo_ctx* ctx, const TabSpec& ts, int emit, long long p0, int P, int valid, double* var_out, long long out_ld,
-                         void* vall, long long v_count) {
-  dim3 grid((unsigned)(P / DV_BP), (unsigned)ctx->ms.G);
-  cudaFuncSetAttribute(k_solve_fused<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM_F);
-  k_solve_fused<D><<<grid, 256, DV_SMEM_F, ctx->stream>>>(ctx->ms, ctx->gs, ts, emit, p0, valid, var_out, out_ld, vall, v_count);
-}
 static int fused_dispatch(sbo_ctx* ctx, const TabSpec& ts, int emit, long long p0, int P, int valid, double* var_out, long long out_ld,
                           void* vall, long long v_count) {
-  switch (ctx->ms.d) {
-    case 1: launch_fused<1>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    case 2: launch_fused<2>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    case 3: launch_fused<3>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    case 4: launch_fused<4>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    case 5: launch_fused<5>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    case 6: launch_fused<6>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    case 7: launch_fused<7>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-    default: launch_fused<8>(ctx, ts, emit, p0, P, valid, var_out, out_ld, vall, v_count); break;
-  }
+  dim3 grid((unsigned)(P / DV_BP), (unsigned)ctx->ms.G);
+  SBO_TRY((with_int<1, SBO_MAX_D>(ctx->ms.d, [&](auto D) -> int {
+    SBO_CUDA(cudaFuncSetAttribute(k_solve_fused<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, DV_SMEM_F));
+    k_solve_fused<D><<<grid, 256, DV_SMEM_F, ctx->stream>>>(ctx->ms, ctx->gs, ts, emit, p0, valid, var_out, out_ld, vall, v_count);
+    return SBO_OK;
+  })));
   SBO_LAUNCH_CHECK();
   return SBO_OK;
 }

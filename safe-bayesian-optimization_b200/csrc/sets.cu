@@ -501,17 +501,17 @@ int sets_pass1(sbo_ctx* ctx, double beta, int rule, int strict, sbo_sets_result*
   ev_reset(ctx, 3);
   ev_begin(ctx, 3);
   SBO_CUDA(cudaMemsetAsync(ctx->result.p, 0, sizeof(SetsDeviceResult), ctx->stream));
-#define P1V(GG) k_sets_pass1_v4<GG><<<nblocks, ST, 0, ctx->stream>>>(count, ctx->gs, (const double*)ctx->mean.p, (const double*)ctx->var.p, \
-      beta, rule, strict, (uint32_t*)ctx->m_safe.p, (uint32_t*)ctx->m_unsafe.p, (SetsPartial*)ctx->partials.p)
-  if (vec) {
-    switch (ctx->ms.G) { case 1: P1V(1); break; case 2: P1V(2); break; case 3: P1V(3); break; case 4: P1V(4); break;
-                         case 5: P1V(5); break; case 6: P1V(6); break; case 7: P1V(7); break; default: P1V(8); break; }
-  } else
-#undef P1V
-  k_sets_pass1<<<nblocks, ST, 0, ctx->stream>>>(ctx->ms.G, count, ctx->gs, (const double*)ctx->mean.p,
-                                                (const double*)ctx->var.p, beta, rule, strict,
-                                                (uint32_t*)ctx->m_safe.p, (uint32_t*)ctx->m_unsafe.p,
-                                                (SetsPartial*)ctx->partials.p);
+  if (vec)
+    with_int<1, SBO_MAX_G>(ctx->ms.G, [&](auto G) {
+      k_sets_pass1_v4<G><<<nblocks, ST, 0, ctx->stream>>>(count, ctx->gs, (const double*)ctx->mean.p, (const double*)ctx->var.p,
+                                                          beta, rule, strict, (uint32_t*)ctx->m_safe.p, (uint32_t*)ctx->m_unsafe.p,
+                                                          (SetsPartial*)ctx->partials.p);
+    });
+  else
+    k_sets_pass1<<<nblocks, ST, 0, ctx->stream>>>(ctx->ms.G, count, ctx->gs, (const double*)ctx->mean.p,
+                                                  (const double*)ctx->var.p, beta, rule, strict,
+                                                  (uint32_t*)ctx->m_safe.p, (uint32_t*)ctx->m_unsafe.p,
+                                                  (SetsPartial*)ctx->partials.p);
   SBO_LAUNCH_CHECK();
   k_sets_final1<<<1, ST, 0, ctx->stream>>>((const SetsPartial*)ctx->partials.p, nblocks, (SetsDeviceResult*)ctx->result.p);
   SBO_LAUNCH_CHECK();
@@ -574,14 +574,10 @@ int argreduce_run(sbo_ctx* ctx, int kind, const uint32_t* mask_dev, const double
   const double* var = (const double*)ctx->var.p;
   ev_reset(ctx, 5);
   ev_begin(ctx, 5);
-#define AR_LAUNCH(K) k_argreduce<K><<<nblocks, ST, 0, ctx->stream>>>(ctx->gs, mean, var, ctx->beta, mask_dev, t[0], t[1], t[2], t[3], t[4], t[5], t[6], t[7], part)
-  switch (kind) {
-    case SBO_ARGMAX_VAR0: AR_LAUNCH(SBO_ARGMAX_VAR0); break;
-    case SBO_ARGMIN_LCB0: AR_LAUNCH(SBO_ARGMIN_LCB0); break;
-    case SBO_ARGMIN_UCB0: AR_LAUNCH(SBO_ARGMIN_UCB0); break;
-    default: AR_LAUNCH(SBO_ARGMIN_DIST); break;
-  }
-#undef AR_LAUNCH
+  with_int<SBO_ARGMAX_VAR0, SBO_ARGMIN_DIST>(kind, [&](auto K) {
+    k_argreduce<K><<<nblocks, ST, 0, ctx->stream>>>(ctx->gs, mean, var, ctx->beta, mask_dev, t[0], t[1], t[2], t[3], t[4], t[5], t[6],
+                                                    t[7], part);
+  });
   SBO_LAUNCH_CHECK();
   k_argreduce_final<<<1, ST, 0, ctx->stream>>>(part, nblocks, kind == SBO_ARGMAX_VAR0 ? 1 : 0, res);
   SBO_LAUNCH_CHECK();
