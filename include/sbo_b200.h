@@ -274,6 +274,41 @@ int sbo_goose_step_sharded(sbo_ctx* ctx, double beta, int unsafe_rule, const dou
 int sbo_goose_step_sharded_ex(sbo_ctx* ctx, double beta, int mode, int precision, int unsafe_rule, const double* L /* G or NULL */,
                               sbo_step_result* out);
 
+/* ---- batch SafeOpt acquisition: q safe query points per step (additive; no reference counterpart) -------------------
+ * GP-BUCB-style hallucination on the objective GP (index 0), in its normalised units.  The candidates are C = M u E of the
+ * last SafeOpt pair stage on the local shard (M = SBO_MASK_MIN; E = the union of its SBO_MASK_EXPANDER masks: Lipschitz mode
+ * one per constraint, fantasy mode which = 0, bounds mode the certified members).  S, M and E stay those of the real data,
+ * so every pick is in S.  After picks x_1..x_b (hallucinated observations with noise sn = exp(2 hyp[d+1, 0]) + eps_f32,
+ * whatever their values) the objective variance is the exact GP posterior variance
+ *   v_b(p) = max(0, v_{b-1}(p) - w_b(p)^2),   w_b(p) = (c(p, x_b) - sum_{j<b} R_bj w_j(p)) / R_bb,
+ *   c(p, x) = k(p, x) - k(X, p)^T K^-1 k(X, x),   [c(x_i, x_j)] + sn I = R R^T (lower Cholesky, one row per pick),
+ * v_0 = the step's var_0.  Pick b uses the decision rule of test/test_SafeOpt.py:153-158 on v_{b-1}: std_M = sqrt(max over M
+ * of var_0 in raw units) and std_E the same over E (lowest global index on ties); M's point if std_M > std_E, else E's; a
+ * set that is empty yields to the other.  Pick 1 is the step's x_new.  A point may be picked again (what the rule says at
+ * noise sn).  A batch reads the step's state and writes none of it: model, posterior, masks and pair results are unchanged.
+ * Every entry point needs a SafeOpt pair stage (sbo_expander or a sharded SafeOpt step, with sbo_sets_pass2) since the last
+ * model, grid, shard, posterior or set change, and fails with SBO_ERR_INVALID after a GoOSE target stage. */
+#define SBO_BATCH_MAX_Q 256   /* picks per batch */
+typedef struct sbo_batch_pick {
+  int64_t idx;                          /* global index of this pick; -1 = M and E both empty */
+  int32_t from_expander, pad;           /* 0: taken from M, 1: from E */
+  double  std_min; int64_t idx_min;     /* sqrt(max v * Y_std0^2) over M under the earlier picks (0 / -1 if empty) */
+  double  std_exp; int64_t idx_exp;     /* the same over E */
+} sbo_batch_pick;
+/* one GPU: q picks with no host synchronisation between them (about 3q launches, one copy to the host at the end).
+ * picks[q] out; *n_picked = q, or 0 when M and E are both empty (picks[0].idx = -1). */
+int sbo_safeopt_batch(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n_picked);
+/* the same in three steps for a grid sharded over ranks; the batch-side state is computed identically on every rank:
+ *   sbo_batch_prepare  compact this rank's candidates, v = var_0 (*n_candidates_local = |C| of the shard)
+ *   sbo_batch_local    this rank's optima for the next pick (GLOBAL indices; idx / from_expander apply the rule locally)
+ *                      -> the caller reduces (std, index) over the ranks (largest std, lowest index) and applies the rule
+ *   sbo_batch_commit   hallucinate an observation at the chosen GLOBAL index (the same on every rank); at most q commits */
+int sbo_batch_prepare(sbo_ctx* ctx, int q, int64_t* n_candidates_local);
+int sbo_batch_local(sbo_ctx* ctx, sbo_batch_pick* local_optima);
+int sbo_batch_commit(sbo_ctx* ctx, int64_t global_idx);
+/* the three steps over the library's communicator (sbo_comm_init): one small all-gather per pick; every rank gets the same picks */
+int sbo_safeopt_batch_sharded(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n_picked);
+
 /* ---- instrumentation ------------------------------------------------------------------------ */
 /* number of kernels this library launched on ctx since the last reset */
 int64_t sbo_kernel_launches(sbo_ctx* ctx, int reset);

@@ -23,6 +23,7 @@ ARGMAX_VAR0, ARGMIN_LCB0, ARGMIN_UCB0, ARGMIN_DIST = 0, 1, 2, 3
 MASK_SAFE, MASK_MIN, MASK_UNSAFE, MASK_USER, MASK_EXPANDER, MASK_TARGET = 0, 1, 2, 3, 4, 5
 # covariance function name (models/GP_Safe.GP kernel argument) -> enum sbo_kernel
 KERNELS = {"RBF": 0, "Matern32": 1, "Matern52": 2}
+BATCH_MAX_Q = 256                  # SBO_BATCH_MAX_Q: picks per batch acquisition
 PHASES = ("model", "crosscov", "solve", "sets", "pairs", "argreduce", "pair_prep", "refine")
 
 
@@ -49,6 +50,11 @@ class StepResult(C.Structure):
 
 class PairsInfo(C.Structure):
     _fields_ = [("n_x_local", C.c_int64), ("n_z_local", C.c_int64), ("row_doubles", C.c_int64), ("vrow_bytes", C.c_int64)]
+
+
+class BatchPick(C.Structure):
+    _fields_ = [("idx", C.c_int64), ("from_expander", C.c_int32), ("pad", C.c_int32),
+                ("std_min", C.c_double), ("idx_min", C.c_int64), ("std_exp", C.c_double), ("idx_exp", C.c_int64)]
 
 
 _P = C.c_void_p
@@ -103,6 +109,11 @@ SIGNATURES = {
     "sbo_safeopt_step_sharded": (C.c_int, [_P, C.c_double, C.c_int, C.c_int, C.c_int, _D, C.POINTER(StepResult)]),
     "sbo_goose_step_sharded": (C.c_int, [_P, C.c_double, C.c_int, _D, C.POINTER(StepResult)]),
     "sbo_goose_step_sharded_ex": (C.c_int, [_P, C.c_double, C.c_int, C.c_int, C.c_int, _D, C.POINTER(StepResult)]),
+    "sbo_safeopt_batch": (C.c_int, [_P, C.c_int, C.POINTER(BatchPick), C.POINTER(C.c_int)]),
+    "sbo_batch_prepare": (C.c_int, [_P, C.c_int, _I64]),
+    "sbo_batch_local": (C.c_int, [_P, C.POINTER(BatchPick)]),
+    "sbo_batch_commit": (C.c_int, [_P, C.c_int64]),
+    "sbo_safeopt_batch_sharded": (C.c_int, [_P, C.c_int, C.POINTER(BatchPick), C.POINTER(C.c_int)]),
     "sbo_kernel_launches": (C.c_int64, [_P, C.c_int]),
     "sbo_mem_peak": (C.c_int64, [_P, C.c_int]),
     "sbo_phase_ms": (C.c_int, [_P, C.c_int, _D]),

@@ -105,7 +105,8 @@ int sbo_destroy(sbo_ctx* ctx) {
                     &ctx->kx, &ctx->lmax, &ctx->vall, &ctx->tile_bb, &ctx->nll_K, &ctx->nll_in, &ctx->m_safe, &ctx->m_unsafe, &ctx->m_min, &ctx->m_user, &ctx->m_exp,
                     &ctx->m_tgt, &ctx->partials, &ctx->result, &ctx->scan_a, &ctx->scan_b, &ctx->xs_idx, &ctx->zs_idx,
                     &ctx->xs_pay, &ctx->zs_pay, &ctx->hits, &ctx->counts, &ctx->pairctr, &ctx->imp_rows, &ctx->vx, &ctx->vz,
-                    &ctx->aux_x, &ctx->aux_z, &ctx->pp_x, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->pp_g, &ctx->tc_row, &ctx->tc_col, &ctx->tc_err, &ctx->exp_rows, &ctx->exp_v, &ctx->key_x, &ctx->key_z, &ctx->perm_x, &ctx->perm_z, &ctx->sort_ws, &ctx->tile_keys, &ctx->item_mask, &ctx->item_list, &ctx->gz_mask, &ctx->gz_idx, &ctx->gz_pay, &ctx->st_score, &ctx->st_mask, &ctx->tabs, &ctx->tc_stats, &ctx->amb_list, &ctx->amb_ctr, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts, &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_rows, &ctx->m_und, &ctx->amb_cell, &ctx->amb_hist, &ctx->amb_tgt})
+                    &ctx->aux_x, &ctx->aux_z, &ctx->pp_x, &ctx->pp_m, &ctx->pp_v, &ctx->pp_k, &ctx->pp_g, &ctx->tc_row, &ctx->tc_col, &ctx->tc_err, &ctx->exp_rows, &ctx->exp_v, &ctx->key_x, &ctx->key_z, &ctx->perm_x, &ctx->perm_z, &ctx->sort_ws, &ctx->tile_keys, &ctx->item_mask, &ctx->item_list, &ctx->gz_mask, &ctx->gz_idx, &ctx->gz_pay, &ctx->st_score, &ctx->st_mask, &ctx->tabs, &ctx->tc_stats, &ctx->amb_list, &ctx->amb_ctr, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts, &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_rows, &ctx->m_und, &ctx->amb_cell, &ctx->amb_hist, &ctx->amb_tgt,
+                    &ctx->bt_mask, &ctx->bt_idx, &ctx->bt_flag, &ctx->bt_v, &ctx->bt_w, &ctx->bt_part, &ctx->bt_pick})
     free_buf(*b);
   ev_collect(ctx);
   for (cudaEvent_t e : ctx->evpool) cudaEventDestroy(e);
@@ -165,7 +166,7 @@ int sbo_get_model(sbo_ctx* ctx, double* L, double* W, double* alpha) {
   return SBO_OK;
 }
 
-static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = false; ctx->keep_v = 0; }
+static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = false; ctx->keep_v = 0; }
 
 int sbo_set_grid(sbo_ctx* ctx, int d, const int64_t* pts_per_dim, const double* lo, const double* hi) {
   ENTER();

@@ -342,4 +342,45 @@ int sbo_goose_step_sharded_ex(sbo_ctx* ctx, double beta, int mode, int precision
   return SBO_OK;
 }
 
+// batch SafeOpt acquisition (batch.cu) on the sharded grid: per pick one all-gather of the ranks' local optima, reduced on the
+// raw variances (largest, lowest index on ties) so that every rank commits the same global index
+int sbo_safeopt_batch_sharded(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n_picked) {
+  if (!ctx) return sbo_fail(nullptr, SBO_ERR_INVALID, "null context");
+  cudaSetDevice(ctx->device);
+  SBO_REQUIRE(ctx->comm != nullptr, "sbo_safeopt_batch_sharded: call sbo_comm_init first");
+  SBO_REQUIRE(picks && n_picked, "null result");
+  const int R = ctx->comm->nranks;
+  SBO_TRY(batch_prepare(ctx, q, nullptr));
+  std::vector<double> g;
+  int n = 0;
+  for (int b = 0; b < q; ++b) {
+    BatchRec loc;
+    SBO_TRY(batch_local(ctx, &loc));
+    double mine[4] = {loc.vmin, (double)loc.imin, loc.vexp, (double)loc.iexp};
+    SBO_TRY(gather_record(ctx, mine, 4, g));
+    BatchRec r;
+    int64_t im, ie;
+    reduce_arg(g, 4, R, 0, true, &r.vmin, &im);
+    reduce_arg(g, 4, R, 2, true, &r.vexp, &ie);
+    r.imin = im; r.iexp = ie;
+    const bool hm = r.imin >= 0, he = r.iexp >= 0;
+    if (!hm) r.vmin = 0.0;
+    if (!he) r.vexp = 0.0;
+    const bool take_min = hm && (!he || sqrt(r.vmin) > sqrt(r.vexp));    // test/test_SafeOpt.py:153-158, empty set yields
+    r.idx = take_min ? r.imin : r.iexp;
+    r.from_exp = (!take_min && he) ? 1 : 0;
+    r.pad = 0;
+    batch_pick_of(r, &picks[b]);
+    if (r.idx < 0) {                                  // M and E are empty on every rank, and stay so
+      for (int k = b + 1; k < q; ++k) picks[k] = picks[b];
+      break;
+    }
+    n = b + 1;
+    if (b + 1 < q) SBO_TRY(batch_commit(ctx, r.idx));
+  }
+  ctx->bt.prepared = false;
+  *n_picked = n;
+  return SBO_OK;
+}
+
 }  // extern "C"

@@ -244,6 +244,21 @@ struct PairStage {
   long long n_ambiguous = 0, n_refined_safe = 0;     // split-TF32 refinement statistics of the last run
 };
 
+// state of a batch SafeOpt acquisition (batch.cu)
+struct BatchRec {                 // device record of one pick: raw objective variances, GLOBAL indices (-1 = empty)
+  long long idx;
+  int from_exp, pad;
+  double vmin; long long imin;
+  double vexp; long long iexp;
+};
+struct BatchStage {
+  bool prepared = false;
+  int q = 0, b = 0;               // picks asked for / observations hallucinated so far
+  long long nc = 0;               // local candidates |C|
+  int nparts = 0;                 // block partials of the candidate kernel
+  long long gen = 0;              // exp_gen of the pair stage the batch was prepared on
+};
+
 struct sbo_comm;   // comm.cu: NCCL communicator + gathered buffers
 
 struct sbo_ctx {
@@ -271,6 +286,8 @@ struct sbo_ctx {
   DevBuf vall;               // [(G-1)][count][npad] rows of V for the constraints
   // sets
   bool have_sets = false, have_sets2 = false;
+  bool have_exp = false;     // the last pair stage was a SafeOpt expander on the current sets (m_exp valid; batch.cu needs it)
+  long long exp_gen = 0;     // counts those stages: a prepared batch belongs to one of them
   double beta = 0.0;
   DevBuf m_safe, m_unsafe, m_min, m_user, m_exp, m_tgt;
   DevBuf partials, result;
@@ -292,6 +309,8 @@ struct sbo_ctx {
   DevBuf st_score, st_mask;               // StableOpt: per-x_c worst-case score and robust-safe bitmask
   DevBuf gz_mask, gz_idx, gz_pay;         // all-gathered unsafe set of a sharded Lipschitz expander
   PairStage ps;
+  BatchStage bt;
+  DevBuf bt_mask, bt_idx, bt_flag, bt_v, bt_w, bt_part, bt_pick;   // batch: C = M u E, membership bits, v[C], w[q][C], partials, pick side
   // timing: event pairs are recorded without host syncs and summed per phase by ev_collect()
   struct EvPair { cudaEvent_t a, b; int phase; };
   std::vector<EvPair> evlog;
@@ -385,5 +404,9 @@ int pairs_set_global_unsafe(sbo_ctx* ctx, const void* gathered_words_dev, long l
 int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_dev, sbo_pair_result* out, int32_t* counts_host);
 int pairs_fantasy(sbo_ctx* ctx, int precision, double beta, sbo_pair_result* out, int32_t* counts_host);
 int pairs_goose_fantasy(sbo_ctx* ctx, int precision, double beta, sbo_pair_result* out);
+int batch_prepare(sbo_ctx* ctx, int q, long long* n_candidates);
+int batch_local(sbo_ctx* ctx, BatchRec* out);
+int batch_commit(sbo_ctx* ctx, long long global_idx);
+void batch_pick_of(const BatchRec& r, sbo_batch_pick* out);
 uint32_t* mask_ptr(sbo_ctx* ctx, int mask_kind, int which);
 long long mask_words(const sbo_ctx* ctx);

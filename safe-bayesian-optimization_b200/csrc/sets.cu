@@ -525,7 +525,7 @@ int sets_pass1(sbo_ctx* ctx, double beta, int rule, int strict, sbo_sets_result*
   ctx->n_unsafe_local = r.n_unsafe;
   ctx->beta = beta;
   ctx->have_sets = true;
-  ctx->have_sets2 = false;
+  ctx->have_sets2 = ctx->have_exp = false;
   return SBO_OK;
 }
 

@@ -100,6 +100,48 @@ def run_safeopt(GP_m, n_iteration=10, noise=0., stop_std=0.01, on_iteration=None
     return data
 
 
+def safeopt_batch_iteration(GP_m, q):
+    """One batch acquisition of SafeOpt: q safe points for parallel experiments (BO.Batch).  Pick 1 is safeopt_iteration's
+    x_new; the others follow the same rule with the earlier picks as pending observations.  Returns (X (m, d), info)."""
+    t0 = time.perf_counter()
+    X, std, info = GP_m.Batch(q)
+    info = dict(info, std=np.asarray(std), acquisition_seconds=time.perf_counter() - t0)
+    if len(X) == 0:
+        raise EmptySafeSet("SafeOpt batch: the safe set is empty on the grid (no minimiser and no expander)")
+    return np.asarray(X, dtype=np.float64), info
+
+
+def run_safeopt_batch(GP_m, q, n_iteration=10, noise=0., stop_std=0.01, on_iteration=None, hypopt=None):
+    """run_safeopt with q experiments per iteration: each iteration takes a batch of q safe points, evaluates the q plants
+    and adds the samples one by one with ``add_sample``; it stops like run_safeopt, on the stds of pick 1 (the step's own
+    minimiser and expander).  Returns the dict of run_safeopt with one row per evaluated point plus ``batch`` (the
+    iteration of each row) and one ``info`` per iteration."""
+    data = {"i": [], "batch": [], "obj": [], "con": [], "x_0": [], "x_1": [], "info": []}
+    row = 0
+    for it in range(n_iteration):
+        X, info = safeopt_batch_iteration(GP_m, q)
+        outputs = [GP_m.calculate_plant_outputs(x, noise) for x in X]
+        for x, y in zip(X, outputs):
+            data["i"].append(row)
+            data["batch"].append(it)
+            data["obj"].append(y[0])
+            data["con"].append(y[1] if len(y) > 1 else np.nan)
+            data["x_0"].append(x[0])
+            data["x_1"].append(x[1] if x.shape[0] > 1 else np.nan)
+            row += 1
+        data["info"].append(info)
+        if on_iteration is not None:
+            on_iteration(it, GP_m, X, outputs, info)
+        for x, y in zip(X, outputs):
+            if hypopt is None:
+                GP_m.add_sample(x, y)
+            else:
+                GP_m.add_sample(x, y, hypopt=hypopt)
+        if info["std_expander"] < stop_std and info["std_minimizer"] < stop_std:
+            break
+    return data
+
+
 def run_goose(GP_m, n_iteration=10, noise=0., f_opt=0.145249, tol=0.005, on_iteration=None, hypopt=None):
     """test/test_GoOSE.py:142-190 without the plotting side effects; stops when the noiseless objective at x_new is
     within ``tol`` of ``f_opt`` (``:182``; pass f_opt=None to run all iterations)."""

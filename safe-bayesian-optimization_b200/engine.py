@@ -428,6 +428,44 @@ class GridEngine:
                                                      int(prec), int(unsafe_rule), Lp, C.byref(r)))
         return self._step_dict(r, True)
 
+    # -- batch SafeOpt acquisition (csrc/batch.cu): q safe query points per step ----------------------------------------
+    @staticmethod
+    def _pick_dict(p):
+        return {k: getattr(p, k) for k, _ in capi.BatchPick._fields_ if k != "pad"}
+
+    def safeopt_batch(self, q):
+        """q query points from the last SafeOpt step (sbo_safeopt_batch): a list of n_picked dicts with idx (global),
+        from_expander, std_min / idx_min and std_exp / idx_exp under the earlier picks; empty when M and E are empty."""
+        q = int(q)
+        arr = (capi.BatchPick * max(q, 1))()
+        n = C.c_int()
+        self._ck(self._lib.sbo_safeopt_batch(self._h, q, arr, C.byref(n)))
+        return [self._pick_dict(arr[b]) for b in range(n.value)]
+
+    def safeopt_batch_sharded(self, q):
+        """safeopt_batch on a grid sharded over the library's communicator (sbo_comm_init); every rank gets the same picks."""
+        q = int(q)
+        arr = (capi.BatchPick * max(q, 1))()
+        n = C.c_int()
+        self._ck(self._lib.sbo_safeopt_batch_sharded(self._h, q, arr, C.byref(n)))
+        return [self._pick_dict(arr[b]) for b in range(n.value)]
+
+    def batch_prepare(self, q):
+        """Staged batch, step 1: compact this shard's candidates M u E; returns their number."""
+        n = C.c_int64()
+        self._ck(self._lib.sbo_batch_prepare(self._h, int(q), C.byref(n)))
+        return int(n.value)
+
+    def batch_local(self):
+        """Staged batch, step 2: this shard's optima for the next pick (global indices)."""
+        p = capi.BatchPick()
+        self._ck(self._lib.sbo_batch_local(self._h, C.byref(p)))
+        return self._pick_dict(p)
+
+    def batch_commit(self, global_idx):
+        """Staged batch, step 3: hallucinate an observation at the chosen global index."""
+        self._ck(self._lib.sbo_batch_commit(self._h, int(global_idx)))
+
     # -- whole steps (drivers' decision rules) ------------------------------------------------
     def safeopt_step(self, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=capi.UNSAFE_ALL, L=None,
                      upload=True, kernel="RBF"):

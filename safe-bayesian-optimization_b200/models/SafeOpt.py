@@ -12,6 +12,9 @@ Additive keyword arguments (defaults reproduce the reference's semantics):
   precision            'fp64' | 'tf32' | 'tf32x3' (fantasy GEMM only; the tensor-core modes re-evaluate every pair inside their
                        error bound in FP64, so all three return the FP64 counts)
   unsafe_rule          'all' (reference: lcb_constraint_min returns the MAX, SafeOpt.py:73-77) | 'any'
+
+Additive method ``Batch(q)``: q safe query points for parallel experiments from the same step (hallucinated variance
+downdates of the objective GP; include/sbo_b200.h, sbo_safeopt_batch).
 """
 from __future__ import annotations
 
@@ -152,3 +155,20 @@ class BO(GP):
         if ex["best_idx"] < 0:
             return self._x(-1), 0.0
         return self._x(ex["best_idx"]), float(np.sqrt(ex["best_value"]))
+
+    def Batch(self, q):
+        """Additive: q safe query points of this step for parallel experiments -> (X (m, d), std (m,), info), m <= q.
+        Pick 1 is the point the reference's decision rule takes (test/test_SafeOpt.py:153-158); each later pick applies the
+        same rule to the objective variance conditioned on the earlier picks as pending observations (values unknown).  The
+        safe, minimiser and expander sets stay those of the real data, so every point is in the safe set.  std[i] is the
+        standard deviation of the set pick i was taken from; info["picks"] holds both sets' optima per pick.  m = 0 when the
+        minimiser and expander sets are empty."""
+        self.Expander()                     # the SafeOpt pair stage of the cached step (computed once per model version)
+        picks = self.engine.safeopt_batch(q)
+        d = self.bound.shape[0]
+        X = np.array([self._x(p["idx"]) for p in picks], dtype=np.float64).reshape(len(picks), d)
+        std = np.array([p["std_exp"] if p["from_expander"] else p["std_min"] for p in picks], dtype=np.float64)
+        first = picks[0] if picks else {"std_min": 0.0, "std_exp": 0.0}
+        info = {"picks": picks, "chose": ["expander" if p["from_expander"] else "minimizer" for p in picks],
+                "std_minimizer": float(first["std_min"]), "std_expander": float(first["std_exp"])}
+        return X, std, info

@@ -308,3 +308,27 @@ def goose_step(eng, ds, beta, unsafe_rule=capi.UNSAFE_ALL, L=None, upload=True, 
         (d, i), = reduce_arg([(ld, li)], device, False, group)
         out["x_new_idx"] = out["explore_idx"] = i
     return out
+
+
+def safeopt_batch(eng, q, device=None, group=None):
+    """Batch SafeOpt acquisition (GridEngine.safeopt_batch) on a sharded grid, after a SafeOpt step of this module on every
+    rank: per pick each rank reports its local optima over M and E, the ranks agree on the global ones (largest std, lowest
+    index on ties) and apply the pick rule, and every rank hallucinates the same observation.  Every rank returns the same
+    list of picks."""
+    if getattr(eng, "comm_ready", False) and group is None:
+        return eng.safeopt_batch_sharded(q)
+    device = torch.device("cuda", eng.device) if device is None else device
+    eng.batch_prepare(q)
+    picks = []
+    for b in range(int(q)):
+        loc = eng.batch_local()
+        (sm, im), (se, ie) = reduce_arg([(loc["std_min"], loc["idx_min"]), (loc["std_exp"], loc["idx_exp"])], device, True, group)
+        sm, se = (sm if im >= 0 else 0.0), (se if ie >= 0 else 0.0)
+        take_min = im >= 0 and (ie < 0 or sm > se)                 # test/test_SafeOpt.py:153-158, an empty set yields
+        idx = im if take_min else ie
+        if idx < 0:                                                # M and E are empty on every rank, and stay so
+            break
+        picks.append({"idx": idx, "from_expander": 0 if take_min else 1, "std_min": sm, "idx_min": im, "std_exp": se, "idx_exp": ie})
+        if b + 1 < q:
+            eng.batch_commit(idx)
+    return picks
