@@ -309,6 +309,49 @@ int sbo_batch_commit(sbo_ctx* ctx, int64_t global_idx);
 /* the three steps over the library's communicator (sbo_comm_init): one small all-gather per pick; every rank gets the same picks */
 int sbo_safeopt_batch_sharded(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n_picked);
 
+/* ---- batch GoOSE acquisition: q distinct safe query points per step (additive; no reference counterpart) ------------
+ * The hallucination of the SafeOpt batch above (same noise, same downdate of the objective variance v), over the candidates
+ * C = S u T of the local shard: S = SBO_MASK_SAFE of the last sets pass 1, T = the union of the SBO_MASK_TARGET masks of the
+ * last GoOSE target stage (Lipschitz mode one per constraint, fantasy mode which = 0, bounds mode the certified members).  The
+ * mean does not change; lcb_0(p) = mean_0(p) - beta*sqrt(v(p)) in raw units with the beta of that sets pass.  Pick b, on v
+ * conditioned on picks 1..b-1:
+ *   S_b = S minus the earlier picks, T_b = T minus the targets earlier explore picks served; S_b empty: no pick;
+ *   (safe_idx, safe_lcb) = argmin over S_b of lcb_0, (target_idx, target_lcb) = argmin over T_b (lowest global index on
+ *   ties; an empty set gives (-1, +inf));
+ *   the rule of test/test_GoOSE.py:158-162: target_idx = -1 or safe_lcb <= target_lcb -> the safe minimum (explore = 0);
+ *   else the point of S_b nearest to target_idx in raw coordinates (squared distance as SBO_ARGMIN_DIST, lowest index on
+ *   ties; explore = 1), and that target is served.
+ * Picks are distinct points of S, so n_picked = min(q, |S|).  Pick 1 is the step's x_new (except after an exact tie of
+ * lcb_0 between target points of different constraint masks).  A batch reads the step's state and writes none of it.
+ * Every entry point needs a GoOSE target stage (sbo_goose_target after sbo_sets_pass1, or a sharded GoOSE step) since the
+ * last model, grid, shard, posterior or set change, and fails with SBO_ERR_INVALID after a SafeOpt pair stage. */
+typedef struct sbo_goose_batch_pick {
+  int64_t idx;                             /* global index of the pick (a point of S); -1 = no pick */
+  int32_t explore, pad;                    /* 0: safe minimum; 1: nearest remaining safe point to target_idx */
+  double  safe_lcb;   int64_t safe_idx;    /* min lcb_0 over S_b under the earlier picks (+inf / -1 if empty) */
+  double  target_lcb; int64_t target_idx;  /* min lcb_0 over T_b (+inf / -1 if empty) */
+  double  dist;                            /* explore: ||x_idx - z_target||_2 in raw units; else 0 */
+} sbo_goose_batch_pick;
+/* one GPU: at most 5 launches per pick, no host synchronisation between picks, one copy to the host at the end.
+ * picks[q] out; *n_picked = min(q, |S|); with S empty picks[0] holds the optima (idx = -1). */
+int sbo_goose_batch(sbo_ctx* ctx, int q, sbo_goose_batch_pick* picks, int* n_picked);
+/* the same in steps for a grid sharded over ranks; the batch-side state is computed identically on every rank:
+ *   sbo_goose_batch_prepare  compact this rank's candidates, v = var_0 (*n_candidates_local = |C| of the shard)
+ *   sbo_goose_batch_local    this rank's (safe, target) optima for the next pick, GLOBAL indices (idx / explore apply the
+ *                            rule locally; idx = -1 for an explore pick, whose point comes from sbo_goose_batch_nearest)
+ *                            -> the caller reduces both (smallest lcb, lowest index) over the ranks
+ *   sbo_goose_batch_nearest  explore picks: this rank's point of S_b nearest to the GLOBAL target index, and its SQUARED
+ *                            distance (-1 / +inf if S_b is empty here) -> the caller reduces (smallest, lowest index)
+ *   sbo_goose_batch_commit   the pick and the target it served (-1: a safe pick), the same on every rank: hallucinate an
+ *                            observation at the pick and remove both from S_b / T_b; at most q commits */
+int sbo_goose_batch_prepare(sbo_ctx* ctx, int q, int64_t* n_candidates_local);
+int sbo_goose_batch_local(sbo_ctx* ctx, sbo_goose_batch_pick* local_optima);
+int sbo_goose_batch_nearest(sbo_ctx* ctx, int64_t target_global_idx, int64_t* idx, double* dist2);
+int sbo_goose_batch_commit(sbo_ctx* ctx, int64_t pick_global_idx, int64_t served_target_global_idx);
+/* the steps over the library's communicator (sbo_comm_init): one small all-gather per pick, a second one for an explore
+ * pick; every rank gets the same picks */
+int sbo_goose_batch_sharded(sbo_ctx* ctx, int q, sbo_goose_batch_pick* picks, int* n_picked);
+
 /* ---- instrumentation ------------------------------------------------------------------------ */
 /* number of kernels this library launched on ctx since the last reset */
 int64_t sbo_kernel_launches(sbo_ctx* ctx, int reset);

@@ -57,6 +57,11 @@ class BatchPick(C.Structure):
                 ("std_min", C.c_double), ("idx_min", C.c_int64), ("std_exp", C.c_double), ("idx_exp", C.c_int64)]
 
 
+class GooseBatchPick(C.Structure):
+    _fields_ = [("idx", C.c_int64), ("explore", C.c_int32), ("pad", C.c_int32), ("safe_lcb", C.c_double), ("safe_idx", C.c_int64),
+                ("target_lcb", C.c_double), ("target_idx", C.c_int64), ("dist", C.c_double)]
+
+
 _P = C.c_void_p
 _D = C.POINTER(C.c_double)
 _I64 = C.POINTER(C.c_int64)
@@ -114,6 +119,12 @@ SIGNATURES = {
     "sbo_batch_local": (C.c_int, [_P, C.POINTER(BatchPick)]),
     "sbo_batch_commit": (C.c_int, [_P, C.c_int64]),
     "sbo_safeopt_batch_sharded": (C.c_int, [_P, C.c_int, C.POINTER(BatchPick), C.POINTER(C.c_int)]),
+    "sbo_goose_batch": (C.c_int, [_P, C.c_int, C.POINTER(GooseBatchPick), C.POINTER(C.c_int)]),
+    "sbo_goose_batch_prepare": (C.c_int, [_P, C.c_int, _I64]),
+    "sbo_goose_batch_local": (C.c_int, [_P, C.POINTER(GooseBatchPick)]),
+    "sbo_goose_batch_nearest": (C.c_int, [_P, C.c_int64, _I64, _D]),
+    "sbo_goose_batch_commit": (C.c_int, [_P, C.c_int64, C.c_int64]),
+    "sbo_goose_batch_sharded": (C.c_int, [_P, C.c_int, C.POINTER(GooseBatchPick), C.POINTER(C.c_int)]),
     "sbo_kernel_launches": (C.c_int64, [_P, C.c_int]),
     "sbo_mem_peak": (C.c_int64, [_P, C.c_int]),
     "sbo_phase_ms": (C.c_int, [_P, C.c_int, _D]),

@@ -166,7 +166,7 @@ int sbo_get_model(sbo_ctx* ctx, double* L, double* W, double* alpha) {
   return SBO_OK;
 }
 
-static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = false; ctx->keep_v = 0; }
+static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false; ctx->keep_v = 0; }
 
 int sbo_set_grid(sbo_ctx* ctx, int d, const int64_t* pts_per_dim, const double* lo, const double* hi) {
   ENTER();

@@ -383,4 +383,48 @@ int sbo_safeopt_batch_sharded(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n
   return SBO_OK;
 }
 
+// batch GoOSE acquisition (batch.cu) on the sharded grid: per pick one all-gather of the ranks' (safe, target) optima, and
+// for an explore pick one of their nearest points to the target, both reduced to the smallest value with the lowest global
+// index on ties (as sbo_goose_step_sharded_ex), so that every rank commits the same pick
+int sbo_goose_batch_sharded(sbo_ctx* ctx, int q, sbo_goose_batch_pick* picks, int* n_picked) {
+  if (!ctx) return sbo_fail(nullptr, SBO_ERR_INVALID, "null context");
+  cudaSetDevice(ctx->device);
+  SBO_REQUIRE(ctx->comm != nullptr, "sbo_goose_batch_sharded: call sbo_comm_init first");
+  SBO_REQUIRE(picks && n_picked, "null result");
+  const int R = ctx->comm->nranks;
+  SBO_TRY(goose_batch_prepare(ctx, q, nullptr));
+  std::vector<double> g;
+  int n = 0;
+  for (int b = 0; b < q; ++b) {
+    sbo_goose_batch_pick loc;
+    SBO_TRY(goose_batch_local(ctx, &loc));
+    double mine[4] = {loc.safe_lcb, (double)loc.safe_idx, loc.target_lcb, (double)loc.target_idx};
+    SBO_TRY(gather_record(ctx, mine, 4, g));
+    sbo_goose_batch_pick r;
+    reduce_arg(g, 4, R, 0, false, &r.safe_lcb, &r.safe_idx);
+    reduce_arg(g, 4, R, 2, false, &r.target_lcb, &r.target_idx);
+    const bool explore = r.safe_idx >= 0 && r.target_idx >= 0 && !(r.safe_lcb <= r.target_lcb);   // test_GoOSE.py:158-162
+    r.explore = explore ? 1 : 0;
+    r.pad = 0;
+    r.idx = r.safe_idx;
+    r.dist = 0.0;
+    if (explore) {
+      long long li; double ld2;
+      SBO_TRY(goose_batch_nearest(ctx, r.target_idx, &li, &ld2));
+      double m[2] = {ld2, (double)li};
+      SBO_TRY(gather_record(ctx, m, 2, g));
+      double d2;
+      reduce_arg(g, 2, R, 0, false, &d2, &r.idx);
+      r.dist = sqrt(d2);
+    }
+    picks[b] = r;
+    if (r.idx < 0) break;                             // S_b is empty on every rank, and stays so
+    n = b + 1;
+    if (b + 1 < q) SBO_TRY(goose_batch_commit(ctx, r.idx, explore ? r.target_idx : -1));
+  }
+  ctx->bt.prepared = false;
+  *n_picked = n;
+  return SBO_OK;
+}
+
 }  // extern "C"

@@ -244,7 +244,7 @@ struct PairStage {
   long long n_ambiguous = 0, n_refined_safe = 0;     // split-TF32 refinement statistics of the last run
 };
 
-// state of a batch SafeOpt acquisition (batch.cu)
+// state of a batch SafeOpt or GoOSE acquisition (batch.cu)
 struct BatchRec {                 // device record of one pick: raw objective variances, GLOBAL indices (-1 = empty)
   long long idx;
   int from_exp, pad;
@@ -253,10 +253,11 @@ struct BatchRec {                 // device record of one pick: raw objective va
 };
 struct BatchStage {
   bool prepared = false;
+  bool goose = false;             // prepared for the GoOSE rule (C = S u T) instead of SafeOpt's (C = M u E)
   int q = 0, b = 0;               // picks asked for / observations hallucinated so far
   long long nc = 0;               // local candidates |C|
   int nparts = 0;                 // block partials of the candidate kernel
-  long long gen = 0;              // exp_gen of the pair stage the batch was prepared on
+  long long gen = 0;              // exp_gen (SafeOpt) or tgt_gen (GoOSE) of the pair stage the batch was prepared on
 };
 
 struct sbo_comm;   // comm.cu: NCCL communicator + gathered buffers
@@ -288,6 +289,8 @@ struct sbo_ctx {
   bool have_sets = false, have_sets2 = false;
   bool have_exp = false;     // the last pair stage was a SafeOpt expander on the current sets (m_exp valid; batch.cu needs it)
   long long exp_gen = 0;     // counts those stages: a prepared batch belongs to one of them
+  bool have_tgt = false;     // the same for a GoOSE target stage (m_tgt valid; the GoOSE batch needs it)
+  long long tgt_gen = 0;
   double beta = 0.0;
   DevBuf m_safe, m_unsafe, m_min, m_user, m_exp, m_tgt;
   DevBuf partials, result;
@@ -310,7 +313,7 @@ struct sbo_ctx {
   DevBuf gz_mask, gz_idx, gz_pay;         // all-gathered unsafe set of a sharded Lipschitz expander
   PairStage ps;
   BatchStage bt;
-  DevBuf bt_mask, bt_idx, bt_flag, bt_v, bt_w, bt_part, bt_pick;   // batch: C = M u E, membership bits, v[C], w[q][C], partials, pick side
+  DevBuf bt_mask, bt_idx, bt_flag, bt_v, bt_w, bt_part, bt_pick;   // batch: C = M u E (S u T), membership bits, v[C], w[q][C], partials, pick side
   // timing: event pairs are recorded without host syncs and summed per phase by ev_collect()
   struct EvPair { cudaEvent_t a, b; int phase; };
   std::vector<EvPair> evlog;
@@ -320,6 +323,7 @@ struct sbo_ctx {
   int64_t opt_posterior_variant = 1;  // 0: FP64 SIMT register tiles, 1: FP64 tensor cores (DMMA m8n8k4)
   int64_t opt_fantasy_prune = 1;      // 1 (default): exact key-ordered tile pruning of the fantasy expander (pairs.cu); 0: every pair
   long long n_unsafe_local = 0;
+  long long n_safe_local = 0;         // |S| of the local shard after the last sets pass 1 (the GoOSE batch's pick count)
   int64_t opt_fantasy_variant = -1;  // -1 auto; bit 0: BN=256 (2 TMEM slots) instead of 128 (4 slots); bit 1: 8 epilogue warps;
                                      // bit 2: 2-CTA pairs (cta_group::2, 256x256 tile pairs)
   int64_t opt_posterior_fused = 0;    // 1: meshgrid: separable factor tables + fused solve, no cross-covariance scratch (12 MB instead of 33.6 GB
@@ -408,5 +412,9 @@ int batch_prepare(sbo_ctx* ctx, int q, long long* n_candidates);
 int batch_local(sbo_ctx* ctx, BatchRec* out);
 int batch_commit(sbo_ctx* ctx, long long global_idx);
 void batch_pick_of(const BatchRec& r, sbo_batch_pick* out);
+int goose_batch_prepare(sbo_ctx* ctx, int q, long long* n_candidates);
+int goose_batch_local(sbo_ctx* ctx, sbo_goose_batch_pick* out);
+int goose_batch_nearest(sbo_ctx* ctx, long long target, long long* idx, double* dist2);
+int goose_batch_commit(sbo_ctx* ctx, long long pick, long long served_target);
 uint32_t* mask_ptr(sbo_ctx* ctx, int mask_kind, int which);
 long long mask_words(const sbo_ctx* ctx);

@@ -248,7 +248,7 @@ int model_upload(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_
       return sbo_fail(ctx, SBO_ERR_NUMERIC, "K of GP " + std::to_string(g) + " is not positive definite at pivot " +
                                                 std::to_string(info[g] - 1));
   ctx->have_model = true;
-  ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = false;
+  ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   return SBO_OK;
 }
 
@@ -372,7 +372,7 @@ int model_append(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_ne
       ctx->have_model = false;
       return sbo_fail(ctx, SBO_ERR_NUMERIC, "appended sample makes K of GP " + std::to_string(g) + " numerically singular");
     }
-  ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = false;
+  ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   return SBO_OK;
 }
 

@@ -1254,7 +1254,7 @@ int pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const doub
   const long long count = gs.count;
   PairStage& ps = ctx->ps;
   ps = PairStage{};
-  ctx->have_exp = false;
+  ctx->have_exp = ctx->have_tgt = false;
   ctx->refine_cells = ctx->refine_rows = 0;
   ps.mode = mode; ps.precision = precision; ps.beta = beta;
   ps.row_doubles = 2 * d + 3 * nc + 1;
@@ -1736,8 +1736,10 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
   if (ps.counted) out->pairs_evaluated = (int64_t)h[0] * ps.count_scale;
   else out->pairs_evaluated = ps.pairs_evaluated;
   if (out->pairs_evaluated > out->pairs_algorithmic) out->pairs_evaluated = out->pairs_algorithmic;
-  ctx->have_exp = !goose;              // the SafeOpt expander masks are complete: a batch acquisition may start from them
+  ctx->have_exp = !goose;              // the expander (target) masks are complete: a batch acquisition may start from them
+  ctx->have_tgt = goose != 0;
   if (!goose) ++ctx->exp_gen;
+  else ++ctx->tgt_gen;
   if (!have) return SBO_OK;
   // per-constraint arg-reduction, then first-best across constraints (SafeOpt.py:120-122 / GoOSE.py:110-112)
   const double keep5 = ctx->phase_ms[5];

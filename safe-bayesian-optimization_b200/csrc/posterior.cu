@@ -692,7 +692,7 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   if (keep_v && ms.G > 1) ctx->keep_v = keep_v;
   ctx->have_post = true;
   ctx->have_grad = with_grad != 0;
-  ctx->have_sets = ctx->have_sets2 = ctx->have_exp = false;
+  ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   return SBO_OK;
 }
 

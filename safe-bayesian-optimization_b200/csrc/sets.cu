@@ -523,9 +523,10 @@ int sets_pass1(sbo_ctx* ctx, double beta, int rule, int strict, sbo_sets_result*
   r.max_var = -INFINITY; r.max_var_i = -1; r.n_min = 0;
   if (out) fill_result(r, out);
   ctx->n_unsafe_local = r.n_unsafe;
+  ctx->n_safe_local = r.n_safe;
   ctx->beta = beta;
   ctx->have_sets = true;
-  ctx->have_sets2 = ctx->have_exp = false;
+  ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   return SBO_OK;
 }
 

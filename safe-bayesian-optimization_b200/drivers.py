@@ -168,6 +168,51 @@ def run_goose(GP_m, n_iteration=10, noise=0., f_opt=0.145249, tol=0.005, on_iter
     return data
 
 
+def goose_batch_iteration(GP_m, q):
+    """One batch acquisition of GoOSE: q distinct safe points for parallel experiments (BO.Batch).  Pick 1 is
+    goose_iteration's x_new; the others follow the same rule over the safe points and targets not yet used, with the
+    earlier picks as pending observations.  Returns (X (m, d), info)."""
+    t0 = time.perf_counter()
+    X, lcb, info = GP_m.Batch(q)
+    info = dict(info, lcb=np.asarray(lcb), acquisition_seconds=time.perf_counter() - t0)
+    if len(X) == 0:
+        raise EmptySafeSet("GoOSE batch: the safe set is empty on the grid (no safe minimum and no reachable target)")
+    return np.asarray(X, dtype=np.float64), info
+
+
+def run_goose_batch(GP_m, q, n_iteration=10, noise=0., f_opt=0.145249, tol=0.005, on_iteration=None, hypopt=None):
+    """run_goose with q experiments per iteration: each iteration takes a batch of q safe points, evaluates the q plants
+    and adds the samples one by one with ``add_sample``; it stops like run_goose, when the noiseless objective at pick 1
+    (the step's own x_new) is within ``tol`` of ``f_opt`` (f_opt=None runs all iterations).  Returns the dict of run_goose
+    with one row per evaluated point plus ``batch`` (the iteration of each row) and one ``info`` per iteration."""
+    data = {"i": [], "batch": [], "obj": [], "con": [], "x_0": [], "x_1": [], "x_target_0": [], "x_target_1": [], "info": []}
+    row = 0
+    for it in range(n_iteration):
+        X, info = goose_batch_iteration(GP_m, q)
+        outputs = [GP_m.calculate_plant_outputs(x, noise) for x in X]
+        for x, y, xt in zip(X, outputs, info["x_target"]):
+            data["i"].append(row)
+            data["batch"].append(it)
+            data["obj"].append(y[0])
+            data["con"].append(y[1] if len(y) > 1 else np.nan)
+            data["x_0"].append(x[0])
+            data["x_1"].append(x[1] if x.shape[0] > 1 else np.nan)
+            data["x_target_0"].append(xt[0])
+            data["x_target_1"].append(xt[1] if xt.shape[0] > 1 else np.nan)
+            row += 1
+        data["info"].append(info)
+        if on_iteration is not None:
+            on_iteration(it, GP_m, X, outputs, info)
+        for x, y in zip(X, outputs):
+            if hypopt is None:
+                GP_m.add_sample(x, y)
+            else:
+                GP_m.add_sample(x, y, hypopt=hypopt)
+        if f_opt is not None and abs(GP_m.plant_system[0](X[0]) - f_opt) <= tol:
+            break
+    return data
+
+
 def run_multiple(make_bo, x_init, r, n_sample, n_start, n_iteration, noise, algorithm="safeopt", path=None,
                  stop_std=0.01, seeds=None):
     """test/test_SafeOpt.py:188-253 / :255-322 and the GoOSE counterparts: ``n_start`` independent runs, each

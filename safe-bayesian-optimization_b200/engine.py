@@ -466,6 +466,53 @@ class GridEngine:
         """Staged batch, step 3: hallucinate an observation at the chosen global index."""
         self._ck(self._lib.sbo_batch_commit(self._h, int(global_idx)))
 
+    # -- batch GoOSE acquisition (csrc/batch.cu): q distinct safe query points per step ---------------------------------
+    @staticmethod
+    def _goose_pick_dict(p):
+        return {k: getattr(p, k) for k, _ in capi.GooseBatchPick._fields_ if k != "pad"}
+
+    def goose_batch(self, q):
+        """q query points from the last GoOSE step (sbo_goose_batch): a list of min(q, |S|) dicts with idx (global), explore,
+        safe_lcb / safe_idx and target_lcb / target_idx under the earlier picks, and dist (explore picks)."""
+        q = int(q)
+        arr = (capi.GooseBatchPick * max(q, 1))()
+        n = C.c_int()
+        self._ck(self._lib.sbo_goose_batch(self._h, q, arr, C.byref(n)))
+        return [self._goose_pick_dict(arr[b]) for b in range(n.value)]
+
+    def goose_batch_sharded(self, q):
+        """goose_batch on a grid sharded over the library's communicator (sbo_comm_init); every rank gets the same picks."""
+        q = int(q)
+        arr = (capi.GooseBatchPick * max(q, 1))()
+        n = C.c_int()
+        self._ck(self._lib.sbo_goose_batch_sharded(self._h, q, arr, C.byref(n)))
+        return [self._goose_pick_dict(arr[b]) for b in range(n.value)]
+
+    def goose_batch_prepare(self, q):
+        """Staged GoOSE batch, step 1: compact this shard's candidates S u T; returns their number."""
+        n = C.c_int64()
+        self._ck(self._lib.sbo_goose_batch_prepare(self._h, int(q), C.byref(n)))
+        return int(n.value)
+
+    def goose_batch_local(self):
+        """Staged GoOSE batch, step 2: this shard's (safe, target) optima for the next pick (global indices); idx is -1 for an
+        explore pick, whose point goose_batch_nearest finds."""
+        p = capi.GooseBatchPick()
+        self._ck(self._lib.sbo_goose_batch_local(self._h, C.byref(p)))
+        return self._goose_pick_dict(p)
+
+    def goose_batch_nearest(self, target_idx):
+        """Staged GoOSE batch, explore picks: this shard's remaining safe point nearest to the global target index ->
+        (global index, squared distance); (-1, inf) when none is left here."""
+        i, d2 = C.c_int64(), C.c_double()
+        self._ck(self._lib.sbo_goose_batch_nearest(self._h, int(target_idx), C.byref(i), C.byref(d2)))
+        return int(i.value), float(d2.value)
+
+    def goose_batch_commit(self, pick_idx, served_target_idx=-1):
+        """Staged GoOSE batch, step 3: hallucinate an observation at the pick and retire it and the target it served
+        (-1: a safe pick)."""
+        self._ck(self._lib.sbo_goose_batch_commit(self._h, int(pick_idx), int(served_target_idx)))
+
     # -- whole steps (drivers' decision rules) ------------------------------------------------
     def safeopt_step(self, ds, beta, mode="lipschitz", precision="fp64", unsafe_rule=capi.UNSAFE_ALL, L=None,
                      upload=True, kernel="RBF"):

@@ -5,6 +5,10 @@ arg-reduction (plus, for ``Target``, the pair kernel with the reduction over the
 grid pipeline.  Same constructor and return values as the reference; ``expander_mode='fantasy'`` (with
 ``precision`` 'fp64' | 'tf32' | 'tf32x3') replaces the Lipschitz reachability test of ``Target`` by the
 fantasy test of the SafeOpt expander: z is reachable if the GP update with y_i = ucb_i(x) makes it safe.
+
+Additive method ``Batch(q)``: q distinct safe query points for parallel experiments from the same step (GoOSE's rule on
+hallucinated variance downdates of the objective GP; include/sbo_b200.h, sbo_goose_batch).  It replaces the SafeOpt batch
+that this class would otherwise inherit, which applies the SafeOpt rule to a GoOSE object.
 """
 from __future__ import annotations
 
@@ -50,3 +54,23 @@ class BO(_GridBO):
         capi = self._capi()
         idx, _ = self.engine.argreduce(capi.ARGMIN_DIST, capi.MASK_SAFE, 0, np.asarray(target, dtype=np.float64))
         return self._x(idx)
+
+    def Batch(self, q):
+        """Additive: q distinct safe query points of this step for parallel experiments -> (X (m, d), lcb (m,), info),
+        m = min(q, number of safe grid points).  Pick 1 is the point the reference's decision rule takes
+        (test/test_GoOSE.py:158-162); each later pick applies the same rule, over the safe points and targets not yet used,
+        to lcb_0 with the objective variance conditioned on the earlier picks as pending observations (values unknown).
+        The safe and target sets stay those of the real data, so every point is in the safe set.  lcb[i] is the lcb_0 of
+        the set pick i was decided on (the safe minimum, or the target it explores towards); info holds the per-pick
+        records ("picks"), "chose" ('safe_minimum' | 'explore'), "x_target" (m, d; NaN rows for safe picks) and pick 1's
+        "min_safe_lcb" / "target_lcb"."""
+        self.Target()                       # the GoOSE target stage of the cached step (computed once per model version)
+        picks = self.engine.goose_batch(q)
+        d = self.bound.shape[0]
+        X = np.array([self._x(p["idx"]) for p in picks], dtype=np.float64).reshape(len(picks), d)
+        lcb = np.array([p["target_lcb"] if p["explore"] else p["safe_lcb"] for p in picks], dtype=np.float64)
+        x_target = np.array([self._x(p["target_idx"] if p["explore"] else -1) for p in picks], dtype=np.float64).reshape(len(picks), d)
+        first = picks[0] if picks else {"safe_lcb": np.inf, "target_lcb": np.inf}
+        info = {"picks": picks, "chose": ["explore" if p["explore"] else "safe_minimum" for p in picks], "x_target": x_target,
+                "min_safe_lcb": float(first["safe_lcb"]), "target_lcb": float(first["target_lcb"])}
+        return X, lcb, info

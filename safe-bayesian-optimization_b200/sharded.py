@@ -332,3 +332,30 @@ def safeopt_batch(eng, q, device=None, group=None):
         if b + 1 < q:
             eng.batch_commit(idx)
     return picks
+
+
+def goose_batch(eng, q, device=None, group=None):
+    """Batch GoOSE acquisition (GridEngine.goose_batch) on a sharded grid, after a GoOSE step of this module on every rank:
+    per pick each rank reports its local optima of lcb_0 over S_b and T_b, the ranks agree on the global ones (smallest,
+    lowest index on ties) and apply the rule of test/test_GoOSE.py:158-162; an explore pick takes the globally nearest
+    remaining safe point to the target.  Every rank hallucinates the same observation and returns the same picks."""
+    if getattr(eng, "comm_ready", False) and group is None:
+        return eng.goose_batch_sharded(q)
+    device = torch.device("cuda", eng.device) if device is None else device
+    eng.goose_batch_prepare(q)
+    picks = []
+    for b in range(int(q)):
+        loc = eng.goose_batch_local()
+        (sl, si), (tl, ti) = reduce_arg([(loc["safe_lcb"], loc["safe_idx"]), (loc["target_lcb"], loc["target_idx"])], device, False, group)
+        if si < 0:                                                 # S_b is empty on every rank, and stays so
+            break
+        explore = ti >= 0 and not sl <= tl                         # test/test_GoOSE.py:158-162
+        idx, dist = si, 0.0
+        if explore:
+            (d2, idx), = reduce_arg([eng.goose_batch_nearest(ti)[::-1]], device, False, group)
+            dist = float(np.sqrt(d2))
+        picks.append({"idx": idx, "explore": int(explore), "safe_lcb": sl, "safe_idx": si, "target_lcb": tl, "target_idx": ti,
+                      "dist": dist})
+        if b + 1 < q:
+            eng.goose_batch_commit(idx, ti if explore else -1)
+    return picks
