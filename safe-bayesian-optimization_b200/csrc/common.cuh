@@ -330,7 +330,7 @@ struct sbo_ctx {
                                       // of DRAM traffic at C4, but 52.5 vs 40.0 ms: the table loads stall the DMMA loop) | 0 (default): two kernels + scratch
   int64_t opt_posterior_tables = 0;   // 1: meshgrid cross-covariance values from the separable factor tables instead of exp() (measured slower:
                                       // 13.5 vs 9.0 ms at C4 -- the kernel is bound by its Kx stores and address stream, not by exp)
-  int64_t opt_posterior_chunk_mb = 0; // Kx scratch per chunk in MB (0 = default 48: L2 resident)
+  int64_t opt_posterior_chunk_mb = 0; // Kx scratch per chunk in MB (0 = default 1024; never less than one wave of the solve, posterior.cu chunk_points)
   int64_t opt_prior_mean_zero = 0;    // 1: zero prior mean for every GP (GP_Robust.py:322-323, StableOpt); 0: GP_Safe.py:331-332
   int64_t opt_fantasy_f64_variant = 1; // FP64 fantasy expander: 1 (default) tensor cores (DMMA 128x64 tiles) | 0 SIMT reference kernel
   int64_t opt_fantasy_refine = 2;     // tensor-core fantasy expander: pairs the FP32/TF32 error bound cannot settle are re-evaluated in FP64 (exact

@@ -593,7 +593,7 @@ static int solve_dispatch(sbo_ctx* ctx, const double* Kx, int P, long long p0, i
   return SBO_OK;
 }
 
-// K1 fused path (meshgrid grids, option "posterior_fused", default 1): separable factor tables, table-based mean /
+// K1 fused path (meshgrid grids, option "posterior_fused", default 0): separable factor tables, table-based mean /
 // gradient kernel (no Kx store), fused solve kernel (no Kx load).
 static int build_tables(sbo_ctx* ctx, TabSpec* ts) {
   const ModelSpec& ms = ctx->ms;
