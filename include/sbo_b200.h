@@ -126,6 +126,20 @@ int sbo_point_coords(sbo_ctx* ctx, int64_t global_idx, double* x /* d */);
  *   1 = FP64 rows, 2 = FP32 rows rounded to TF32 (tensor-core operand), 3 = split-TF32 rows [hi | lo]
  *   (three-pass TF32 GEMM, ~FP32 accuracy). */
 int sbo_posterior(sbo_ctx* ctx, int with_grad, int keep_v, double* mean, double* var);
+/* bring the last sbo_posterior of this context up to the model after the sbo_append_sample calls made since (same with_grad,
+ * same keep_v); mean/var as in sbo_posterior (NULL = keep on device).  Appending leaves the leading block of L and of
+ * W = L^-1 unchanged, so only the m new rows of W enter:  e_r(p) = sum_j W[r][j] k_j(p) for the new rows r,
+ * var' = max(0, var/Y_std^2 - sum_r e_r^2) * Y_std^2 per GP, and the kept V rows gain the m columns e(p) (entries of the
+ * old rows untouched).  Mean and L_i are recomputed from the new alpha with the loop of sbo_posterior: bitwise what
+ * sbo_posterior returns on the same model with the default options.  n kernel values and m*n FMAs per point and GP, no
+ * triangular solve; ceil(m/8) kernel launches.  Works on the local shard (contiguous or block-cyclic), no collective.
+ *   info->rows = m, the samples appended since; m = 0: nothing to do.  info->recomputed = 1: V rows were kept and the
+ *   appends grew the padded factor (the V-row stride changed), so the full sbo_posterior ran with the same flags.
+ * SBO_ERR_INVALID, nothing modified: no sbo_posterior since the last sbo_set_model(_ex), sbo_set_grid, sbo_set_points,
+ * sbo_set_shard or sbo_set_shard_cyclic, or kept V rows freed by sbo_release(1) since.  Afterwards the sets, pair stages,
+ * batches and sbo_lipschitz (with_grad) work as after sbo_posterior. */
+typedef struct sbo_update_info { int64_t rows; int32_t recomputed, pad; } sbo_update_info;
+int sbo_posterior_update(sbo_ctx* ctx, double* mean, double* var, sbo_update_info* info);
 /* GP_inference at m arbitrary points (the single-point API behind BO.mean/ucb/lcb,
  * SafeOpt.py:29-45): x[m*d] row-major -> mean[m*G], var[m*G] POINT-major like the reference. */
 int sbo_point_posterior(sbo_ctx* ctx, int64_t m, const double* x, double* mean, double* var);
@@ -359,7 +373,7 @@ int64_t sbo_kernel_launches(sbo_ctx* ctx, int reset);
 int64_t sbo_mem_peak(sbo_ctx* ctx, int reset);
 /* device time of named phases of the last calls, milliseconds (CUDA events on the ctx stream).
  * phase: 0 model, 1 posterior(crosscov), 2 posterior(solve), 3 sets, 4 pairs, 5 argreduce, 6 pair preparation,
- *        7 FP64 refinement of the split-TF32 fantasy expander */
+ *        7 FP64 refinement of the split-TF32 fantasy expander, 8 posterior update (sbo_posterior_update) */
 int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms);
 /* FP64 refinement of the last pair stage on ctx (fantasy_refine = 2 / 1): the cells the pass was cut into and the FP64 rows
  * V = L^-1 K(X, p) it computed (one cell: one row per distinct candidate and unsafe point of the ambiguous list; more cells

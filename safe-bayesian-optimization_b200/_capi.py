@@ -24,7 +24,7 @@ MASK_SAFE, MASK_MIN, MASK_UNSAFE, MASK_USER, MASK_EXPANDER, MASK_TARGET = 0, 1, 
 # covariance function name (models/GP_Safe.GP kernel argument) -> enum sbo_kernel
 KERNELS = {"RBF": 0, "Matern32": 1, "Matern52": 2}
 BATCH_MAX_Q = 256                  # SBO_BATCH_MAX_Q: picks per batch acquisition
-PHASES = ("model", "crosscov", "solve", "sets", "pairs", "argreduce", "pair_prep", "refine")
+PHASES = ("model", "crosscov", "solve", "sets", "pairs", "argreduce", "pair_prep", "refine", "posterior_update")
 
 
 class SetsResult(C.Structure):
@@ -57,6 +57,10 @@ class BatchPick(C.Structure):
                 ("std_min", C.c_double), ("idx_min", C.c_int64), ("std_exp", C.c_double), ("idx_exp", C.c_int64)]
 
 
+class UpdateInfo(C.Structure):
+    _fields_ = [("rows", C.c_int64), ("recomputed", C.c_int32), ("pad", C.c_int32)]
+
+
 class GooseBatchPick(C.Structure):
     _fields_ = [("idx", C.c_int64), ("explore", C.c_int32), ("pad", C.c_int32), ("safe_lcb", C.c_double), ("safe_idx", C.c_int64),
                 ("target_lcb", C.c_double), ("target_idx", C.c_int64), ("dist", C.c_double)]
@@ -84,6 +88,7 @@ SIGNATURES = {
     "sbo_set_shard": (C.c_int, [_P, C.c_int64, C.c_int64]),
     "sbo_point_coords": (C.c_int, [_P, C.c_int64, _D]),
     "sbo_posterior": (C.c_int, [_P, C.c_int, C.c_int, _D, _D]),
+    "sbo_posterior_update": (C.c_int, [_P, _D, _D, C.POINTER(UpdateInfo)]),
     "sbo_point_posterior": (C.c_int, [_P, C.c_int64, _D, _D, _D]),
     "sbo_lipschitz": (C.c_int, [_P, _D]),
     "sbo_point_mean_grad": (C.c_int, [_P, C.c_int, C.c_int64, _D, _D]),

@@ -134,6 +134,7 @@ int sbo_set_model_ex(sbo_ctx* ctx, int kernel, int n, int d, int G, const double
                      const double* X_mean, const double* X_std, const double* Y_mean, const double* Y_std, const double* hyp) {
   ENTER();
   ctx->have_model = false;
+  ctx->up.valid = false;
   return model_upload(ctx, kernel, n, d, G, X_norm, Y_norm, X_mean, X_std, Y_mean, Y_std, hyp);
 }
 
@@ -166,7 +167,7 @@ int sbo_get_model(sbo_ctx* ctx, double* L, double* W, double* alpha) {
   return SBO_OK;
 }
 
-static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false; ctx->keep_v = 0; }
+static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false; ctx->keep_v = 0; ctx->up.valid = false; }
 
 int sbo_set_grid(sbo_ctx* ctx, int d, const int64_t* pts_per_dim, const double* lo, const double* hi) {
   ENTER();
@@ -258,6 +259,18 @@ int sbo_point_coords(sbo_ctx* ctx, int64_t p, double* x) {
 int sbo_posterior(sbo_ctx* ctx, int with_grad, int keep_v, double* mean, double* var) {
   ENTER();
   SBO_TRY(posterior_run(ctx, with_grad, keep_v));
+  const size_t bytes = sizeof(double) * (size_t)ctx->ms.G * ctx->gs.count;
+  if (mean) SBO_CUDA(cudaMemcpyAsync(mean, ctx->mean.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (var) SBO_CUDA(cudaMemcpyAsync(var, ctx->var.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  SBO_CUDA(cudaStreamSynchronize(ctx->stream));
+  ev_collect(ctx);
+  return SBO_OK;
+}
+
+int sbo_posterior_update(sbo_ctx* ctx, double* mean, double* var, sbo_update_info* info) {
+  ENTER();
+  sbo_update_info tmp;
+  SBO_TRY(posterior_update(ctx, info ? info : &tmp));
   const size_t bytes = sizeof(double) * (size_t)ctx->ms.G * ctx->gs.count;
   if (mean) SBO_CUDA(cudaMemcpyAsync(mean, ctx->mean.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
   if (var) SBO_CUDA(cudaMemcpyAsync(var, ctx->var.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
@@ -436,7 +449,7 @@ int sbo_refine_stats(sbo_ctx* ctx, int64_t* cells, int64_t* fp64_rows) {
 
 int sbo_phase_ms(sbo_ctx* ctx, int phase, double* ms) {
   ENTER();
-  SBO_REQUIRE(phase >= 0 && phase < 8 && ms, "bad phase");
+  SBO_REQUIRE(phase >= 0 && phase < 9 && ms, "bad phase");
   *ms = ctx->phase_ms[phase];
   return SBO_OK;
 }
@@ -465,7 +478,10 @@ int sbo_stable_minmax(sbo_ctx* ctx, int n_controlled, int fun_kind, double beta,
 int sbo_release(sbo_ctx* ctx, int what) {
   ENTER();
   SBO_CUDA(cudaStreamSynchronize(ctx->stream));
-  if (what & 1) { ctx->mem_now -= (int64_t)ctx->vall.cap; free_buf(ctx->vall); ctx->keep_v = 0; }
+  if (what & 1) {
+    if (ctx->keep_v) ctx->up.valid = false;        // the update would have to extend rows that are gone
+    ctx->mem_now -= (int64_t)ctx->vall.cap; free_buf(ctx->vall); ctx->keep_v = 0;
+  }
   if (what & 2) {
     for (DevBuf* b : {&ctx->vx, &ctx->vz, &ctx->exp_v, &ctx->tc_row, &ctx->tc_col, &ctx->imp_rows}) { ctx->mem_now -= (int64_t)b->cap; free_buf(*b); }
     // workspaces of the FP64 refinement: the ambiguous-pair list, its points, rank maps, buckets and FP64 rows

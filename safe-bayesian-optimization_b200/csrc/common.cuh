@@ -285,6 +285,9 @@ struct sbo_ctx {
   DevBuf mean, var, kx, lmax, tabs;     // tabs: separable SE-ARD factor tables of the meshgrid (posterior.cu)
   int keep_v = 0;            // 0 none, 1 fp64, 2 fp32
   DevBuf vall;               // [(G-1)][count][npad] rows of V for the constraints
+  // the last posterior_run as sbo_posterior_update sees it: valid while the model changed only through sbo_append_sample
+  // (model n and npad, the flags it ran with); cleared by a model upload, a grid or shard change and sbo_release(1) of kept V rows
+  struct { bool valid = false, with_grad = false; int n = 0, npad = 0, keep_v = 0; } up;
   // sets
   bool have_sets = false, have_sets2 = false;
   bool have_exp = false;     // the last pair stage was a SafeOpt expander on the current sets (m_exp valid; batch.cu needs it)
@@ -318,7 +321,7 @@ struct sbo_ctx {
   struct EvPair { cudaEvent_t a, b; int phase; };
   std::vector<EvPair> evlog;
   std::vector<cudaEvent_t> evpool;
-  double phase_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  double phase_ms[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   // options
   int64_t opt_posterior_variant = 1;  // 0: FP64 SIMT register tiles, 1: FP64 tensor cores (DMMA m8n8k4)
   int64_t opt_fantasy_prune = 1;      // 1 (default): exact key-ordered tile pruning of the fantasy expander (pairs.cu); 0: every pair
@@ -372,7 +375,8 @@ void sbo_free(sbo_ctx* ctx, DevBuf& b);                         // give a work b
                                              " at " + __FILE__ + ":" + std::to_string(__LINE__)); \
   } while (0)
 
-// phase ids: 0 model, 1 posterior cross-covariance, 2 posterior solve, 3 sets, 4 pairs, 5 arg-reduce, 6 pair prep
+// phase ids: 0 model, 1 posterior cross-covariance, 2 posterior solve, 3 sets, 4 pairs, 5 arg-reduce, 6 pair prep,
+// 7 FP64 refinement, 8 posterior update
 void ev_begin(sbo_ctx* ctx, int phase);   // record a start event on the ctx stream
 void ev_end(sbo_ctx* ctx);                // record the matching stop event
 void ev_reset(sbo_ctx* ctx, int phase);   // zero a phase accumulator
@@ -389,6 +393,7 @@ int ball_mask(sbo_ctx* ctx, int mask_kind, const double* x0, double r);
 int stable_minmax(sbo_ctx* ctx, int n_controlled, int fun_kind, double beta, int64_t* xc_idx, double* value, int64_t* n_robust_safe, double* score_host);
 int nll_batch(sbo_ctx* ctx, int kernel, int n, int d, const double* X_norm, const double* y, int P, const double* hyp, double* nll);
 int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v);
+int posterior_update(sbo_ctx* ctx, sbo_update_info* info);
 int posterior_vrows_dev(sbo_ctx* ctx, long long m, const double* pts_dev, double* vout);
 void posterior_vrows_scratch(const sbo_ctx* ctx, long long m, size_t* mv_bytes, size_t* k_bytes);
 int posterior_points(sbo_ctx* ctx, int64_t m, const double* x, double* mean, double* var);

@@ -5,11 +5,15 @@
 //   grad  = d mean / d x (analytic), L_i = max_p ||grad||_inf               (K1c, optional)
 //   v     = W k  (W = L^-1 lower triangular),  var = max(0, sf2 - |v|^2) * Ystd^2   (K1b)
 //   V rows are optionally kept (FP64 or TF32-rounded FP32) for the fantasy expander GEMM.
+// Update after m appended samples (sbo_append_sample leaves rows 0..n0-1 of W unchanged, so v(p)'s first n0 entries stay):
+//   e_r = sum_{j<=r} W[r][j] k_j,  r = n0..n0+m-1;   var' = max(0, var/Ystd^2 - sum_r e_r^2) * Ystd^2;   V' = [V ; e]
+//   mean and grad from the new alpha                                        (K1a update mode, no solve, no Kx scratch)
 #include "common.cuh"
 #include <math.h>
 
 #define XC_THREADS 128
 #define XC_JT 128
+#define XC_MC 8      // update mode: new rows of W per pass (the e_r accumulators live in registers)
 
 __device__ __forceinline__ float to_tf32(float x) {
   uint32_t r;
@@ -49,17 +53,28 @@ k_build_tables(ModelSpec ms, GridSpec gs, TabSpec ts, double* __restrict__ tab) 
   tab[(size_t)g * ts.goff + ts.koff[k] + e] = v;
 }
 
+// update mode of K1a (MC > 0): rows r0 .. r0+mr-1 of W in this pass; var is read and rewritten in place; V-row columns
+// r0 .. r0+mr-1 are written with the rounding of keep_v = emit (0: none kept)
+struct UpdSpec {
+  int r0, mr, emit;
+  double* var;
+  void* vall;
+  long long v_count;
+};
+
 // ---------------------------------------------------------------------------------------------
-// K1a: cross-covariance tile -> Kx scratch [G][npad][P] (points contiguous), mean, optional gradient
+// K1a: cross-covariance tile -> Kx scratch [G][npad][P] (points contiguous), mean, optional gradient.
+// MC > 0: the update mode -- no Kx; e_r for up to MC new rows of W, staged in shared memory beside X and alpha.
 // ---------------------------------------------------------------------------------------------
-template <int D, class KC>
+template <int D, class KC, int MC>
 __global__ void __launch_bounds__(XC_THREADS)
 k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __restrict__ Kx,
            double* __restrict__ mean_out, long long out_ld, double* __restrict__ gradmax,
-           double* __restrict__ grad_out, int grad_gp, TabSpec ts) {
+           double* __restrict__ grad_out, int grad_gp, TabSpec ts, UpdSpec us) {
   __shared__ double Xs[XC_JT * D];
   __shared__ double As[XC_JT];
   __shared__ double red[XC_THREADS / 32];
+  __shared__ double Wr[MC > 0 ? MC * XC_JT : 1];   // referenced only when MC > 0
   const KC kc(ms.kernel);
   const int g = blockIdx.y + ms.g0;
   const int pl = blockIdx.x * XC_THREADS + threadIdx.x;
@@ -92,6 +107,9 @@ k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __
   double gk[D];
 #pragma unroll
   for (int k = 0; k < D; ++k) gk[k] = 0.0;
+  double er[MC > 0 ? MC : 1];
+#pragma unroll
+  for (int i = 0; i < (MC > 0 ? MC : 1); ++i) er[i] = 0.0;
   double* kcol = Kx + (size_t)g * ms.npad * P + pl;
   for (int j0 = 0; j0 < ms.npad; j0 += XC_JT) {
     __syncthreads();
@@ -99,6 +117,12 @@ k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __
       Xs[e] = (j0 * D + e < ms.npad * D) ? ms.Xn[(size_t)j0 * D + e] : 0.0;
     for (int e = threadIdx.x; e < XC_JT; e += XC_THREADS)
       As[e] = (j0 + e < ms.npad) ? ms.alpha[(size_t)g * ms.npad + j0 + e] : 0.0;
+    if constexpr (MC > 0) {
+      for (int e = threadIdx.x; e < MC * XC_JT; e += XC_THREADS) {
+        const int i = e / XC_JT, c = e % XC_JT;
+        Wr[e] = (i < us.mr && j0 + c < ms.n) ? ms.W[((size_t)g * ms.npad + us.r0 + i) * ms.npad + j0 + c] : 0.0;
+      }
+    }
     __syncthreads();
     const int jn = min(XC_JT, ms.npad - j0);
     if (in_chunk) {
@@ -123,6 +147,10 @@ k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __
 #pragma unroll
             for (int k = 0; k < D; ++k) gk[k] += wg * df[k];
           }
+          if constexpr (MC > 0) {
+#pragma unroll
+            for (int i = 0; i < MC; ++i) er[i] = fma(Wr[i * XC_JT + j], kv, er[i]);   // rows of W are zero right of the diagonal
+          }
         }
         if (Kx) kcol[(size_t)(j0 + j) * P] = kv;
       }
@@ -146,6 +174,33 @@ k_crosscov(ModelSpec ms, GridSpec gs, long long p0, int P, int valid, double* __
       if (threadIdx.x == 0) {
         for (int w = 1; w < XC_THREADS / 32; ++w) gm = fmax(gm, red[w]);
         atomicMax((unsigned long long*)(gradmax + g), (unsigned long long)__double_as_longlong(gm));
+      }
+    }
+  }
+  if constexpr (MC > 0) {
+    if (ok) {
+      double s = 0.0;
+#pragma unroll
+      for (int i = 0; i < MC; ++i) s = fma(er[i], er[i], s);                      // er[i] = 0 for i >= mr
+      const size_t o = (size_t)g * out_ld + p0 + pl;
+      const double y2 = ms.Ystd[g] * ms.Ystd[g];
+      us.var[o] = fmax(0.0, us.var[o] / y2 - s) * y2;                              // a clamped var stays 0
+      if (us.emit && g > 0 && us.vall) {                                           // rounding of the solve epilogues
+        const int np = ms.npad;
+        const size_t row = ((size_t)(g - 1) * us.v_count + p0 + pl) * (us.emit == 3 ? 2 * np : np) + us.r0;
+#pragma unroll
+        for (int i = 0; i < MC; ++i) {
+          if (i >= us.mr) break;
+          if (us.emit == 1) {
+            reinterpret_cast<double*>(us.vall)[row + i] = er[i];
+          } else if (us.emit == 2) {
+            reinterpret_cast<float*>(us.vall)[row + i] = to_tf32((float)er[i]);
+          } else {
+            const float hi = to_tf32((float)er[i]);
+            reinterpret_cast<float*>(us.vall)[row + i] = hi;
+            reinterpret_cast<float*>(us.vall)[row + i + np] = to_tf32((float)(er[i] - (double)hi));
+          }
+        }
       }
     }
   }
@@ -564,8 +619,8 @@ static int crosscov_dispatch(sbo_ctx* ctx, const GridSpec& gs, long long p0, int
   ModelSpec msl = ctx->ms; msl.g0 = g0;
   dim3 grid((unsigned)cdiv(P, XC_THREADS), (unsigned)(ctx->ms.G - g0));
   with_int<1, SBO_MAX_D>(msl.d, [&](auto D) { with_kernel(msl.kernel, [&](auto kc) {
-    k_crosscov<D, decltype(kc)><<<grid, XC_THREADS, 0, ctx->stream>>>(msl, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax,
-                                                                      grad_out, grad_gp, ts);
+    k_crosscov<D, decltype(kc), 0><<<grid, XC_THREADS, 0, ctx->stream>>>(msl, gs, p0, P, valid, Kx, mean_out, out_ld, gradmax,
+                                                                         grad_out, grad_gp, ts, UpdSpec{});
   }); });
   SBO_LAUNCH_CHECK();
   return SBO_OK;
@@ -647,6 +702,7 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   SBO_REQUIRE(ctx->have_grid, "sbo_posterior: no grid (call sbo_set_grid / sbo_set_points)");
   SBO_REQUIRE(ctx->gs.d == ctx->ms.d, "grid and model dimensions differ");
   SBO_REQUIRE(keep_v >= 0 && keep_v <= 3, "keep_v must be 0, 1, 2 or 3");
+  ctx->up.valid = false;     // mean / var / V rows are overwritten from here on
   const ModelSpec& ms = ctx->ms;
   const long long count = ctx->gs.count;
   SBO_REQUIRE(count > 0, "empty shard");
@@ -693,6 +749,53 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   ctx->have_post = true;
   ctx->have_grad = with_grad != 0;
   ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
+  ctx->up.valid = true;
+  ctx->up.n = ms.n; ctx->up.npad = ms.npad;
+  ctx->up.with_grad = with_grad != 0; ctx->up.keep_v = keep_v;
+  return SBO_OK;
+}
+
+// sbo_posterior_update: the last posterior_run brought up to the model after the sbo_append_sample calls since.  Rows
+// up.n .. n-1 of W are the new ones; ceil(m / XC_MC) passes of the K1a update mode, the first also writes mean and the
+// Lipschitz constants (bitwise what posterior_run computes with the default options: the same loop in the same order).
+int posterior_update(sbo_ctx* ctx, sbo_update_info* info) {
+  SBO_REQUIRE(ctx->have_model, "sbo_posterior_update: no model");
+  SBO_REQUIRE(ctx->up.valid, "sbo_posterior_update: no posterior to update -- none since the last sbo_set_model, sbo_set_grid, "
+                             "sbo_set_points or sbo_set_shard, or its V rows were released (call sbo_posterior)");
+  const ModelSpec& ms = ctx->ms;
+  const int m = ms.n - ctx->up.n;
+  info->rows = m; info->recomputed = 0; info->pad = 0;
+  if (m == 0) return SBO_OK;
+  ev_reset(ctx, 8);
+  if (ctx->keep_v && ms.npad != ctx->up.npad) {    // the V-row stride changed with the padding: recompute
+    SBO_TRY(posterior_run(ctx, ctx->up.with_grad, ctx->up.keep_v));
+    info->recomputed = 1;
+    return SBO_OK;
+  }
+  const long long count = ctx->gs.count;
+  const bool with_grad = ctx->up.with_grad;
+  if (with_grad) SBO_CUDA(cudaMemsetAsync(ctx->lmax.p, 0, sizeof(double) * SBO_MAX_G, ctx->stream));
+  const long long CH = 1LL << 30;                  // points per launch (int offsets inside the kernel)
+  for (long long p0 = 0; p0 < count; p0 += CH) {
+    const int valid = (int)((count - p0) < CH ? (count - p0) : CH);
+    for (int r0 = ctx->up.n; r0 < ms.n; r0 += XC_MC) {
+      const bool first = r0 == ctx->up.n;
+      UpdSpec us{r0, (ms.n - r0) < XC_MC ? (ms.n - r0) : XC_MC, ctx->keep_v, (double*)ctx->var.p, ctx->vall.p, count};
+      dim3 grid((unsigned)cdiv(valid, XC_THREADS), (unsigned)ms.G);
+      ev_begin(ctx, 8);
+      with_int<1, SBO_MAX_D>(ms.d, [&](auto D) { with_kernel(ms.kernel, [&](auto kc) {
+        k_crosscov<D, decltype(kc), XC_MC><<<grid, XC_THREADS, 0, ctx->stream>>>(
+            ms, ctx->gs, p0, valid, valid, nullptr, first ? (double*)ctx->mean.p : nullptr, count,
+            (first && with_grad) ? (double*)ctx->lmax.p : nullptr, nullptr, -1, TabSpec{}, us);
+      }); });
+      ev_end(ctx);
+      SBO_LAUNCH_CHECK();
+    }
+  }
+  ctx->have_post = true;
+  ctx->have_grad = with_grad;
+  ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
+  ctx->up.n = ms.n; ctx->up.npad = ms.npad;
   return SBO_OK;
 }
 

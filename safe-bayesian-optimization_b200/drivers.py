@@ -73,12 +73,29 @@ def goose_iteration(GP_m):
         "target_lcb": float(target_lcb), "chose": chose, "acquisition_seconds": dt}
 
 
+def _check_append_mode(hypopt, fixed_model):
+    if fixed_model and hypopt is not None:
+        raise ValueError("fixed_model keeps the installed hyper-parameters: pass hypopt=None")
+
+
+def _append(GP_m, x, y, hypopt, fixed_model):
+    if fixed_model:
+        GP_m.add_sample_fixed(x, y)
+    elif hypopt is None:
+        GP_m.add_sample(x, y)
+    else:
+        GP_m.add_sample(x, y, hypopt=hypopt)
+
+
 def run_safeopt(GP_m, n_iteration=10, noise=0., stop_std=0.01, on_iteration=None, require_lipschitz_ucb=False,
-                hypopt=None):
+                hypopt=None, fixed_model=False):
     """test/test_SafeOpt.py:135-186 without the plotting side effects (pass ``on_iteration(i, GP_m, x_new, y, info)``
     to draw frames, e.g. with utils_SafeOpt.create_data_for_plot + plot_safe_region_Benoit).
     ``hypopt`` (additive): keep these hyper-parameters instead of refitting in every ``add_sample``.
+    ``fixed_model`` (additive): append every sample with ``add_sample_fixed`` -- installed hyper-parameters and
+    normalisation kept, the next step updates the grid posterior instead of recomputing it (not with ``hypopt``).
     Returns the reference's ``data`` dict: i, obj, con, x_0, x_1 (+ per-iteration info)."""
+    _check_append_mode(hypopt, fixed_model)
     data = {"i": [], "obj": [], "con": [], "x_0": [], "x_1": [], "info": []}
     for i in range(n_iteration):
         x_new, info = safeopt_iteration(GP_m, require_lipschitz_ucb)
@@ -91,10 +108,7 @@ def run_safeopt(GP_m, n_iteration=10, noise=0., stop_std=0.01, on_iteration=None
         data["info"].append(info)
         if on_iteration is not None:
             on_iteration(i, GP_m, x_new, plant_output, info)
-        if hypopt is None:
-            GP_m.add_sample(x_new, plant_output)
-        else:
-            GP_m.add_sample(x_new, plant_output, hypopt=hypopt)
+        _append(GP_m, x_new, plant_output, hypopt, fixed_model)
         if info["std_expander"] < stop_std and info["std_minimizer"] < stop_std:       # :178
             break
     return data
@@ -142,9 +156,12 @@ def run_safeopt_batch(GP_m, q, n_iteration=10, noise=0., stop_std=0.01, on_itera
     return data
 
 
-def run_goose(GP_m, n_iteration=10, noise=0., f_opt=0.145249, tol=0.005, on_iteration=None, hypopt=None):
+def run_goose(GP_m, n_iteration=10, noise=0., f_opt=0.145249, tol=0.005, on_iteration=None, hypopt=None,
+              fixed_model=False):
     """test/test_GoOSE.py:142-190 without the plotting side effects; stops when the noiseless objective at x_new is
-    within ``tol`` of ``f_opt`` (``:182``; pass f_opt=None to run all iterations)."""
+    within ``tol`` of ``f_opt`` (``:182``; pass f_opt=None to run all iterations).  ``hypopt`` and ``fixed_model`` as in
+    run_safeopt."""
+    _check_append_mode(hypopt, fixed_model)
     data = {"i": [], "obj": [], "con": [], "x_0": [], "x_1": [], "x_target_0": [], "x_target_1": [], "info": []}
     for i in range(n_iteration):
         x_new, info = goose_iteration(GP_m)
@@ -159,10 +176,7 @@ def run_goose(GP_m, n_iteration=10, noise=0., f_opt=0.145249, tol=0.005, on_iter
         data["info"].append(info)
         if on_iteration is not None:
             on_iteration(i, GP_m, x_new, plant_output, info)
-        if hypopt is None:
-            GP_m.add_sample(x_new, plant_output)
-        else:
-            GP_m.add_sample(x_new, plant_output, hypopt=hypopt)
+        _append(GP_m, x_new, plant_output, hypopt, fixed_model)
         if f_opt is not None and abs(GP_m.plant_system[0](x_new) - f_opt) <= tol:
             break
     return data

@@ -211,6 +211,22 @@ class GridEngine:
         self._ck(self._lib.sbo_posterior(self._h, int(with_grad), int(keep_v), None, None))
         return None
 
+    def posterior_update(self, fetch=True):
+        """Bring the last posterior up to the model after the append_sample calls made since (sbo_posterior_update), with
+        the same with_grad and keep_v.  Returns ((mean, var) as in posterior() or None, info) with info = {"rows": samples
+        appended since that posterior, "recomputed": True when the update ran the full posterior (V rows kept and the
+        padded factor grew)}.  Raises ValueError when anything else changed the model, grid or shard since."""
+        info = capi.UpdateInfo()
+        if fetch:
+            mean = np.empty((self.G, self.count))
+            var = np.empty((self.G, self.count))
+            self._ck(self._lib.sbo_posterior_update(self._h, capi.dptr(mean), capi.dptr(var), C.byref(info)))
+            out = (mean.T, var.T)
+        else:
+            self._ck(self._lib.sbo_posterior_update(self._h, None, None, C.byref(info)))
+            out = None
+        return out, {"rows": int(info.rows), "recomputed": bool(info.recomputed)}
+
     def point_posterior(self, x):
         x = _f64(x).reshape(-1, self.d)
         m = x.shape[0]

@@ -209,6 +209,10 @@ class GP:
         self.update_inference_dataset()
         ds = self.inference_datasets                    # the device already holds this state: no upload on the next call
         self._uploaded = (id(ds), self._version, id(ds.get("hypopt")), id(ds.get("X_norm")))
+        self._on_model_appended()
+
+    def _on_model_appended(self):
+        """The device model gained samples through sbo_append_sample only (subclasses may update instead of recompute)."""
         self._on_model_changed()
 
     # ------------------------------------------------------------------ inference (GPU)

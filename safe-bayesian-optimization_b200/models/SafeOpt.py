@@ -41,12 +41,18 @@ class BO(GP):
         self.unsafe_rule = unsafe_rule
         self._grid_set = False
         self._step = None
+        self._post_keep_v = None          # keep_v of the engine's last step posterior; None: the next step recomputes it
 
     # ------------------------------------------------------------------ grid pipeline plumbing
     def _capi(self):
         return package()._capi
 
     def _on_model_changed(self):
+        self._step = None
+        self._post_keep_v = None
+
+    def _on_model_appended(self):
+        # add_sample_fixed: the next step brings the last posterior up to the grown model (sbo_posterior_update)
         self._step = None
 
     def _ensure_grid(self):
@@ -60,16 +66,22 @@ class BO(GP):
             self.grid_shape = tuple(pts)
             self._grid_set = True
             self._step = None
+            self._post_keep_v = None
 
     def _ensure_step(self):
-        """Posterior + sets for the current model, computed once per model version."""
+        """Posterior + sets for the current model, computed once per model version.  After add_sample_fixed the
+        posterior is updated with the appended samples instead of recomputed."""
         self._ensure_uploaded(self.inference_datasets)
         self._ensure_grid()
         if self._step is None:
             capi = self._capi()
             fantasy = self.expander_mode == 'fantasy'
             keep_v = capi.PRECISIONS[self.precision][1] if fantasy else 0
-            self.engine.posterior(with_grad=True, keep_v=keep_v, fetch=False)
+            if self._post_keep_v == keep_v:
+                self.engine.posterior_update(fetch=False)
+            else:
+                self.engine.posterior(with_grad=True, keep_v=keep_v, fetch=False)
+                self._post_keep_v = keep_v
             rule = capi.UNSAFE_ALL if self.unsafe_rule == 'all' else capi.UNSAFE_ANY
             self._step = {"sets": self.engine.sets(self.b, rule), "L": self.engine.lipschitz()}
         return self._step
@@ -84,6 +96,7 @@ class BO(GP):
         self._ensure_uploaded(self.inference_datasets)
         self._ensure_grid()
         self._step = None
+        self._post_keep_v = None
         return self.engine.posterior(with_grad=False, keep_v=0, fetch=True)
 
     def safe_mask(self, kind='safe'):
