@@ -234,7 +234,8 @@ int sbo_goose_target_ex(sbo_ctx* ctx, int mode, int precision, double beta, cons
  *   sbo_pairs_finish_dev  masks + arg-reductions on the local shard; the local candidates are rows
  *                         [offset, offset + n_x_local) of the reduced result.  `out` holds LOCAL optima with
  *                         GLOBAL indices; the caller reduces them across ranks (value, then lowest index).
- * sbo_expander / sbo_goose_target are these five steps on one GPU. */
+ * sbo_expander / sbo_goose_target are these five steps on one GPU.  Any model, grid, shard, posterior or sets-pass-1 change
+ * invalidates a prepared stage, and sbo_release(1) a fantasy stage's export: the staged calls then fail with SBO_ERR_INVALID. */
 typedef struct sbo_pairs_info { int64_t n_x_local, n_z_local, row_doubles, vrow_bytes; } sbo_pairs_info;
 int sbo_pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const double* L /* G or NULL */, sbo_pairs_info* info);
 int sbo_pairs_export_dev(sbo_ctx* ctx, void* rows_dev, void* vrows_dev);

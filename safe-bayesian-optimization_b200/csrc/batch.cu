@@ -396,12 +396,12 @@ k_goose_finish(const BatchPart* __restrict__ near, int nparts, int b, int mode, 
 // host drivers
 // ---------------------------------------------------------------------------------------------
 static int batch_valid(sbo_ctx* ctx) {
-  SBO_REQUIRE(ctx->bt.prepared && !ctx->bt.goose && ctx->have_exp && ctx->bt.gen == ctx->exp_gen,
+  SBO_REQUIRE(ctx->bt.prepared && !ctx->bt.goose && ctx->have_exp,
               "no prepared batch for the current SafeOpt pair stage (call sbo_batch_prepare after the step)");
   return SBO_OK;
 }
 static int goose_valid(sbo_ctx* ctx) {
-  SBO_REQUIRE(ctx->bt.prepared && ctx->bt.goose && ctx->have_tgt && ctx->bt.gen == ctx->tgt_gen,
+  SBO_REQUIRE(ctx->bt.prepared && ctx->bt.goose && ctx->have_tgt,
               "no prepared GoOSE batch for the current GoOSE target stage (call sbo_goose_batch_prepare after the step)");
   return SBO_OK;
 }
@@ -445,8 +445,8 @@ static int launch_choose(sbo_ctx* ctx, int b) {
 // the candidates C = a u (union of the n_exp masks b), compacted, and the initial state (v = var_0, membership bits)
 static int prepare_candidates(sbo_ctx* ctx, int q, bool goose, long long* n_candidates) {
   BatchStage& bs = ctx->bt;
-  bs = BatchStage{};
-  bs.goose = goose;
+  stage_changed(ctx, Change::BATCH);
+  bs.goose = goose; bs.b = 0;
   const long long count = ctx->gs.count, nw = mask_words(ctx);
   const int n_exp = ctx->ms.G > 1 ? ctx->ms.G - 1 : 1;
   SBO_TRY(sbo_ensure(ctx, ctx->bt_mask, sizeof(uint32_t) * (size_t)nw));
@@ -465,8 +465,7 @@ static int prepare_candidates(sbo_ctx* ctx, int q, bool goose, long long* n_cand
   SBO_TRY(sbo_ensure(ctx, ctx->bt_part, sizeof(BatchPart) * (size_t)bs.nparts * (goose ? 2 : 1)));
   SBO_TRY(sbo_ensure(ctx, ctx->bt_pick, pick_bytes(q, ctx->ms.npad)));
   SBO_TRY(launch_update(ctx, -1));
-  bs.gen = goose ? ctx->tgt_gen : ctx->exp_gen;
-  bs.prepared = true;
+  stage_changed(ctx, Change::BATCH_PREPARED);
   if (n_candidates) *n_candidates = nc;
   return SBO_OK;
 }
@@ -602,7 +601,7 @@ int sbo_safeopt_batch(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n_picked)
   SBO_REQUIRE(picks && n_picked, "null result");
   long long nc = 0;
   SBO_TRY(batch_prepare(ctx, q, &nc));
-  ctx->bt.prepared = false;                     // the whole batch runs here; the staged calls need their own prepare
+  stage_changed(ctx, Change::BATCH);            // the whole batch runs here; the staged calls need their own prepare
   std::vector<BatchRec> rec(q);
   if (nc == 0) {                                // M and E are both empty, and stay so
     SBO_TRY(launch_choose(ctx, 0));
@@ -659,7 +658,7 @@ int sbo_goose_batch(sbo_ctx* ctx, int q, sbo_goose_batch_pick* picks, int* n_pic
   cudaSetDevice(ctx->device);
   SBO_REQUIRE(picks && n_picked, "null result");
   SBO_TRY(goose_batch_prepare(ctx, q, nullptr));
-  ctx->bt.prepared = false;                     // the whole batch runs here; the staged calls need their own prepare
+  stage_changed(ctx, Change::BATCH);            // the whole batch runs here; the staged calls need their own prepare
   // every pick retires one point of S, and a pick exists while S_b is not empty: exactly min(q, |S|) picks
   const int n = (int)std::min<long long>(q, ctx->n_safe_local);
   sbo_goose_batch_pick* rec = goose_recs(pick_ptrs(ctx));

@@ -40,6 +40,60 @@ void sbo_free(sbo_ctx* ctx, DevBuf& b) {
 
 static void free_buf(DevBuf& b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
 
+// The one place that decides which stages stay valid.  A change to a stage makes every later stage of the pipeline stale;
+// sets pass 2 hangs off pass 1 and makes nothing stale.
+void stage_changed(sbo_ctx* ctx, Change c) {
+  enum { POST, SETS, PAIRS, BATCH, NONE } stale = NONE;   // the first stage c makes stale; the later ones go with it
+  switch (c) {
+    case Change::GRID:
+      ctx->keep_v = 0;
+      [[fallthrough]];
+    case Change::MODEL:
+      ctx->up.valid = false;
+      stale = POST; break;
+    case Change::APPEND:             // what sbo_posterior_update is for: ctx->up stays valid
+      stale = POST; break;
+    case Change::POSTERIOR:
+      ctx->keep_v = 0; ctx->up.valid = false;
+      stale = POST; break;
+    case Change::POSTERIOR_DONE:
+      ctx->have_post = true; ctx->have_grad = ctx->up.with_grad;
+      ctx->keep_v = ctx->ms.G > 1 ? ctx->up.keep_v : 0;   // V rows exist for the constraints only
+      ctx->up.valid = true;
+      stale = SETS; break;
+    case Change::SETS1:
+      ctx->have_sets = true; ctx->have_sets2 = false;
+      stale = PAIRS; break;
+    case Change::SETS2:
+      ctx->have_sets2 = true; break;
+    case Change::PAIRS:
+      stale = PAIRS; break;
+    case Change::PAIRS_PREPARED:
+      ctx->ps.prepared = ctx->ps.exportable = true; break;
+    case Change::PAIRS_IMPORTED:
+      ctx->ps.imported = true; break;
+    case Change::EXPANDER:
+    case Change::TARGET:             // a batch belongs to the pair stage result it was prepared on
+      ctx->have_exp = c == Change::EXPANDER; ctx->have_tgt = c == Change::TARGET;
+      stale = BATCH; break;
+    case Change::BATCH:
+      stale = BATCH; break;
+    case Change::BATCH_PREPARED:
+      ctx->bt.prepared = true; break;
+    case Change::RELEASE_V:          // the update would have to extend rows that are gone, and the export reads them
+      if (ctx->keep_v) ctx->up.valid = false;
+      ctx->keep_v = 0;
+      if (ctx->ps.mode == SBO_MODE_FANTASY) ctx->ps.exportable = false;
+      break;
+    case Change::RELEASE_PAIRS:      // an unfinished stage loses its operands; the masks of a finished one and a batch stay
+      ctx->ps = PairStage{}; break;
+  }
+  if (stale <= POST) ctx->have_post = ctx->have_grad = false;
+  if (stale <= SETS) ctx->have_sets = ctx->have_sets2 = false;
+  if (stale <= PAIRS) { ctx->ps = PairStage{}; ctx->have_exp = ctx->have_tgt = false; }
+  if (stale <= BATCH) ctx->bt.prepared = false;
+}
+
 void ev_begin(sbo_ctx* ctx, int phase) {
   sbo_ctx::EvPair p;
   p.phase = phase;
@@ -134,7 +188,7 @@ int sbo_set_model_ex(sbo_ctx* ctx, int kernel, int n, int d, int G, const double
                      const double* X_mean, const double* X_std, const double* Y_mean, const double* Y_std, const double* hyp) {
   ENTER();
   ctx->have_model = false;
-  ctx->up.valid = false;
+  stage_changed(ctx, Change::MODEL);
   return model_upload(ctx, kernel, n, d, G, X_norm, Y_norm, X_mean, X_std, Y_mean, Y_std, hyp);
 }
 
@@ -167,8 +221,6 @@ int sbo_get_model(sbo_ctx* ctx, double* L, double* W, double* alpha) {
   return SBO_OK;
 }
 
-static void reset_grid_state(sbo_ctx* ctx) { ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false; ctx->keep_v = 0; ctx->up.valid = false; }
-
 int sbo_set_grid(sbo_ctx* ctx, int d, const int64_t* pts_per_dim, const double* lo, const double* hi) {
   ENTER();
   SBO_REQUIRE(d >= 1 && d <= SBO_MAX_D, "d out of range (1..8)");
@@ -189,7 +241,7 @@ int sbo_set_grid(sbo_ctx* ctx, int d, const int64_t* pts_per_dim, const double* 
   g.N = N; g.first = 0; g.count = N;
   ctx->gs = g;
   ctx->have_grid = true;
-  reset_grid_state(ctx);
+  stage_changed(ctx, Change::GRID);
   return SBO_OK;
 }
 
@@ -205,7 +257,7 @@ int sbo_set_points(sbo_ctx* ctx, int64_t N, int d, const double* pts) {
   g.explicit_pts = (const double*)ctx->pts.p;
   ctx->gs = g;
   ctx->have_grid = true;
-  reset_grid_state(ctx);
+  stage_changed(ctx, Change::GRID);
   return SBO_OK;
 }
 
@@ -215,7 +267,7 @@ int sbo_set_shard(sbo_ctx* ctx, int64_t first, int64_t count) {
   SBO_REQUIRE(first >= 0 && count >= 1 && first + count <= ctx->gs.N, "shard out of range");
   ctx->gs.first = first; ctx->gs.count = count;
   ctx->gs.cyc_n = 0; ctx->gs.cyc_rank = 0; ctx->gs.cyc_blk = 0;
-  reset_grid_state(ctx);
+  stage_changed(ctx, Change::GRID);
   return SBO_OK;
 }
 
@@ -235,7 +287,7 @@ int sbo_set_shard_cyclic(sbo_ctx* ctx, int rank, int nranks, int64_t block, int6
   g.cyc_n = nranks; g.cyc_rank = rank; g.cyc_blk = block;
   if (nranks == 1) { g.cyc_n = 0; }
   if (count_out) *count_out = count;
-  reset_grid_state(ctx);
+  stage_changed(ctx, Change::GRID);
   return SBO_OK;
 }
 
@@ -479,8 +531,8 @@ int sbo_release(sbo_ctx* ctx, int what) {
   ENTER();
   SBO_CUDA(cudaStreamSynchronize(ctx->stream));
   if (what & 1) {
-    if (ctx->keep_v) ctx->up.valid = false;        // the update would have to extend rows that are gone
-    ctx->mem_now -= (int64_t)ctx->vall.cap; free_buf(ctx->vall); ctx->keep_v = 0;
+    stage_changed(ctx, Change::RELEASE_V);
+    ctx->mem_now -= (int64_t)ctx->vall.cap; free_buf(ctx->vall);
   }
   if (what & 2) {
     for (DevBuf* b : {&ctx->vx, &ctx->vz, &ctx->exp_v, &ctx->tc_row, &ctx->tc_col, &ctx->imp_rows}) { ctx->mem_now -= (int64_t)b->cap; free_buf(*b); }
@@ -488,7 +540,7 @@ int sbo_release(sbo_ctx* ctx, int what) {
     for (DevBuf* b : {&ctx->amb_list, &ctx->amb_mask, &ctx->amb_xd, &ctx->amb_zd, &ctx->amb_rx, &ctx->amb_rz, &ctx->amb_pts,
                       &ctx->amb_vx, &ctx->amb_vz, &ctx->amb_cell, &ctx->amb_hist, &ctx->amb_tgt})
       sbo_free(ctx, *b);
-    ctx->ps = PairStage{};
+    stage_changed(ctx, Change::RELEASE_PAIRS);
   }
   return SBO_OK;
 }

@@ -378,7 +378,7 @@ int sbo_safeopt_batch_sharded(sbo_ctx* ctx, int q, sbo_batch_pick* picks, int* n
     n = b + 1;
     if (b + 1 < q) SBO_TRY(batch_commit(ctx, r.idx));
   }
-  ctx->bt.prepared = false;
+  stage_changed(ctx, Change::BATCH);
   *n_picked = n;
   return SBO_OK;
 }
@@ -422,7 +422,7 @@ int sbo_goose_batch_sharded(sbo_ctx* ctx, int q, sbo_goose_batch_pick* picks, in
     n = b + 1;
     if (b + 1 < q) SBO_TRY(goose_batch_commit(ctx, r.idx, explore ? r.target_idx : -1));
   }
-  ctx->bt.prepared = false;
+  stage_changed(ctx, Change::BATCH);
   *n_picked = n;
   return SBO_OK;
 }

@@ -230,6 +230,7 @@ struct DevBuf {
 // state of the staged pair driver (pairs.cu)
 struct PairStage {
   bool prepared = false, imported = false, counted = false, sorted = false;   // sorted: fantasy operands in key order (exact pruning)
+  bool exportable = false;   // prepared, and a fantasy stage's V rows (what sbo_pairs_export reads) not released since
   int mode = 0, precision = 0, row_doubles = 0, count_scale = 1;
   double beta = 0.0;
   double L[SBO_MAX_G] = {0, 0, 0, 0, 0, 0, 0, 0};   // L[c] for constraint c+1
@@ -257,7 +258,6 @@ struct BatchStage {
   int q = 0, b = 0;               // picks asked for / observations hallucinated so far
   long long nc = 0;               // local candidates |C|
   int nparts = 0;                 // block partials of the candidate kernel
-  long long gen = 0;              // exp_gen (SafeOpt) or tgt_gen (GoOSE) of the pair stage the batch was prepared on
 };
 
 struct sbo_comm;   // comm.cu: NCCL communicator + gathered buffers
@@ -286,14 +286,12 @@ struct sbo_ctx {
   int keep_v = 0;            // 0 none, 1 fp64, 2 fp32
   DevBuf vall;               // [(G-1)][count][npad] rows of V for the constraints
   // the last posterior_run as sbo_posterior_update sees it: valid while the model changed only through sbo_append_sample
-  // (model n and npad, the flags it ran with); cleared by a model upload, a grid or shard change and sbo_release(1) of kept V rows
+  // (model n and npad, the flags it ran with)
   struct { bool valid = false, with_grad = false; int n = 0, npad = 0, keep_v = 0; } up;
   // sets
   bool have_sets = false, have_sets2 = false;
   bool have_exp = false;     // the last pair stage was a SafeOpt expander on the current sets (m_exp valid; batch.cu needs it)
-  long long exp_gen = 0;     // counts those stages: a prepared batch belongs to one of them
   bool have_tgt = false;     // the same for a GoOSE target stage (m_tgt valid; the GoOSE batch needs it)
-  long long tgt_gen = 0;
   double beta = 0.0;
   DevBuf m_safe, m_unsafe, m_min, m_user, m_exp, m_tgt;
   DevBuf partials, result;
@@ -343,6 +341,26 @@ struct sbo_ctx {
   int64_t opt_pair_cull = 1;         // Lipschitz pair kernels: exact bounding-box culling of staged tiles
   int64_t opt_fantasy_gx = 0;        // 2-CTA kernel: x tile pairs per raster group (0 = default)
 };
+
+// What a call did to the pipeline  model -> posterior -> sets pass 1 (-> pass 2) -> pair stage -> batch.  stage_changed()
+// (capi.cu) decides what that leaves valid; no other code writes have_post, have_grad, have_sets(2), have_exp, have_tgt,
+// keep_v, up.valid, ps.prepared / imported / exportable or bt.prepared.
+enum class Change {
+  MODEL,            // sbo_set_model(_ex) starts replacing the model
+  APPEND,           // sbo_append_sample starts growing it: the last posterior can still be updated
+  GRID,             // sbo_set_grid / _points / _shard / _shard_cyclic
+  POSTERIOR,        // a posterior run starts overwriting mean, var and the kept V rows
+  POSTERIOR_DONE,   // a posterior run or update completed with the flags in ctx->up
+  SETS1, SETS2,     // a sets pass completed
+  PAIRS,            // sbo_pairs_prepare starts a new pair stage
+  PAIRS_PREPARED, PAIRS_IMPORTED,
+  EXPANDER, TARGET, // sbo_pairs_finish_dev completed the SafeOpt expander / GoOSE target masks
+  BATCH,            // a batch starts its prepare, or ran whole: the staged batch calls need a new prepare
+  BATCH_PREPARED,
+  RELEASE_V,        // sbo_release(1)
+  RELEASE_PAIRS,    // sbo_release(2)
+};
+void stage_changed(sbo_ctx* ctx, Change c);
 
 extern thread_local std::string g_sbo_last_error;
 

@@ -248,7 +248,6 @@ int model_upload(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_
       return sbo_fail(ctx, SBO_ERR_NUMERIC, "K of GP " + std::to_string(g) + " is not positive definite at pivot " +
                                                 std::to_string(info[g] - 1));
   ctx->have_model = true;
-  ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   return SBO_OK;
 }
 
@@ -313,6 +312,7 @@ int model_append(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_ne
   ModelSpec& ms = ctx->ms;
   const int n = ms.n, d = ms.d, G = ms.G;
   SBO_REQUIRE(n + 1 <= 16384, "n out of range");
+  stage_changed(ctx, Change::APPEND);
   ev_reset(ctx, 0);
   ev_begin(ctx, 0);
   if (n + 1 > ms.npad) {
@@ -372,7 +372,6 @@ int model_append(sbo_ctx* ctx, const double* x_norm_new, const double* y_norm_ne
       ctx->have_model = false;
       return sbo_fail(ctx, SBO_ERR_NUMERIC, "appended sample makes K of GP " + std::to_string(g) + " numerically singular");
     }
-  ctx->have_post = ctx->have_grad = ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   return SBO_OK;
 }
 

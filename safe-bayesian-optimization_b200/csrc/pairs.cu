@@ -1253,8 +1253,7 @@ int pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const doub
   const int nc = ms.G - 1, d = gs.d;
   const long long count = gs.count;
   PairStage& ps = ctx->ps;
-  ps = PairStage{};
-  ctx->have_exp = ctx->have_tgt = false;
+  stage_changed(ctx, Change::PAIRS);
   ctx->refine_cells = ctx->refine_rows = 0;
   ps.mode = mode; ps.precision = precision; ps.beta = beta;
   ps.row_doubles = 2 * d + 3 * nc + 1;
@@ -1317,7 +1316,7 @@ int pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const doub
     }
   }
   ev_end(ctx);
-  ps.prepared = true;
+  stage_changed(ctx, Change::PAIRS_PREPARED);
   if (info) {
     info->n_x_local = nx; info->n_z_local = ps.nz_full; info->row_doubles = ps.row_doubles;
     info->vrow_bytes = (mode == SBO_MODE_FANTASY) ? (int64_t)(v_elem_size(ctx) * (size_t)nc * vrow_elems(ctx)) : 0;
@@ -1327,7 +1326,7 @@ int pairs_prepare(sbo_ctx* ctx, int mode, int precision, double beta, const doub
 
 int pairs_export(sbo_ctx* ctx, void* rows_dev, void* vrows_dev) {
   PairStage& ps = ctx->ps;
-  SBO_REQUIRE(ps.prepared, "sbo_pairs_export: call sbo_pairs_prepare first");
+  SBO_REQUIRE(ps.exportable, "sbo_pairs_export: call sbo_pairs_prepare first");
   const long long nx = ps.nx_local;
   if (nx == 0) return SBO_OK;
   SBO_REQUIRE(rows_dev != nullptr, "null export buffer");
@@ -1356,7 +1355,7 @@ int pairs_import(sbo_ctx* ctx, long long n_total, const void* rows_dev, const vo
   SBO_REQUIRE(ps.prepared, "sbo_pairs_import: call sbo_pairs_prepare first");
   SBO_REQUIRE(n_total >= 0, "bad candidate count");
   ps.nx_total = n_total;
-  ps.imported = true;
+  stage_changed(ctx, Change::PAIRS_IMPORTED);
   if (n_total == 0) return SBO_OK;
   SBO_REQUIRE(rows_dev != nullptr, "null import buffer");
   const ModelSpec& ms = ctx->ms;
@@ -1736,10 +1735,8 @@ int pairs_finish(sbo_ctx* ctx, int goose, long long offset, const void* result_d
   if (ps.counted) out->pairs_evaluated = (int64_t)h[0] * ps.count_scale;
   else out->pairs_evaluated = ps.pairs_evaluated;
   if (out->pairs_evaluated > out->pairs_algorithmic) out->pairs_evaluated = out->pairs_algorithmic;
-  ctx->have_exp = !goose;              // the expander (target) masks are complete: a batch acquisition may start from them
-  ctx->have_tgt = goose != 0;
-  if (!goose) ++ctx->exp_gen;
-  else ++ctx->tgt_gen;
+  // the expander (target) masks are complete: a batch acquisition may start from them
+  stage_changed(ctx, goose ? Change::TARGET : Change::EXPANDER);
   if (!have) return SBO_OK;
   // per-constraint arg-reduction, then first-best across constraints (SafeOpt.py:120-122 / GoOSE.py:110-112)
   const double keep5 = ctx->phase_ms[5];

@@ -702,7 +702,7 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   SBO_REQUIRE(ctx->have_grid, "sbo_posterior: no grid (call sbo_set_grid / sbo_set_points)");
   SBO_REQUIRE(ctx->gs.d == ctx->ms.d, "grid and model dimensions differ");
   SBO_REQUIRE(keep_v >= 0 && keep_v <= 3, "keep_v must be 0, 1, 2 or 3");
-  ctx->up.valid = false;     // mean / var / V rows are overwritten from here on
+  stage_changed(ctx, Change::POSTERIOR);
   const ModelSpec& ms = ctx->ms;
   const long long count = ctx->gs.count;
   SBO_REQUIRE(count > 0, "empty shard");
@@ -715,7 +715,6 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
   const bool fused = separable && ctx->opt_posterior_variant == 1 && ctx->opt_posterior_fused;
   const long long P = fused ? cdiv(count, 128) * 128 : chunk_points(ctx, ms, count);
   if (!fused) SBO_TRY(sbo_ensure(ctx, ctx->kx, sizeof(double) * (size_t)ms.G * ms.npad * P));
-  ctx->keep_v = 0;
   if (keep_v && ms.G > 1) {
     const size_t esz = keep_v == 1 ? sizeof(double) : (keep_v == 3 ? 2 * sizeof(float) : sizeof(float));
     SBO_TRY(sbo_ensure(ctx, ctx->vall, esz * (size_t)(ms.G - 1) * count * ms.npad));
@@ -745,13 +744,9 @@ int posterior_run(sbo_ctx* ctx, int with_grad, int keep_v) {
                              (ms.G > 1) ? keep_v : 0, ctx->vall.p, count));
     ev_end(ctx);
   }
-  if (keep_v && ms.G > 1) ctx->keep_v = keep_v;
-  ctx->have_post = true;
-  ctx->have_grad = with_grad != 0;
-  ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
-  ctx->up.valid = true;
   ctx->up.n = ms.n; ctx->up.npad = ms.npad;
   ctx->up.with_grad = with_grad != 0; ctx->up.keep_v = keep_v;
+  stage_changed(ctx, Change::POSTERIOR_DONE);
   return SBO_OK;
 }
 
@@ -792,10 +787,8 @@ int posterior_update(sbo_ctx* ctx, sbo_update_info* info) {
       SBO_LAUNCH_CHECK();
     }
   }
-  ctx->have_post = true;
-  ctx->have_grad = with_grad;
-  ctx->have_sets = ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
   ctx->up.n = ms.n; ctx->up.npad = ms.npad;
+  stage_changed(ctx, Change::POSTERIOR_DONE);
   return SBO_OK;
 }
 

@@ -525,8 +525,7 @@ int sets_pass1(sbo_ctx* ctx, double beta, int rule, int strict, sbo_sets_result*
   ctx->n_unsafe_local = r.n_unsafe;
   ctx->n_safe_local = r.n_safe;
   ctx->beta = beta;
-  ctx->have_sets = true;
-  ctx->have_sets2 = ctx->have_exp = ctx->have_tgt = false;
+  stage_changed(ctx, Change::SETS1);
   return SBO_OK;
 }
 
@@ -554,7 +553,7 @@ int sets_pass2(sbo_ctx* ctx, double min_ucb0, sbo_sets_result* out) {
   SBO_CUDA(cudaStreamSynchronize(ctx->stream));
   ev_collect(ctx);
   if (out) fill_result(r, out);
-  ctx->have_sets2 = true;
+  stage_changed(ctx, Change::SETS2);
   return SBO_OK;
 }
 
