@@ -187,8 +187,6 @@ int sbo_set_stream(sbo_ctx* ctx, void* cuda_stream) {
 int sbo_set_model_ex(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_norm, const double* Y_norm,
                      const double* X_mean, const double* X_std, const double* Y_mean, const double* Y_std, const double* hyp) {
   ENTER();
-  ctx->have_model = false;
-  stage_changed(ctx, Change::MODEL);
   return model_upload(ctx, kernel, n, d, G, X_norm, Y_norm, X_mean, X_std, Y_mean, Y_std, hyp);
 }
 

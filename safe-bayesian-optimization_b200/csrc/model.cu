@@ -180,6 +180,10 @@ int model_upload(sbo_ctx* ctx, int kernel, int n, int d, int G, const double* X_
   SBO_REQUIRE(G >= 1 && G <= SBO_MAX_G, "G out of range (1..8)");
   SBO_REQUIRE(X_norm && Y_norm && X_mean && X_std && Y_mean && Y_std && hyp, "null model pointer");
   SBO_REQUIRE(kernel_valid(kernel), "unknown kernel (SBO_KERNEL_SE, SBO_KERNEL_MATERN32 or SBO_KERNEL_MATERN52)");
+  // a refused argument leaves the installed model and every stage built on it untouched; from here on the old model is
+  // overwritten, so it and everything after it is invalid until this upload succeeds
+  ctx->have_model = false;
+  stage_changed(ctx, Change::MODEL);
   ev_reset(ctx, 0);
   ev_begin(ctx, 0);
   ModelSpec& ms = ctx->ms;
